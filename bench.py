@@ -4,7 +4,7 @@
 One "step" = one fused pass of the hot path (stages 1-3 + merge + emit) over one batch of synthetic
 rows: int64 key, fp64 value, sum + mean + count, N rows per GPU, G groups.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--rows R] [--groups G] [--sweep]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--rows R] [--groups G] [--sweep] [--dump-outputs DIR]
   python bench.py --impl reference ...      # the reference's CPU path (oracle port) on host cores
 
 Prints ONE JSON line (rank 0).  See DESIGN.md §Measurement for how every field is derived.
@@ -46,7 +46,14 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-rows", type=int, default=100_000_000, help="rows of the bounded CPU-baseline sample")
     ap.add_argument("--extras", action="store_true", help="(default at N=1) config 3 (multi-key, nullable), config 4 (resample OHLC), scattered keys, ...")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (group keys and one array "
+                    "per aggregate) to DIR/<name>.npy as float64; a fixed seeded sample of the groups beyond 64 MB in all")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must be at least 0")
+    return args
 
 
 def peaks():
@@ -124,6 +131,39 @@ def algorithmic_bytes(n_rows: int, n_groups: int, n_aggs: int) -> float:
     return 16.0 * n_rows + n_groups * (8.0 + 8.0 * n_aggs)
 
 
+DUMP_BYTES = 64_000_000      # --dump-outputs: bytes on disk over all files (and all ranks)
+NPY_HEADER_BYTES = 4096      # allowance per file for the .npy header (128 bytes for a 1-D float64 array)
+
+
+def step_outputs(h, limit_bytes: int) -> dict:
+    """What a caller of the timed path receives from handle `h`: the group keys in result order and one array per
+    aggregate, as float64 (the benchmark's keys are group ids below 2^53: exact).  When their .npy files would take
+    more than `limit_bytes`, every array keeps the same fixed seeded sample of group positions, which is stored as
+    `group_index`."""
+    import numpy as np
+    out = {"keys": h.unique().to_numpy(zero_copy_only=False).astype(np.float64)}
+    for a in AGGS:
+        out[a] = h.fetch(a).to_numpy(zero_copy_only=False).astype(np.float64)
+    n = len(out["keys"])
+    if len(out) * (NPY_HEADER_BYTES + 8 * n) > limit_bytes:
+        files = len(out) + 1
+        cap = max(0, (limit_bytes - files * NPY_HEADER_BYTES) // (8 * files))
+        pos = np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+        out = {k: v[pos] for k, v in out.items()}
+        out["group_index"] = pos.astype(np.float64)
+    return out
+
+
+def dump_outputs(h, outdir: str, rank: int = 0, world: int = 1):
+    """--dump-outputs: step_outputs(h) as outdir/<name>.npy; with several ranks each writes the groups it owns as
+    <name>_rank<r>.npy within its share of the byte limit."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    tag = f"_rank{rank}" if world > 1 else ""
+    for name, a in step_outputs(h, DUMP_BYTES // world).items():
+        np.save(os.path.join(outdir, f"{name}{tag}.npy"), a)
+
+
 def _hostgen():
     """hostgen.py (numpy data generator) loaded by path: importing the package would load libpa_b200.so,
     which must not appear in the reference arm's process."""
@@ -170,7 +210,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warm = max(args.steps, 1), args.warmup
+    steps, warm = args.steps, args.warmup
     rows = min(args.cpu_rows, args.rows)
     for _ in range(min(warm, 1)):
         cpu_reference(min(rows, 1_000_000), args.groups)
@@ -259,21 +299,26 @@ def main():
             if len(handles) > 2:
                 handles.pop(0).close()      # (recycled by the library without synchronising)
 
-    def finish_steps():
+    def finish_steps(dump_dir=None):
         nonlocal launches, merged_groups
         t = gb.timing()                     # completes the last local pass (reads its status words)
         scan_ms.append(t["scan_ms"])
-        launches += t["launches"] * (args.steps if args.steps > 0 else 1)
+        launches += t["launches"] * args.steps
         if world > 1:
             m = handles[-1]
             merged_groups = m.groupSize()   # completes the last merge
             launches += (2 + m.timing()["launches"]) * args.steps
+            if dump_dir:
+                dump_outputs(m, dump_dir, rank, world)
             while handles:
                 handles.pop().close()
+        elif dump_dir:
+            dump_outputs(gb, dump_dir)
 
     for _ in range(args.warmup):
         step()
-    finish_steps()
+    if args.warmup:
+        finish_steps()
     scan_ms.clear(); launches = 0
     barrier()
     sampler = ClockSampler(local)
@@ -288,7 +333,7 @@ def main():
     e1.record(stream)
     barrier()
     clocks = sampler.stop() if rank == 0 else None
-    finish_steps()
+    finish_steps(args.dump_outputs)
     ms = e0.elapsed_time(e1)
     tms = torch.tensor([ms], device=dev, dtype=torch.float64)
     if dist is not None:

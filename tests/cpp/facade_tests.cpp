@@ -4,7 +4,10 @@
 // hence the tiny REQUIRE harness.  Needs a GPU (run by tests/test_facade_gpu.py).
 #include <cmath>
 #include <cstdio>
+#include <cstdlib>
+#include <filesystem>
 #include <iostream>
+#include <stdexcept>
 #include <string>
 
 #include <arrow/compute/api.h>
@@ -381,7 +384,14 @@ static void test_sort_and_ingest() {
   {
     // Parquet file -> readParquet
     auto table = pd::ReturnOrThrowOnFailure(arrow::Table::FromRecordBatches({df.array()}));
-    const std::string path = "/tmp/pa_b200_facade_test.parquet";
+    // a directory of our own: a fixed file name in the temp directory may belong to another user of the machine
+    std::string dir = (std::filesystem::temp_directory_path() / "pa_b200_facade_XXXXXX").string();
+    if (!mkdtemp(dir.data())) throw std::runtime_error("mkdtemp failed for " + dir);
+    struct RemoveOnExit {   // also when a call below throws
+      std::string dir;
+      ~RemoveOnExit() { std::error_code ec; std::filesystem::remove_all(dir, ec); }
+    } cleanup{dir};
+    const std::string path = dir + "/facade_test.parquet";
     auto out = pd::ReturnOrThrowOnFailure(arrow::io::FileOutputStream::Open(path));
     pd::ThrowOnFailure(parquet::arrow::WriteTable(*table, arrow::default_memory_pool(), out, 1 << 20));
     pd::ThrowOnFailure(out->Close());
@@ -389,7 +399,7 @@ static void test_sort_and_ingest() {
     REQUIRE(pq.array()->Equals(*df.array()));
     auto s = pd::ReturnOrThrowOnFailure(pq.to_device().group_by("k"s).count("v"));
     REQUIRE(s.values<int64_t>() == (std::vector<int64_t>{3, 2, 2, 1}));
-    REQUIRE_THROWS(pd::DataFrame::readParquet("/tmp/does_not_exist.parquet"));
+    REQUIRE_THROWS(pd::DataFrame::readParquet(dir + "/does_not_exist.parquet"));
   }
 }
 

@@ -70,3 +70,12 @@ def test_traffic_stamp_matches_the_kernel_source():
     t = json.load(open(os.path.join(ROOT, "profiles", "r2_traffic.json")))["k_lowcard_scan"]
     sha = hashlib.sha256(open(os.path.join(ROOT, t["source"]), "rb").read()).hexdigest()[:16]
     assert t["source_sha"] == sha, "lowcard.cuh changed after the traffic capture: re-capture (scripts/r2_run50.sh) and restamp"
+
+
+@pytest.mark.parametrize("flags", [["--steps", "0"], ["--warmup", "-1"]])
+def test_bench_refuses_step_counts_it_cannot_time(flags):
+    """--steps is the number of timed steps: zero of them has no time per step, so the run stops before any work."""
+    import subprocess
+    import sys
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *flags], capture_output=True, text=True, timeout=120)
+    assert r.returncode == 2 and "must be at least" in r.stderr, r.stderr[-2000:]

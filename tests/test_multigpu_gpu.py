@@ -12,7 +12,7 @@ ALL = ["sum", "mean", "count", "min", "max", "first", "last"]
 FMT = {pa.float64(): "g", pa.int64(): "l", pa.float32(): "f", pa.int32(): "i"}
 
 
-def _run_sharded(pab, rb, key, col, aggs, world, path="auto"):
+def _run_sharded(pab, rb, key, col, aggs, world, path="auto", on_merged=None):
     import torch
     from pandasarrow_b200 import distributed as D
     from pandasarrow_b200._lib import PA_PARTIAL_WORDS as W
@@ -45,6 +45,8 @@ def _run_sharded(pab, rb, key, col, aggs, world, path="auto"):
         if len(k):
             own = D.owner_of(k.fill_null(0).to_numpy().astype(np.int64), world, is_null=np.asarray(k.is_null()))
             assert (own == o).all()
+        if on_merged is not None:
+            on_merged(o, m)
         m.close()
     fr = np.concatenate(firsts)
     order = pa.array(np.argsort(fr, kind="stable"))
@@ -82,6 +84,48 @@ def test_sharded_matches_oracle(world, G, path):
     assert sum(res["count"].to_pylist()) == int(hg.valid_mask(n).sum())
     assert len(np.unique(first_rows)) == len(first_rows)
 
+
+
+@pytest.mark.parametrize("n,G", [(400_003, 1000), (12_000_000, 3_000_000)])
+def test_bench_dump_outputs_per_rank(tmp_path, n, G):
+    """bench.py --dump-outputs at N > 1: every owner writes the groups it merged as <name>_rank<r>.npy, all ranks
+    together within the 64 MB on disk (the second case is sampled: ~1.5 M groups per rank); checked against numpy."""
+    import importlib.util
+    import os
+    import pandasarrow_b200 as pab
+    from pandasarrow_b200 import hostgen as hg
+    spec = importlib.util.spec_from_file_location("pa_bench", os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    world = 2
+    k, v = hg.keys(n, G), hg.vals(n)
+    rb = pa.record_batch({"k": pa.array(k), "v": pa.array(v)})
+    rank_keys = {}
+
+    def dump(o, m):
+        rank_keys[o] = m.unique().to_numpy().astype(np.float64)
+        bench.dump_outputs(m, str(tmp_path), o, world)
+
+    _run_sharded(pab, rb, "k", "v", bench.AGGS, world, on_merged=dump)
+    assert sum(os.path.getsize(tmp_path / f) for f in os.listdir(tmp_path)) <= 64_000_000
+    cnt = np.bincount(k, minlength=G)
+    s = np.bincount(k, weights=v, minlength=G)
+    seen = 0
+    for o in range(world):
+        got = {a: np.load(tmp_path / f"{a}_rank{o}.npy") for a in ["keys"] + bench.AGGS}
+        if os.path.exists(tmp_path / f"group_index_rank{o}.npy"):
+            pos = np.load(tmp_path / f"group_index_rank{o}.npy").astype(np.int64)
+            assert 0 < len(pos) < len(rank_keys[o]) and (np.diff(pos) > 0).all()
+        else:
+            pos = np.arange(len(rank_keys[o]))
+            seen += len(pos)
+        assert np.array_equal(got["keys"], rank_keys[o][pos])
+        g = got["keys"].astype(np.int64)
+        assert np.array_equal(got["count"], cnt[g].astype(np.float64))
+        assert np.max(np.abs(got["sum"] - s[g]) / s[g]) <= 1e-12
+        assert np.max(np.abs(got["mean"] - s[g] / cnt[g]) / (s[g] / cnt[g])) <= 1e-12
+    if G == 1000:
+        assert seen == np.count_nonzero(cnt)           # unsampled: the ranks' files hold every group once
 
 def test_sharded_int_values_and_single_rank():
     import pandasarrow_b200 as pab
