@@ -93,7 +93,10 @@ struct ArrowDeviceArray {
  *   MIN/MAX input dtype; NaN skipped unless the group is all-NaN; null for an all-null group
  *   FIRST/LAST value at the first/last row of the group, nulls NOT skipped (positional)
  * Second-stage aggregates (GROUPBY_AGG(product), GROUPBY_NUMERIC_AGG(variance|stddev), dataframe.cpp:1516-1536):
- * a second pass over keys + values after the fused one, single-GPU handles only.
+ * a second pass over keys + values after the fused one.  Row-range shards (multi-GPU, chunked) run it per shard and
+ * merge the terms (PA_PARTIAL_WORDS_STAGE2 records): the per-shard M2 = sum of (x - mean_s)^2 combined with Chan's update
+ * in source-rank order, the per-shard products multiplied in that order.  pa_groupby_aggregate on a merged handle
+ * still refuses them.
  *   PRODUCT  int*->int64 (wraps), uint*->uint64, float/double->double; null for an all-null group
  *   VARIANCE/STDDEV  double, ddof 0, two-pass (mean, then squared deviations) as arrow::compute's
  *            scalar kernel; null for an all-null group (the reference's wrapper drops that validity)
@@ -304,11 +307,20 @@ int pa_sort_indices(pa_groupby* sorted, struct ArrowArray* out, struct ArrowSche
 /* Number of this handle's groups owned by each of n_parts ranks (host array, after an aggregate). */
 int pa_groupby_partials_count(pa_groupby* g, int32_t n_parts, int64_t* counts_host);
 /* Writes the records, grouped by owner rank in ascending order, into caller-provided DEVICE memory
- * (capacity_records >= sum of counts).  Must follow pa_groupby_partials_count with the same n_parts. */
+ * (capacity_records >= sum of counts).  Must follow pa_groupby_partials_count with the same n_parts.
+ * Always PA_PARTIAL_WORDS-word records, also after an aggregate with product / variance / stddev. */
 int pa_groupby_partials_export(pa_groupby* g, int32_t n_parts, void* dev_records, int64_t capacity_records);
+/* Stage-2 records: the PA_PARTIAL_WORDS words, then this handle's M2 = sum of (x - mean)^2 of the group (double bits;
+ * mean = sum / count as the second pass computed it) and its product (raw 64 bits: double, or wrapped (u)int64).  Same
+ * preconditions as pa_groupby_partials_export; PA_ERR_STATE when the last aggregate computed none of
+ * product / variance / stddev (a flag in the record says which of the two terms it holds). */
+#define PA_PARTIAL_WORDS_STAGE2 13
+int pa_groupby_partials_export_stage2(pa_groupby* g, int32_t n_parts, void* dev_records, int64_t capacity_records);
 /* Joins received records (DEVICE memory, grouped by source rank; counts_by_source on the host) by key,
  * folds them in source-rank order and orders the groups by global first row.  The returned handle
- * answers num_groups / unique / fetch for the aggregates in agg_mask.  value_format / key_format are
+ * answers num_groups / unique / fetch for the aggregates in agg_mask (PA_AGG_ALL and PA_AGG_STAGE2 bits).  The
+ * records are PA_PARTIAL_WORDS_STAGE2 words wide exactly when agg_mask has a PA_AGG_STAGE2 bit (then PA_ERR_STATE if
+ * a record lacks the terms asked for), PA_PARTIAL_WORDS otherwise.  value_format / key_format are
  * the Arrow format strings of the value and (single) key column. */
 int pa_merge_create(const void* dev_records, const int64_t* counts_by_source, int32_t n_sources, uint32_t agg_mask,
                     const char* value_format, const char* key_format, const pa_options* opt, pa_groupby** out);
@@ -320,7 +332,7 @@ int pa_merge_create(const void* dev_records, const int64_t* counts_by_source, in
  * (no synchronisation).  All ranks exchange the blocks with an equal-split all-to-all and hand what they
  * received (n_sources blocks, in source-rank order) to pa_merge_create_padded, which returns
  * PA_ERR_STATE when any source sent the overflow marker (every rank sees it: fall back to
- * pa_groupby_partials_count / _export / pa_merge_create). */
+ * pa_groupby_partials_count / _export / pa_merge_create).  PA_AGG_ALL bits only (PA_PARTIAL_WORDS-word records). */
 int pa_groupby_partials_export_padded(pa_groupby* g, int32_t n_parts, void* dev_blocks, int64_t block_records);
 int pa_merge_create_padded(const void* dev_blocks, int32_t n_sources, int64_t block_records, uint32_t agg_mask,
                            const char* value_format, const char* key_format, const pa_options* opt, pa_groupby** out);
@@ -328,7 +340,8 @@ int pa_merge_create_padded(const void* dev_blocks, int32_t n_sources, int64_t bl
 /* Host frames larger than free device memory (or than 2^32-2 rows): the columns are aggregated chunk_rows rows at a
  * time — each chunk copied through the pinned staging pipeline, aggregated with row_base = its first row and exported as
  * partial records — and the chunks' records are merged like ranks' (sources folded in row order, groups in global
- * first-appearance order).  Single key column; sum / mean / count / min / max / first / last.  `merged_out` answers
+ * first-appearance order).  Single key column; sum / mean / count / min / max / first / last / product / variance / stddev
+ * (those three travel in PA_PARTIAL_WORDS_STAGE2-word records).  `merged_out` answers
  * num_groups / unique / fetch like a merged multi-GPU handle.  At most 64 chunks. */
 int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const struct ArrowSchema* key_schema,
                                  const struct ArrowDeviceArray* values, const struct ArrowSchema* value_schema,
@@ -342,7 +355,8 @@ int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const stru
  * rank's row shard (pa_options.row_base = its first global row), the owner bucketing, the exchange of counts
  * (ncclAllGather) and records (grouped ncclSend / ncclRecv), and the owner-side merge; `merged_out` answers
  * num_groups / unique / fetch / first_rows for the groups with hash(key) % world == rank.  Send / receive / merge
- * scratch stays on the communicator between steps.  Aggregates: PA_AGG_ALL bits. */
+ * scratch stays on the communicator between steps.  Aggregates: PA_AGG_ALL and PA_AGG_STAGE2 bits (the latter travel in
+ * PA_PARTIAL_WORDS_STAGE2-word records, see pa_groupby_partials_export_stage2). */
 #define PA_COMM_ID_BYTES 128
 typedef struct pa_comm pa_comm;
 int pa_comm_unique_id(void* out_id, int64_t capacity_bytes);
@@ -354,7 +368,7 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
 /* Device time (ms) of the last step's phases: [0] local pass, [1] count + export, [2] exchange, [3] merge, [4] total. */
 int pa_comm_last_phases(pa_comm* c, double phase_ms[5]);
 /* How the last step's partial aggregates travelled: bytes per group record (32: compact records of sum / mean of floats /
- * count; 88: the full PA_PARTIAL_WORDS record), whether the local pass handed over the bucketed path's unordered group
+ * count; 88: the full PA_PARTIAL_WORDS record; 104: the PA_PARTIAL_WORDS_STAGE2 record), whether the local pass handed over the bucketed path's unordered group
  * records without ordering them first (0 / 1), and the slots of the merge's join table. */
 int pa_comm_last_exchange(pa_comm* c, int32_t* record_bytes, int32_t* unordered_export, int64_t* merge_table_slots);
 

@@ -15,6 +15,8 @@ PA_AGG = {"sum": 1, "mean": 2, "count": 4, "min": 8, "max": 16, "first": 32, "la
           "product": 128, "variance": 256, "stddev": 512, "all": 1024, "any": 2048, "count_distinct": 4096}
 PA_PATH_AUTO, PA_PATH_LOWCARD, PA_PATH_GLOBAL = 0, 1, 2
 PA_PARTIAL_WORDS = 11
+PA_PARTIAL_WORDS_STAGE2 = 13   # records that also carry the product / variance terms
+PA_AGG_STAGE2 = 128 | 256 | 512
 
 # every symbol include/pa_b200.h declares
 EXPORTS = [
@@ -24,6 +26,7 @@ EXPORTS = [
     "pa_groupby_row_ids", "pa_groupby_groupings", "pa_groupby_take_grouped", "pa_groupby_groupings_timing", "pa_groupby_last_timing", "pa_groupby_last_path", "pa_groupby_last_detail",
     "pa_groupby_sync",
     "pa_groupby_destroy", "pa_column_to_device", "pa_sort_create", "pa_sort_indices", "pa_resample_create", "pa_resample_create_calendar", "pa_downsample_create", "pa_groupby_partials_count", "pa_groupby_partials_export",
+    "pa_groupby_partials_export_stage2",
     "pa_merge_create", "pa_groupby_aggregate_chunked", "pa_groupby_partials_export_padded", "pa_merge_create_padded", "pa_groupby_first_rows", "pa_synth_keys_i64", "pa_synth_vals_f64",
     "pa_synth_validity", "pa_synth_timestamps",
     "pa_comm_unique_id", "pa_comm_create", "pa_comm_adopt", "pa_comm_destroy", "pa_groupby_sharded_aggregate", "pa_comm_last_phases", "pa_comm_last_exchange",
@@ -128,6 +131,7 @@ def load():
                                        C.c_int32, C.c_int32, C.POINTER(PaOptions), C.POINTER(P)]
     L.pa_groupby_partials_count.argtypes = [P, C.c_int32, C.POINTER(C.c_int64)]
     L.pa_groupby_partials_export.argtypes = [P, C.c_int32, P, C.c_int64]
+    L.pa_groupby_partials_export_stage2.argtypes = [P, C.c_int32, P, C.c_int64]
     L.pa_merge_create.argtypes = [P, C.POINTER(C.c_int64), C.c_int32, C.c_uint32, C.c_char_p, C.c_char_p,
                                   C.POINTER(PaOptions), C.POINTER(P)]
     L.pa_groupby_aggregate_chunked.argtypes = [C.POINTER(ArrowDeviceArray), C.POINTER(ArrowSchema), C.POINTER(ArrowDeviceArray), C.POINTER(ArrowSchema),

@@ -449,6 +449,11 @@ struct pa_groupby {
   GroupResult res{};
   // outputs of the last aggregate
   std::vector<AggOut> outs;
+  // product / variance / stddev of the last aggregate: which of them it computed (PA_AGG_STAGE2 bits, 0 = none) and its
+  // per-group terms — M2 = sum of (x - mean)^2 and the product — kept until the next aggregate for the stage-2 partial
+  // export (pa_groupby_partials_export_stage2); on a merged handle, the merged terms
+  uint32_t s2_ext = 0;
+  DevBuf s2_m2, s2_prod;
   bool last_wide = false;
   int last_vc = VC_I, last_vw = 8;
   std::string last_vfmt = "l";
@@ -1268,25 +1273,19 @@ int verify_string_keys(pa_groupby* g, bool* collided) {
   return PA_OK;
 }
 
-// product / variance / stddev (stage2.cuh): the second pass over keys + values, after the ordinary pass has
-// produced sum (or the double sum) and count per group.  Appends its outputs to g->outs.
-int run_stage2(pa_groupby* g, const Column* val, uint32_t ext) {
+// Outputs of product / variance / stddev (k_stage2_emit) from the per-group terms on the handle (g->s2_m2 / s2_prod):
+// after the second pass on a rank's rows, or after the merge of stage-2 records.  Appends them to g->outs.
+int emit_stage2(pa_groupby* g, int vc, uint32_t ext) {
   cudaStream_t st = g->stream;
   const uint32_t G = g->G;
-  const int vc = val->vc;
   const size_t words = (static_cast<size_t>(G) + 31) / 32 + 1;
-  const bool want_m2 = (ext & (AGG_VARIANCE | AGG_STDDEV)) != 0, want_prod = (ext & AGG_PRODUCT) != 0;
-  DevBuf mean, m2, prod;
   const size_t gbytes = static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8;
-  PA_TRY(mean.alloc(gbytes, st));
-  if (want_m2) PA_TRY(m2.alloc(gbytes, st));
-  if (want_prod) PA_TRY(prod.alloc(gbytes, st));
   Stage2Emit e{};
   e.r = g->res;
   e.G = G;
   e.vc = vc;
-  e.m2 = m2.as<double>();
-  e.prod = prod.as<unsigned long long>();
+  e.m2 = (ext & (AGG_VARIANCE | AGG_STDDEV)) ? g->s2_m2.as<double>() : nullptr;
+  e.prod = (ext & AGG_PRODUCT) ? g->s2_prod.as<unsigned long long>() : nullptr;
   auto add = [&](uint32_t bit, const std::string& fmt, void** vptr, uint32_t** bptr) -> int {
     g->outs.emplace_back();
     AggOut& o = g->outs.back();
@@ -1306,9 +1305,31 @@ int run_stage2(pa_groupby* g, const Column* val, uint32_t ext) {
   if (ext & AGG_VARIANCE) { PA_TRY(add(AGG_VARIANCE, "g", &v, &b)); e.o_var = static_cast<double*>(v); e.o_var_valid = b; }
   if (ext & AGG_STDDEV) { PA_TRY(add(AGG_STDDEV, "g", &v, &b)); e.o_std = static_cast<double*>(v); e.o_std_valid = b; }
   if (G == 0) return PA_OK;
+  k_stage2_emit<<<(G + 255) / 256, 256, 0, st>>>(e);
+  CUDA_TRY(cudaGetLastError());
+  return PA_OK;
+}
+
+// product / variance / stddev (stage2.cuh): the second pass over keys + values, after the ordinary pass has
+// produced sum (or the double sum) and count per group.  Appends its outputs to g->outs; the per-group M2 / product stay
+// on the handle (g->s2_m2 / s2_prod) until the next aggregate.
+int run_stage2(pa_groupby* g, const Column* val, uint32_t ext) {
+  cudaStream_t st = g->stream;
+  const uint32_t G = g->G;
+  const int vc = val->vc;
+  const bool want_m2 = (ext & (AGG_VARIANCE | AGG_STDDEV)) != 0, want_prod = (ext & AGG_PRODUCT) != 0;
+  DevBuf mean;
+  const size_t gbytes = static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8;
+  PA_TRY(mean.alloc(gbytes, st));
+  if (want_m2) PA_TRY(g->s2_m2.alloc(gbytes, st)); else g->s2_m2.reset();
+  if (want_prod) PA_TRY(g->s2_prod.alloc(gbytes, st)); else g->s2_prod.reset();
+  double* m2 = want_m2 ? g->s2_m2.as<double>() : nullptr;
+  unsigned long long* prod = want_prod ? g->s2_prod.as<unsigned long long>() : nullptr;
+  g->s2_ext = ext;
+  if (G == 0) return emit_stage2(g, vc, ext);
   RowLookup lk;
   PA_TRY(build_row_lookup(g, &lk));
-  k_stage2_init<<<(G + 255) / 256, 256, 0, st>>>(g->res, G, vc, mean.as<double>(), m2.as<double>(), prod.as<unsigned long long>());
+  k_stage2_init<<<(G + 255) / 256, 256, 0, st>>>(g->res, G, vc, mean.as<double>(), m2, prod);
   CUDA_TRY(cudaGetLastError());
   Stage2Args a{};
   a.ids = lk.a;
@@ -1317,8 +1338,8 @@ int run_stage2(pa_groupby* g, const Column* val, uint32_t ext) {
   a.voff = val->bit_off;
   a.vw = val->width;
   a.mean = mean.as<double>();
-  a.m2 = m2.as<double>();
-  a.prod = prod.as<unsigned long long>();
+  a.m2 = m2;
+  a.prod = prod;
   a.use_smem = G <= S2_SMEM_SLOTS ? 1u : 0u;
   a.rlog = 0;
   // (replicas only while they stay small: the key -> id lookups want the L1 that shared memory takes away —
@@ -1335,11 +1356,10 @@ int run_stage2(pa_groupby* g, const Column* val, uint32_t ext) {
     kern<<<grid, S2_THREADS, smem, st>>>(a);
     CUDA_TRY(cudaGetLastError());
   }
-  k_stage2_emit<<<(G + 255) / 256, 256, 0, st>>>(e);
-  CUDA_TRY(cudaGetLastError());
+  PA_TRY(emit_stage2(g, vc, ext));
   g->last_launches += 5;
   CUDA_TRY(cudaEventRecord(g->ev[4], st));
-  // (mean / m2 / prod and the lookup table are released in stream order when this scope ends)
+  // (mean and the lookup table are released in stream order when this scope ends)
   return PA_OK;
 }
 
@@ -2012,6 +2032,9 @@ static int aggregate_entry(pa_groupby* g, const struct ArrowDeviceArray* values,
     g->pending_prev_G = prev_G;
     g->pending_had_groups = had;
   }
+  // the stage-2 terms of an earlier aggregate do not belong to this one (run_stage2 sets them again)
+  g->s2_ext = 0;
+  if (!ext) { g->s2_m2.reset(); g->s2_prod.reset(); }
   PA_TRY(aggregate_impl(g, &val, agg_mask, deferred));
   if (g->pending) return PA_OK;
   if (had && prev_G != g->G) return set_err(PA_ERR_STATE, "group count changed between passes (%u vs %u)", prev_G, g->G);
@@ -2931,8 +2954,11 @@ int pa_groupby_partials_count(pa_groupby* g, int32_t n_parts, int64_t* counts_ho
   return PA_OK;
 }
 
-// `compact`: REC_WORDS_COMPACT-word records (merge.cuh) — the sharded step's own format for narrow aggregate sets
-static int partials_export(pa_groupby* g, int32_t n_parts, void* dev_records, int64_t capacity_records, bool compact) {
+static_assert(REC_WORDS == PA_PARTIAL_WORDS && REC_WORDS_STAGE2 == PA_PARTIAL_WORDS_STAGE2, "public record widths");
+
+// `words`: REC_WORDS (the public record), REC_WORDS_STAGE2 (plus the stage-2 terms of the last aggregate) or
+// REC_WORDS_COMPACT (merge.cuh) — the sharded step's own format for narrow aggregate sets
+static int partials_export(pa_groupby* g, int32_t n_parts, void* dev_records, int64_t capacity_records, int words) {
   if (!g || !dev_records) return set_err(PA_ERR_INVALID, "null argument");
   if (g->parts_n != n_parts) return set_err(PA_ERR_STATE, "call pa_groupby_partials_count(n_parts=%d) first", n_parts);
   if (capacity_records < static_cast<int64_t>(g->G)) return set_err(PA_ERR_INVALID, "record buffer too small");
@@ -2946,7 +2972,15 @@ static int partials_export(pa_groupby* g, int32_t n_parts, void* dev_records, in
   PartialsArgs a{};
   a.r = g->res; a.G = g->G; a.nparts = n_parts; a.row_base = g->opt.row_base;
   a.vw = g->last_vw; a.wide = g->last_wide;
-  a.compact = compact;
+  a.words = words;
+  if (words == REC_WORDS_STAGE2) {
+    if (!g->s2_ext) return set_err(PA_ERR_STATE, "the last aggregate computed no product / variance / stddev: nothing for stage-2 records");
+    // integer values: the merge recomputes the mean M2 was taken around from the double sum
+    if (g->last_vc != VC_F && (g->s2_ext & (AGG_VARIANCE | AGG_STDDEV)) && !g->res.dsum)
+      return set_err(PA_ERR_STATE, "stage-2 export: the last aggregate kept no double sum");
+    a.m2 = (g->s2_ext & (AGG_VARIANCE | AGG_STDDEV)) ? g->s2_m2.as<double>() : nullptr;
+    a.prod = (g->s2_ext & AGG_PRODUCT) ? g->s2_prod.as<unsigned long long>() : nullptr;
+  }
   for (auto& o : g->outs) {
     if (o.bit == AGG_FIRST) { a.first_vals = o.values.p; a.first_valid = o.valid.as<uint32_t>(); }
     if (o.bit == AGG_LAST) { a.last_vals = o.values.p; a.last_valid = o.valid.as<uint32_t>(); }
@@ -2962,7 +2996,12 @@ static int partials_export(pa_groupby* g, int32_t n_parts, void* dev_records, in
 }
 
 int pa_groupby_partials_export(pa_groupby* g, int32_t n_parts, void* dev_records, int64_t capacity_records) {
-  return partials_export(g, n_parts, dev_records, capacity_records, false);
+  return partials_export(g, n_parts, dev_records, capacity_records, REC_WORDS);
+}
+
+int pa_groupby_partials_export_stage2(pa_groupby* g, int32_t n_parts, void* dev_records, int64_t capacity_records) {
+  if (g && g->merged) return set_err(PA_ERR_STATE, "partials need a finished local aggregate");
+  return partials_export(g, n_parts, dev_records, capacity_records, REC_WORDS_STAGE2);
 }
 
 // Common part of the two merge entry points.  `d_off` = device array [n_sources + 1], exclusive prefix
@@ -2995,7 +3034,9 @@ static int merge_build(pa_groupby* g, const void* dev_records, const uint64_t* d
   MergeArgs a{};
   a.records = static_cast<const uint64_t*>(dev_records);
   a.src_offset = d_off;
-  a.nsrc = n_sources; a.nrec = nrec_max; a.compact = compact;
+  const uint32_t ext = agg_mask & PA_AGG_STAGE2;
+  a.nsrc = n_sources; a.nrec = nrec_max;
+  a.words = compact ? REC_WORDS_COMPACT : (ext ? REC_WORDS_STAGE2 : REC_WORDS);
   a.status = g->status.as<uint32_t>();
   a.m_first_row = m_first.as<uint64_t>(); a.m_slot = m_slot.as<uint32_t>();
   a.vc = g->last_vc;
@@ -3050,6 +3091,9 @@ static int merge_build(pa_groupby* g, const void* dev_records, const uint64_t* d
   PA_TRY(g->m_last_val.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
   PA_TRY(g->m_first_valid.alloc(std::max<uint32_t>(G, 1), st));
   PA_TRY(g->m_last_valid.alloc(std::max<uint32_t>(G, 1), st));
+  if (ext & (AGG_VARIANCE | AGG_STDDEV)) PA_TRY(g->s2_m2.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
+  if (ext & AGG_PRODUCT) PA_TRY(g->s2_prod.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
+  uint32_t h_no_terms = 0;
   if (G) {
     PA_TRY(s_first.alloc(static_cast<size_t>(G) * 8, st));
     PA_TRY(s_slot.alloc(static_cast<size_t>(G) * 4, st));
@@ -3066,23 +3110,37 @@ static int merge_build(pa_groupby* g, const void* dev_records, const uint64_t* d
     a.o_first_val = g->m_first_val.as<uint64_t>(); a.o_last_val = g->m_last_val.as<uint64_t>();
     a.o_first_valid = g->m_first_valid.as<uint8_t>(); a.o_last_valid = g->m_last_valid.as<uint8_t>();
     a.o_first_row_g = g->m_first_row_g.as<uint64_t>();
-    k_merge_fold<<<(G + 255) / 256, 256, 0, st>>>(a);
-    CUDA_TRY(cudaGetLastError());
+    if (ext) {
+      a.o_m2 = (ext & (AGG_VARIANCE | AGG_STDDEV)) ? g->s2_m2.as<double>() : nullptr;
+      a.o_prod = (ext & AGG_PRODUCT) ? g->s2_prod.as<unsigned long long>() : nullptr;
+      k_merge_fold<true><<<(G + 255) / 256, 256, 0, st>>>(a);
+      CUDA_TRY(cudaGetLastError());
+      CUDA_TRY(cudaMemcpyAsync(&h_no_terms, a.status + ST_NO_TERMS, sizeof h_no_terms, cudaMemcpyDeviceToHost, st));
+    } else {
+      k_merge_fold<false><<<(G + 255) / 256, 256, 0, st>>>(a);
+      CUDA_TRY(cudaGetLastError());
+    }
   }
   CUDA_TRY(cudaEventRecord(g->ev[3], st));
   g->have_groups = true;
   g->last_launches = 4;
   g->last_path = 4;
   PA_TRY(run_emit(g, nullptr, agg_mask));
+  if (ext) {
+    PA_TRY(emit_stage2(g, g->last_vc, ext));
+    g->last_launches += 1;
+  }
   CUDA_TRY(cudaEventRecord(g->ev[4], st));
   CUDA_TRY(cudaStreamSynchronize(st));   // local scratch (table, idx, sort buffers) is released after this point
+  if (h_no_terms) return set_err(PA_ERR_STATE, "partial records carry no variance / product terms for this aggregate mask "
+                                               "(export them with pa_groupby_partials_export_stage2 after an aggregate that computes them)");
   return PA_OK;
 }
 
 int pa_merge_create(const void* dev_records, const int64_t* counts_by_source, int32_t n_sources, uint32_t agg_mask,
                     const char* value_format, const char* key_format, const pa_options* opt, pa_groupby** out) {
   if (!counts_by_source || n_sources < 1 || !value_format || !key_format || !out) return set_err(PA_ERR_INVALID, "null argument");
-  if (agg_mask & ~PA_AGG_ALL) return set_err(PA_ERR_INVALID, "bad aggregate mask");
+  if (agg_mask & ~(PA_AGG_ALL | PA_AGG_STAGE2)) return set_err(PA_ERR_INVALID, "bad aggregate mask");
   HandlePtr g(new pa_groupby());
   PA_TRY(handle_init(g.get(), opt));
   cudaStream_t st = g->stream;
@@ -3113,6 +3171,7 @@ int pa_groupby_partials_export_padded(pa_groupby* g, int32_t n_parts, void* dev_
   PartialsArgs a{};
   a.r = g->res; a.G = g->G; a.nparts = n_parts; a.row_base = g->opt.row_base;
   a.vw = g->last_vw; a.wide = g->last_wide;
+  a.words = REC_WORDS;
   for (auto& o : g->outs) {
     if (o.bit == AGG_FIRST) { a.first_vals = o.values.p; a.first_valid = o.valid.as<uint32_t>(); }
     if (o.bit == AGG_LAST) { a.last_vals = o.values.p; a.last_valid = o.valid.as<uint32_t>(); }
@@ -3239,11 +3298,15 @@ int merge_padded_general(pa_groupby* g, const void* dev_blocks, int32_t n_source
 // columns is copied (staged, §h2d_copy), aggregated with row_base = its first row, and exported as partial records;
 // the owner-side merge then joins the chunks' records exactly as it joins ranks' — sources folded in chunk (= row)
 // order, groups ordered by global first row.  Device memory in use: one chunk of keys and values + the records.
+// Product / variance / stddev: every chunk's two-pass terms travel in stage-2 records (merge.cuh).
 int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const struct ArrowSchema* key_schema,
                                  const struct ArrowDeviceArray* values, const struct ArrowSchema* value_schema,
                                  uint32_t agg_mask, int64_t chunk_rows, const pa_options* opt, pa_groupby** merged_out) {
   if (!keys || !key_schema || !values || !value_schema || !merged_out) return set_err(PA_ERR_INVALID, "null argument");
-  if (agg_mask == 0 || (agg_mask & ~PA_AGG_ALL)) return set_err(PA_ERR_NOT_IMPLEMENTED, "chunked aggregates: sum / mean / count / min / max / first / last");
+  if (agg_mask == 0 || (agg_mask & ~(PA_AGG_ALL | PA_AGG_STAGE2)))
+    return set_err(PA_ERR_NOT_IMPLEMENTED, "chunked aggregates: sum / mean / count / min / max / first / last / product / variance / stddev");
+  const bool stage2 = (agg_mask & PA_AGG_STAGE2) != 0;
+  const size_t RW = stage2 ? PA_PARTIAL_WORDS_STAGE2 : PA_PARTIAL_WORDS;
   if (keys->device_type == ARROW_DEVICE_CUDA || values->device_type == ARROW_DEVICE_CUDA)
     return set_err(PA_ERR_INVALID, "chunked aggregation is for HOST columns (device columns already fit the device)");
   const int64_t n = keys->array.length;
@@ -3276,15 +3339,15 @@ int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const stru
     PA_TRY(pa_groupby_partials_count(h, 1, &cnt));
     counts[static_cast<size_t>(c)] = cnt;
     // grow the record buffer (plain allocation: it outlives the per-chunk handles and their streams)
-    const size_t need = (total + static_cast<uint64_t>(cnt)) * PA_PARTIAL_WORDS * 8;
+    const size_t need = (total + static_cast<uint64_t>(cnt)) * RW * 8;
     if (need > records.bytes) {
       DevBuf bigger;
       bigger.plain = true;
       PA_TRY(bigger.alloc(std::max<size_t>(need * 2, 1u << 20), nullptr));
-      if (total) CUDA_TRY(cudaMemcpy(bigger.p, records.p, total * PA_PARTIAL_WORDS * 8, cudaMemcpyDeviceToDevice));
+      if (total) CUDA_TRY(cudaMemcpy(bigger.p, records.p, total * RW * 8, cudaMemcpyDeviceToDevice));
       records = std::move(bigger);
     }
-    if (cnt) PA_TRY(pa_groupby_partials_export(h, 1, static_cast<char*>(records.p) + total * PA_PARTIAL_WORDS * 8, cnt));
+    if (cnt) PA_TRY((stage2 ? pa_groupby_partials_export_stage2 : pa_groupby_partials_export)(h, 1, static_cast<char*>(records.p) + total * RW * 8, cnt));
     PA_TRY(pa_groupby_sync(h));
     total += static_cast<uint64_t>(cnt);
   }
@@ -3385,7 +3448,8 @@ int pa_comm_last_phases(pa_comm* c, double phase_ms[5]) {
 int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDeviceArray* values,
                                  const struct ArrowSchema* value_schema, uint32_t agg_mask, pa_groupby** merged_out) {
   if (!g || !c || !values || !value_schema || !merged_out) return set_err(PA_ERR_INVALID, "null argument");
-  if (agg_mask == 0 || (agg_mask & ~PA_AGG_ALL)) return set_err(PA_ERR_NOT_IMPLEMENTED, "sharded aggregates: sum / mean / count / min / max / first / last");
+  if (agg_mask == 0 || (agg_mask & ~(PA_AGG_ALL | PA_AGG_STAGE2)))
+    return set_err(PA_ERR_NOT_IMPLEMENTED, "sharded aggregates: sum / mean / count / min / max / first / last / product / variance / stddev");
   if (g->device != c->device) return set_err(PA_ERR_INVALID, "handle lives on device %d, communicator on %d", g->device, c->device);
   if (g->keys.size() != 1 && !g->resample) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of composite keys");
   if (!g->resample && g->keys[0].is_str) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of utf8 keys: dictionary-encode the column against a shared dictionary");
@@ -3395,10 +3459,12 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   CUDA_TRY(cudaEventRecord(c->ev[0], st));
   // 1. local pass.  sum / mean of floats / count need one 32-byte sector per group (compact records, merge.cuh),
   // everything else the full record; with compact records the bucketed path may hand over its unordered group records
-  // as they are (the merge orders by global first row anyway).
+  // as they are (the merge orders by global first row anyway).  Product / variance / stddev: the local pass runs its
+  // second stage too, and the records carry its terms (REC_WORDS_STAGE2).
   int vw_ = 8, vc_ = VC_I;
   PA_TRY(parse_format(value_schema->format, &vw_, &vc_));
-  const bool compact = !is_wide(agg_mask, vc_) && !(agg_mask & (AGG_FIRST | AGG_LAST));
+  const bool stage2 = (agg_mask & PA_AGG_STAGE2) != 0;
+  const bool compact = !stage2 && !is_wide(agg_mask, vc_) && !(agg_mask & (AGG_FIRST | AGG_LAST));
   g->want_unordered = compact && !g->resample;
   const int local_rc = aggregate_entry(g, values, value_schema, agg_mask, false);
   g->want_unordered = false;
@@ -3444,7 +3510,8 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
     row_bound = std::max(row_bound, all[static_cast<size_t>(p) * W1 + W]);
   }
   // 3. export the records grouped by owner
-  const size_t RW = static_cast<size_t>(rec_words(compact));
+  const int words = stage2 ? REC_WORDS_STAGE2 : rec_words(compact);
+  const size_t RW = static_cast<size_t>(words);
   PA_TRY(c->send.alloc(std::max<uint64_t>(send_total, 1) * RW * 8, st));
   PA_TRY(c->recv.alloc(std::max<uint64_t>(recv_total, 1) * RW * 8, st));
   if (unordered) {
@@ -3461,7 +3528,7 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   } else {
     g->parts_n = W;
     g->parts_counts.assign(send_cnt.begin(), send_cnt.end());
-    PA_TRY(partials_export(g, W, c->send.p, static_cast<int64_t>(std::max<uint64_t>(send_total, g->G)), compact));
+    PA_TRY(partials_export(g, W, c->send.p, static_cast<int64_t>(std::max<uint64_t>(send_total, g->G)), words));
   }
   CUDA_TRY(cudaEventRecord(c->ev[2], st));
   // 4. all-to-all of the records

@@ -28,6 +28,7 @@ constexpr int ST_UNSORTED = 2;   // resample: timestamps not sorted
 constexpr int ST_COUNTER = 3;    // scratch append counter
 constexpr int ST_DENSE_MISS = 4; // low-cardinality dense mode met a key outside its window -> rerun in hash mode
 constexpr int ST_PEER_OVERFLOW = 4;  // merge of padded blocks: a source had more groups than a block holds (own status buffer)
+constexpr int ST_NO_TERMS = 2;    // merge of stage-2 records: a record lacks the variance / product terms asked for (own status buffer)
 constexpr int ST_ABORT = 5;      // some CTA gave up (overflow / dense miss): the others stop early, merge is skipped
 constexpr int ST_MODE = 6;       // low-cardinality scan: 1 dense, 2 hash
 constexpr int ST_RLOG = 7;       // low-cardinality scan: log2 of the accumulator replication

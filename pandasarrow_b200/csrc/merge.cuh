@@ -6,6 +6,9 @@
 //   3. k_merge_insert / k_merge_fold join the received records by key and fold them IN SOURCE-RANK
 //      ORDER (at most one record per source and key), so fp64 sums do not depend on arrival order;
 //   4. the merged groups are ordered by their global first row.
+// Product / variance / stddev travel in a longer record (REC_WORDS_STAGE2): every source ships its two-pass terms
+// (M2 = sum of (x - mean)^2 around its own mean, and its product), and k_merge_fold<true> combines them in source-rank
+// order with Chan's pairwise update of (n, mean, M2) and a plain product.
 // The reference has no multi-device path at all (SURVEY.md §2b); this is new structure.
 #pragma once
 #include "group_result.cuh"
@@ -15,7 +18,12 @@ namespace pa {
 // One partial aggregate = PA_REC_WORDS 64-bit words.
 constexpr int REC_KEY = 0, REC_FLAGS = 1, REC_SUM = 2, REC_DSUM = 3, REC_COUNT = 4, REC_FIRST_ROW = 5,
               REC_LAST_ROW = 6, REC_MIN = 7, REC_MAX = 8, REC_FIRST_VAL = 9, REC_LAST_VAL = 10, REC_WORDS = 11;
-constexpr uint64_t RF_KEY_NULL = 1, RF_FIRST_VALID = 2, RF_LAST_VALID = 4;
+// Stage-2 record (PA_PARTIAL_WORDS_STAGE2): the REC_WORDS words above, then M2 (double bits) and the product (raw 64 bits
+// in the value class: double bits for floats, the wrapped (u)int64 otherwise).  RF_HAS_M2 / RF_HAS_PROD say which of the
+// two the source's aggregate computed; the mean M2 was taken around is sum / count (floats) or dsum / count (integers),
+// the division k_stage2_init does, so the merge recomputes it from the record.
+constexpr int REC_M2 = 11, REC_PROD = 12, REC_WORDS_STAGE2 = 13;
+constexpr uint64_t RF_KEY_NULL = 1, RF_FIRST_VALID = 2, RF_LAST_VALID = 4, RF_HAS_M2 = 8, RF_HAS_PROD = 16;
 // Compact record of the sharded step (pa_groupby_sharded_aggregate) when the aggregate set needs nothing but
 // sum / count / first row (sum, mean of floats, count): ONE 32-byte sector per group instead of 88 bytes —
 // 100 M groups per rank: 3.2 GB instead of 8.8 GB written, sent and joined.  Internal to the library (both ends of the
@@ -43,7 +51,10 @@ struct PartialsArgs {
   const void* last_vals; const uint32_t* last_valid;
   int vw;
   bool wide;
-  bool compact;                // write REC_WORDS_COMPACT-word records (narrow aggregate sets, sharded step only)
+  int words;                   // record width: REC_WORDS, REC_WORDS_STAGE2, or REC_WORDS_COMPACT (narrow aggregate sets,
+                               // sharded step only)
+  const double* m2;            // stage-2 records: per-group M2 / product of the last aggregate, or null when it computed none
+  const unsigned long long* prod;
   const uint32_t* G_dev;       // optional: group count on the device (deferred local aggregate)
   const uint32_t* abort_dev;   // optional: non-zero = the local pass failed, send overflow markers
   unsigned long long* counts;  // [nparts] (device)
@@ -71,7 +82,7 @@ __device__ __forceinline__ uint64_t load_raw(const void* p, uint32_t i, int vw) 
 }
 
 __device__ __forceinline__ void write_partial_record(const PartialsArgs& a, uint32_t g, uint8_t kind, uint64_t* rec) {
-  if (a.compact) {   // one sector, two 16-byte stores
+  if (a.words == REC_WORDS_COMPACT) {   // one sector, two 16-byte stores
     ulonglong2 lo, hi;
     lo.x = a.r.key[g];
     lo.y = a.r.sum[g];
@@ -101,6 +112,11 @@ __device__ __forceinline__ void write_partial_record(const PartialsArgs& a, uint
   }
   rec[REC_FIRST_VAL] = fv;
   rec[REC_LAST_VAL] = lv;
+  if (a.words == REC_WORDS_STAGE2) {
+    rec[REC_M2] = a.m2 ? static_cast<uint64_t>(__double_as_longlong(a.m2[g])) : 0ull;
+    rec[REC_PROD] = a.prod ? a.prod[g] : 0ull;
+    flags |= (a.m2 ? RF_HAS_M2 : 0ull) | (a.prod ? RF_HAS_PROD : 0ull);
+  }
   rec[REC_FLAGS] = flags;
 }
 
@@ -123,7 +139,7 @@ __global__ void __launch_bounds__(256) k_partials_scatter(PartialsArgs a) {
   if (threadIdx.x < a.nparts && s_cnt[threadIdx.x])
     s_base[threadIdx.x] = atomicAdd(a.cursor + threadIdx.x, static_cast<unsigned long long>(s_cnt[threadIdx.x]));
   __syncthreads();
-  if (g < a.G) write_partial_record(a, g, kind, a.records + (s_base[o] + local) * rec_words(a.compact));
+  if (g < a.G) write_partial_record(a, g, kind, a.records + (s_base[o] + local) * a.words);
 }
 
 // Few groups: no host round trip.  One CTA writes, for every destination rank, a fixed-size block
@@ -185,7 +201,7 @@ struct MergeArgs {
   const uint64_t* records;       // all received records, grouped by source rank
   const uint64_t* src_offset;    // [nsrc + 1] exclusive prefix of the per-source record counts (device)
   uint32_t nsrc;
-  bool compact;                  // records are REC_WORDS_COMPACT words (see above)
+  int words;                     // record stride: REC_WORDS, REC_WORDS_STAGE2, or REC_WORDS_COMPACT (compact layout, see above)
   uint64_t nrec;                 // upper bound (grid sizing); the exact count is src_offset[nsrc]
   unsigned long long* tkeys;     // cap + 2 keys
   uint64_t cap_mask;
@@ -199,6 +215,8 @@ struct MergeArgs {
   GroupResult out;
   uint64_t* o_first_val; uint64_t* o_last_val; uint8_t* o_first_valid; uint8_t* o_last_valid;
   uint64_t* o_first_row_g;       // global first row of every merged group
+  double* o_m2;                  // stage-2 records: merged M2 / product of every merged group, null when not asked for
+  unsigned long long* o_prod;
   const uint32_t* order;         // slot of the r-th merged group (after the sort)
   uint32_t G;
   int vc;
@@ -210,11 +228,11 @@ __global__ void __launch_bounds__(256) k_merge_insert(MergeArgs a) {
   // source rank of record i (nsrc is small: linear scan of the prefix array)
   uint32_t s = 0;
   while (s + 1 < a.nsrc && i >= a.src_offset[s + 1]) ++s;
-  const uint64_t* rec = a.records + i * rec_words(a.compact);
+  const uint64_t* rec = a.records + i * a.words;
   const uint64_t key = rec[REC_KEY];
   const uint64_t cap = a.cap_mask + 1;
   uint64_t slot;
-  if (rec_key_null(rec, a.compact)) slot = cap;
+  if (rec_key_null(rec, a.words == REC_WORDS_COMPACT)) slot = cap;
   else if (key == kEmptyKey) slot = cap + 1;
   else {
     // Home slot = TOP bits of the partitioning mix of bucketed.cuh (rp_mix; a different function than owner_of's hash,
@@ -251,7 +269,7 @@ __global__ void __launch_bounds__(MC_THREADS) k_merge_compact(MergeArgs a) {
     for (uint32_t s = 0; s < a.nsrc; ++s) {
       const uint32_t i = a.idx[slot * a.nsrc + s];
       if (i == 0xFFFFFFFFu) continue;
-      const uint64_t f = rec_first_row(a.records + static_cast<uint64_t>(i) * rec_words(a.compact), a.compact);
+      const uint64_t f = rec_first_row(a.records + static_cast<uint64_t>(i) * a.words, a.words == REC_WORDS_COMPACT);
       first = f < first ? f : first;
     }
   }
@@ -279,7 +297,12 @@ __global__ void __launch_bounds__(MC_THREADS) k_merge_compact(MergeArgs a) {
   }
 }
 
-// One thread per merged group (final order): fold the sources in rank order.
+// One thread per merged group (final order): fold the sources in rank order.  STAGE2: REC_WORDS_STAGE2-word records,
+// whose M2 and product terms are combined as well — sources without values (count 0) are skipped, the first one that
+// has some sets (n, mean, M2), every later one applies Chan's update
+//   delta = mean_b - mean, n' = n + n_b, M2 += M2_b + delta^2 n n_b / n', mean += delta n_b / n'
+// and the products are multiplied in rank order.  A record without the terms the merge asks for sets ST_NO_TERMS.
+template <bool STAGE2>
 __global__ void __launch_bounds__(256) k_merge_fold(MergeArgs a) {
   const uint32_t g = blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= a.G) return;
@@ -287,10 +310,14 @@ __global__ void __launch_bounds__(256) k_merge_fold(MergeArgs a) {
   uint64_t key = 0, sum = 0, mn = kMinInit, mx = kMaxInit, cnt = 0, first = ~0ull, last = 0, fv = 0, lv = 0;
   double fsum = 0.0, dsum = 0.0;
   bool knull = false, fvalid = false, lvalid = false, any_last = false;
+  uint64_t s2_n = 0;
+  double s2_mean = 0.0, s2_m2 = 0.0;
+  uint64_t s2_prod = a.vc == VC_F ? static_cast<uint64_t>(__double_as_longlong(1.0)) : 1ull;
+  bool s2_missing = false;
   for (uint32_t s = 0; s < a.nsrc; ++s) {
     const uint32_t i = a.idx[slot * a.nsrc + s];
     if (i == 0xFFFFFFFFu) continue;
-    if (a.compact) {   // {key, sum, count | null-key bit, global first row}: one 32-byte sector
+    if (!STAGE2 && a.words == REC_WORDS_COMPACT) {   // {key, sum, count | null-key bit, global first row}: one 32-byte sector
       const ulonglong2* r2 = reinterpret_cast<const ulonglong2*>(a.records + static_cast<uint64_t>(i) * REC_WORDS_COMPACT);
       const ulonglong2 lo = r2[0], hi = r2[1];
       key = lo.x;
@@ -301,9 +328,39 @@ __global__ void __launch_bounds__(256) k_merge_fold(MergeArgs a) {
       first = hi.y < first ? hi.y : first;
       continue;
     }
-    const uint64_t* rec = a.records + static_cast<uint64_t>(i) * REC_WORDS;
+    const uint64_t* rec = a.records + static_cast<uint64_t>(i) * (STAGE2 ? REC_WORDS_STAGE2 : REC_WORDS);
     key = rec[REC_KEY];
     const uint64_t flags = rec[REC_FLAGS];
+    if constexpr (STAGE2) {
+      const uint64_t nb = rec[REC_COUNT];
+      if (a.o_m2) {
+        if (!(flags & RF_HAS_M2)) s2_missing = true;
+        else if (nb) {
+          // the mean M2_b was taken around, computed as k_stage2_init computed it
+          const double mb = __longlong_as_double(static_cast<long long>(rec[a.vc == VC_F ? REC_SUM : REC_DSUM])) / static_cast<double>(nb);
+          const double m2b = __longlong_as_double(static_cast<long long>(rec[REC_M2]));
+          if (s2_n == 0) {
+            s2_mean = mb;
+            s2_m2 = m2b;
+          } else {
+            const double n = static_cast<double>(s2_n), n_b = static_cast<double>(nb), n2 = static_cast<double>(s2_n + nb);
+            const double delta = mb - s2_mean;
+            s2_m2 += m2b + delta * delta * n * n_b / n2;
+            s2_mean += delta * n_b / n2;
+          }
+          s2_n += nb;
+        }
+      }
+      if (a.o_prod) {
+        if (!(flags & RF_HAS_PROD)) s2_missing = true;
+        else if (nb) {
+          const uint64_t pb = rec[REC_PROD];
+          s2_prod = a.vc == VC_F ? static_cast<uint64_t>(__double_as_longlong(__longlong_as_double(static_cast<long long>(s2_prod)) *
+                                                                              __longlong_as_double(static_cast<long long>(pb))))
+                                 : s2_prod * pb;   // wraps, like the single-GPU product
+        }
+      }
+    }
     knull = flags & RF_KEY_NULL;
     if (a.vc == VC_F) fsum += __longlong_as_double(static_cast<long long>(rec[REC_SUM]));
     else sum += rec[REC_SUM];
@@ -321,7 +378,7 @@ __global__ void __launch_bounds__(256) k_merge_fold(MergeArgs a) {
   a.out.count[g] = static_cast<uint32_t>(cnt > 0xFFFFFFFFull ? 0xFFFFFFFFull : cnt);
   if (a.out.count64) a.out.count64[g] = cnt;
   a.out.first_row[g] = 0;
-  if (a.compact) {   // sum / mean / count only: nobody reads last rows, first / last values or min / max (22 B per group less)
+  if (!STAGE2 && a.words == REC_WORDS_COMPACT) {   // sum / mean / count only: nobody reads last rows, first / last values or min / max (22 B per group less)
     a.o_first_row_g[g] = first;
     return;
   }
@@ -333,6 +390,11 @@ __global__ void __launch_bounds__(256) k_merge_fold(MergeArgs a) {
   a.o_last_val[g] = lv;
   a.o_first_valid[g] = fvalid;
   a.o_last_valid[g] = lvalid;
+  if constexpr (STAGE2) {
+    if (a.o_m2) a.o_m2[g] = s2_m2;
+    if (a.o_prod) a.o_prod[g] = s2_prod;
+    if (s2_missing) atomicExch(a.status + ST_NO_TERMS, 1u);
+  }
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -5,6 +5,9 @@
       -> all-to-all of counts, then of records                   (torch.distributed: NCCL over NVLink)
       -> merge by key in source-rank order + order by global first row   (CUDA, pa_merge_create)
 
+Product / variance / stddev take the counted exchange with PA_PARTIAL_WORDS_STAGE2-word records, which also carry every
+shard's two-pass terms (M2 and product); the merge combines them in source-rank order.
+
 Each rank ends up owning the groups with hash(key) % world == rank; `gather_result` concatenates
 the owners' results on every rank and restores global first-appearance order.
 
@@ -17,7 +20,7 @@ from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 
-from ._lib import PA_PARTIAL_WORDS
+from ._lib import PA_AGG, PA_AGG_STAGE2, PA_PARTIAL_WORDS, PA_PARTIAL_WORDS_STAGE2
 
 REC_KEY, REC_FLAGS, REC_SUM, REC_DSUM, REC_COUNT, REC_FIRST_ROW = 0, 1, 2, 3, 4, 5
 
@@ -48,9 +51,10 @@ def owner_of(keys: np.ndarray, world: int, is_null: Optional[np.ndarray] = None)
     return o
 
 
-def exchange_records(send, send_counts: Sequence[int], group=None):
-    """All-to-all of fixed-size records.  `send`: int64 tensor [sum(send_counts), PA_PARTIAL_WORDS],
-    grouped by destination rank.  Returns (recv tensor grouped by source rank, recv_counts)."""
+def exchange_records(send, send_counts: Sequence[int], group=None, words: int = PA_PARTIAL_WORDS):
+    """All-to-all of fixed-size records.  `send`: int64 tensor [sum(send_counts), words] (PA_PARTIAL_WORDS, or
+    PA_PARTIAL_WORDS_STAGE2 for stage-2 records), grouped by destination rank.  Returns (recv tensor grouped by source
+    rank, recv_counts)."""
     import torch
     import torch.distributed as dist
     world = dist.get_world_size(group)
@@ -60,8 +64,8 @@ def exchange_records(send, send_counts: Sequence[int], group=None):
     rc = torch.empty(world, dtype=torch.int64, device=dev)
     dist.all_to_all_single(rc, sc, group=group)
     recv_counts = [int(x) for x in rc.tolist()]
-    recv = torch.empty((sum(recv_counts), PA_PARTIAL_WORDS), dtype=torch.int64, device=dev)
-    w = PA_PARTIAL_WORDS
+    recv = torch.empty((sum(recv_counts), words), dtype=torch.int64, device=dev)
+    w = words
     dist.all_to_all_single(recv.view(-1), send.reshape(-1), output_split_sizes=[c * w for c in recv_counts],
                            input_split_sizes=[int(c) * w for c in send_counts], group=group)
     return recv, recv_counts
@@ -165,6 +169,9 @@ def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_fo
     queued, so consecutive steps pipeline; the first call on the returned handle that needs a result completes
     it (and raises PaError if a rank had overflowed: rerun that step with wait=True).
 
+    product / variance / stddev in `aggs`: always the counted exchange (the padded blocks hold PA_PARTIAL_WORDS-word
+    records only), with stage-2 records.
+
     tail_stream (a torch.cuda.Stream, padded path only): the exchange and the merge run on it, behind an event recorded
     after the export — the handle's own stream is free for the next step's local pass while this step's records travel
     and merge (the serial tail is launch / NCCL latency on a handful of CTAs)."""
@@ -173,8 +180,10 @@ def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_fo
     from .groupby import MergedGroupBy, PaError
     world = dist.get_world_size(group)
     dev = torch.device("cuda", torch.cuda.current_device())
+    stage2 = any(PA_AGG[a] & PA_AGG_STAGE2 for a in aggs)
     if padded is None:
         padded = stream is not None and stream == torch.cuda.current_stream(dev).cuda_stream
+    padded = padded and not stage2
     # padded path: the local pass is only queued (no status read-back); export, exchange and merge are queued
     # behind it, so the host never waits before the merge's own result read.  A local pass that did not fit
     # the optimistic path makes the export send overflow markers, and everything is redone synchronously below.
@@ -206,9 +215,10 @@ def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_fo
                 raise
     counts = gb.partials_count(world)
     dev = torch.device("cuda", torch.cuda.current_device())
-    send = torch.empty((max(sum(counts), 1), PA_PARTIAL_WORDS), dtype=torch.int64, device=dev)
-    gb.partials_export(world, send.data_ptr(), send.shape[0])
-    recv, recv_counts = exchange_records(send[:sum(counts)], counts, group)
+    words = PA_PARTIAL_WORDS_STAGE2 if stage2 else PA_PARTIAL_WORDS
+    send = torch.empty((max(sum(counts), 1), words), dtype=torch.int64, device=dev)
+    gb.partials_export(world, send.data_ptr(), send.shape[0], stage2=stage2)
+    recv, recv_counts = exchange_records(send[:sum(counts)], counts, group, words=words)
     torch.cuda.synchronize()
     merged = MergedGroupBy(recv.data_ptr(), recv_counts, aggs, value_format, key_format, device=dev.index, stream=stream)
     merged._keep = (send, recv)

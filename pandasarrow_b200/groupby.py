@@ -334,8 +334,11 @@ class GroupBy:
         _check(self._L.pa_groupby_partials_count(self._h, n_parts, counts))
         return list(counts)
 
-    def partials_export(self, n_parts: int, records_ptr: int, capacity_records: int):
-        _check(self._L.pa_groupby_partials_export(self._h, n_parts, records_ptr, capacity_records))
+    def partials_export(self, n_parts: int, records_ptr: int, capacity_records: int, stage2: bool = False):
+        """stage2=True: PA_PARTIAL_WORDS_STAGE2-word records that also carry the product / variance terms of the last
+        aggregate (which must have computed product, variance or stddev); else PA_PARTIAL_WORDS-word records."""
+        fn = self._L.pa_groupby_partials_export_stage2 if stage2 else self._L.pa_groupby_partials_export
+        _check(fn(self._h, n_parts, records_ptr, capacity_records))
 
     def partials_export_padded(self, n_parts: int, blocks_ptr: int, block_records: int):
         _check(self._L.pa_groupby_partials_export_padded(self._h, n_parts, blocks_ptr, block_records))
