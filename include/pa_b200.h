@@ -116,7 +116,10 @@ struct ArrowDeviceArray {
 #define PA_AGG_BOOL_ALL 1024u     /* GroupBy::all: boolean ('b') value columns only; bool result, null for an all-null group */
 #define PA_AGG_BOOL_ANY 2048u     /* GroupBy::any */
 #define PA_AGG_COUNT_DISTINCT 4096u /* GroupBy::count_distinct: int64 number of distinct non-null values (by bit pattern, as
-                                      arrow's memo table: -0.0 and +0.0 are two values); single-GPU handles, < 2^31 rows */
+                                      arrow's memo table: -0.0 and +0.0 are two values); < 2^31 rows per handle.  Across
+                                      row-range shards through distinct-pair records (PA_DISTINCT_PAIR_WORDS) and
+                                      pa_merge_distinct_pairs, or in one pa_groupby_sharded_aggregate step; not in
+                                      pa_groupby_aggregate_chunked */
 
 /* ---- kernel path selection (pa_options.path); AUTO is what a caller wants ---- */
 #define PA_PATH_AUTO 0
@@ -318,12 +321,36 @@ int pa_groupby_partials_export(pa_groupby* g, int32_t n_parts, void* dev_records
 int pa_groupby_partials_export_stage2(pa_groupby* g, int32_t n_parts, void* dev_records, int64_t capacity_records);
 /* Joins received records (DEVICE memory, grouped by source rank; counts_by_source on the host) by key,
  * folds them in source-rank order and orders the groups by global first row.  The returned handle
- * answers num_groups / unique / fetch for the aggregates in agg_mask (PA_AGG_ALL and PA_AGG_STAGE2 bits).  The
+ * answers num_groups / unique / fetch for the aggregates in agg_mask (PA_AGG_ALL, PA_AGG_STAGE2, and with value_format
+ * "b" PA_AGG_BOOL_ALL / PA_AGG_BOOL_ANY bits: those merge the records' min / max and count).  The
  * records are PA_PARTIAL_WORDS_STAGE2 words wide exactly when agg_mask has a PA_AGG_STAGE2 bit (then PA_ERR_STATE if
  * a record lacks the terms asked for), PA_PARTIAL_WORDS otherwise.  value_format / key_format are
- * the Arrow format strings of the value and (single) key column. */
+ * the Arrow format strings of the value and (single) key column.  PA_AGG_COUNT_DISTINCT is not a record aggregate:
+ * see pa_merge_distinct_pairs. */
 int pa_merge_create(const void* dev_records, const int64_t* counts_by_source, int32_t n_sources, uint32_t agg_mask,
                     const char* value_format, const char* key_format, const pa_options* opt, pa_groupby** out);
+
+/* count_distinct across shards.  A per-group count does not merge (a value may occur on several shards), so every shard
+ * ships its distinct (key, value) pairs to the key's owner, which deduplicates across sources.  A distinct-pair record is
+ * PA_DISTINCT_PAIR_WORDS 64-bit words: [0] the key, [1] the value widened to 64 bits exactly as count_distinct compares
+ * it (-0.0 / +0.0 and NaNs with different payloads stay distinct), [2] flags, bit 0 = null key.  A handle whose last
+ * aggregate computed count_distinct keeps its D distinct pairs (12 bytes each; at most half of what that aggregate's
+ * sort needs) until the next aggregate or pa_groupby_destroy. */
+#define PA_DISTINCT_PAIR_WORDS 3
+/* Number of this handle's distinct pairs owned by each of n_parts ranks (1 <= n_parts <= 64), routed like the group
+ * records (the null key goes to rank 0).  PA_ERR_STATE when the last aggregate did not compute count_distinct or the
+ * handle is merged; composite and utf8 keys as pa_groupby_partials_count. */
+int pa_groupby_distinct_pairs_count(pa_groupby* g, int32_t n_parts, int64_t* counts_host);
+/* Writes the pairs, grouped by owner rank in ascending order, into caller-provided DEVICE memory (capacity_pairs >= sum of
+ * counts).  Must follow pa_groupby_distinct_pairs_count with the same n_parts. */
+int pa_groupby_distinct_pairs_export(pa_groupby* g, int32_t n_parts, void* dev_pairs, int64_t capacity_pairs);
+/* Adds a PA_AGG_COUNT_DISTINCT output (int64, the merged handle's group order, 0 for a group without pairs) to a handle
+ * made by pa_merge_create or pa_groupby_sharded_aggregate, from the received pairs (DEVICE memory, grouped by source;
+ * counts_by_source on the host; at most 2^32 - 2 in all).  A second call replaces the first.  The count is exact and
+ * does not depend on the order of arrival.  The owner-side set takes 32 bytes per received pair while the call runs.
+ * PA_ERR_STATE on a handle that is not merged, and when a pair names a key that no merged record carried (an
+ * inconsistent exchange). */
+int pa_merge_distinct_pairs(pa_groupby* merged, const void* dev_pairs, const int64_t* counts_by_source, int32_t n_sources);
 
 /* Low-latency variant for few groups — no host round trip before the collective.  Writes, for every
  * destination rank, a fixed-size block of (1 + block_records) records into caller-provided DEVICE memory
@@ -341,7 +368,8 @@ int pa_merge_create_padded(const void* dev_blocks, int32_t n_sources, int64_t bl
  * time — each chunk copied through the pinned staging pipeline, aggregated with row_base = its first row and exported as
  * partial records — and the chunks' records are merged like ranks' (sources folded in row order, groups in global
  * first-appearance order).  Single key column; sum / mean / count / min / max / first / last / product / variance / stddev
- * (those three travel in PA_PARTIAL_WORDS_STAGE2-word records).  `merged_out` answers
+ * (those three travel in PA_PARTIAL_WORDS_STAGE2-word records) and all / any of boolean columns; not count_distinct.
+ * `merged_out` answers
  * num_groups / unique / fetch like a merged multi-GPU handle.  At most 64 chunks. */
 int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const struct ArrowSchema* key_schema,
                                  const struct ArrowDeviceArray* values, const struct ArrowSchema* value_schema,
@@ -356,7 +384,10 @@ int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const stru
  * (ncclAllGather) and records (grouped ncclSend / ncclRecv), and the owner-side merge; `merged_out` answers
  * num_groups / unique / fetch / first_rows for the groups with hash(key) % world == rank.  Send / receive / merge
  * scratch stays on the communicator between steps.  Aggregates: PA_AGG_ALL and PA_AGG_STAGE2 bits (the latter travel in
- * PA_PARTIAL_WORDS_STAGE2-word records, see pa_groupby_partials_export_stage2). */
+ * PA_PARTIAL_WORDS_STAGE2-word records, see pa_groupby_partials_export_stage2), PA_AGG_BOOL_ALL / PA_AGG_BOOL_ANY
+ * (boolean columns), and PA_AGG_COUNT_DISTINCT: the pairs are counted per owner before the count gather, which carries
+ * both counts, travel in a second grouped send / receive after the records and are deduplicated on the merged handle
+ * (pa_merge_distinct_pairs); pair send / receive / set scratch stays on the communicator too. */
 #define PA_COMM_ID_BYTES 128
 typedef struct pa_comm pa_comm;
 int pa_comm_unique_id(void* out_id, int64_t capacity_bytes);
@@ -371,6 +402,9 @@ int pa_comm_last_phases(pa_comm* c, double phase_ms[5]);
  * count; 88: the full PA_PARTIAL_WORDS record; 104: the PA_PARTIAL_WORDS_STAGE2 record), whether the local pass handed over the bucketed path's unordered group
  * records without ordering them first (0 / 1), and the slots of the merge's join table. */
 int pa_comm_last_exchange(pa_comm* c, int32_t* record_bytes, int32_t* unordered_export, int64_t* merge_table_slots);
+/* The last step's count_distinct exchange: distinct pairs this rank sent and received, and the slots of its owner-side
+ * set (all 0 when the step computed no count_distinct). */
+int pa_comm_last_distinct(pa_comm* c, int64_t* pairs_sent, int64_t* pairs_received, int64_t* set_slots);
 
 /* ---- synthetic workload generator (SURVEY.md §8d), used by bench.py and the tests so that the
  * same counter-based splitmix64 streams exist on host and device without PCIe staging.

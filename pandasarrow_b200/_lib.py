@@ -17,6 +17,7 @@ PA_PATH_AUTO, PA_PATH_LOWCARD, PA_PATH_GLOBAL = 0, 1, 2
 PA_PARTIAL_WORDS = 11
 PA_PARTIAL_WORDS_STAGE2 = 13   # records that also carry the product / variance terms
 PA_AGG_STAGE2 = 128 | 256 | 512
+PA_DISTINCT_PAIR_WORDS = 3     # count_distinct across shards: (key, value bits, flags) records
 
 # every symbol include/pa_b200.h declares
 EXPORTS = [
@@ -27,9 +28,11 @@ EXPORTS = [
     "pa_groupby_sync",
     "pa_groupby_destroy", "pa_column_to_device", "pa_sort_create", "pa_sort_indices", "pa_resample_create", "pa_resample_create_calendar", "pa_downsample_create", "pa_groupby_partials_count", "pa_groupby_partials_export",
     "pa_groupby_partials_export_stage2",
+    "pa_groupby_distinct_pairs_count", "pa_groupby_distinct_pairs_export", "pa_merge_distinct_pairs",
     "pa_merge_create", "pa_groupby_aggregate_chunked", "pa_groupby_partials_export_padded", "pa_merge_create_padded", "pa_groupby_first_rows", "pa_synth_keys_i64", "pa_synth_vals_f64",
     "pa_synth_validity", "pa_synth_timestamps",
     "pa_comm_unique_id", "pa_comm_create", "pa_comm_adopt", "pa_comm_destroy", "pa_groupby_sharded_aggregate", "pa_comm_last_phases", "pa_comm_last_exchange",
+    "pa_comm_last_distinct",
 ]
 
 
@@ -132,6 +135,9 @@ def load():
     L.pa_groupby_partials_count.argtypes = [P, C.c_int32, C.POINTER(C.c_int64)]
     L.pa_groupby_partials_export.argtypes = [P, C.c_int32, P, C.c_int64]
     L.pa_groupby_partials_export_stage2.argtypes = [P, C.c_int32, P, C.c_int64]
+    L.pa_groupby_distinct_pairs_count.argtypes = [P, C.c_int32, C.POINTER(C.c_int64)]
+    L.pa_groupby_distinct_pairs_export.argtypes = [P, C.c_int32, P, C.c_int64]
+    L.pa_merge_distinct_pairs.argtypes = [P, P, C.POINTER(C.c_int64), C.c_int32]
     L.pa_merge_create.argtypes = [P, C.POINTER(C.c_int64), C.c_int32, C.c_uint32, C.c_char_p, C.c_char_p,
                                   C.POINTER(PaOptions), C.POINTER(P)]
     L.pa_groupby_aggregate_chunked.argtypes = [C.POINTER(ArrowDeviceArray), C.POINTER(ArrowSchema), C.POINTER(ArrowDeviceArray), C.POINTER(ArrowSchema),
@@ -147,6 +153,7 @@ def load():
     L.pa_groupby_sharded_aggregate.argtypes = [P, P, C.POINTER(ArrowDeviceArray), C.POINTER(ArrowSchema), C.c_uint32, C.POINTER(P)]
     L.pa_comm_last_phases.argtypes = [P, C.POINTER(C.c_double)]
     L.pa_comm_last_exchange.argtypes = [P, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int64)]
+    L.pa_comm_last_distinct.argtypes = [P, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
     L.pa_synth_keys_i64.argtypes = [P, C.c_int64, C.c_int64, C.c_uint64, C.c_uint64, P]
     L.pa_synth_vals_f64.argtypes = [P, C.c_int64, C.c_int64, C.c_uint64, P]
     L.pa_synth_validity.argtypes = [P, C.c_int64, C.c_int64, C.c_uint64, C.c_uint32, P]

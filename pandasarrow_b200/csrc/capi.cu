@@ -454,6 +454,13 @@ struct pa_groupby {
   // export (pa_groupby_partials_export_stage2); on a merged handle, the merged terms
   uint32_t s2_ext = 0;
   DevBuf s2_m2, s2_prod;
+  // count_distinct of the last aggregate: its distinct (local group id, value bits) pairs, cd_n of them, kept until the
+  // next aggregate for pa_groupby_distinct_pairs_export (12 bytes per pair)
+  bool cd_have = false;
+  uint64_t cd_n = 0;
+  DevBuf cd_id, cd_bits;
+  int dp_parts_n = 0;                     // pa_groupby_distinct_pairs_count: n_parts and the pairs per owner
+  std::vector<int64_t> dp_counts;
   bool last_wide = false;
   int last_vc = VC_I, last_vw = 8;
   std::string last_vfmt = "l";
@@ -1408,7 +1415,10 @@ int run_count_distinct(pa_groupby* g, const Column* val) {
   o.width = 8;
   o.nullable = false;
   PA_TRY(o.values.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
-  if (G == 0) return PA_OK;
+  if (G == 0) {
+    g->cd_have = true;   // (no pairs)
+    return PA_OK;
+  }
   DevBuf distinct, id_a, id_b, bits_a, bits_b, tmp;
   PA_TRY(distinct.alloc(static_cast<size_t>(G) * 8, st));
   CUDA_TRY(cudaMemsetAsync(distinct.p, 0, static_cast<size_t>(G) * 8, st));
@@ -1448,10 +1458,30 @@ int run_count_distinct(pa_groupby* g, const Column* val) {
     const int64_t threads = (n + CD_PER_THREAD - 1) / CD_PER_THREAD;
     k_distinct_count<<<static_cast<int>((threads + 255) / 256), 256, 0, st>>>(id_a.as<uint32_t>(), bits_a.as<uint64_t>(), n, distinct.as<unsigned long long>());
     CUDA_TRY(cudaGetLastError());
+    // the distinct pairs themselves, for the multi-GPU exchange: compacted into the sort's free buffers, then copied
+    // to buffers of their own size (12 bytes per pair: at most half of the 24 bytes per row the sort needs)
+    DevBuf cursor;
+    PA_TRY(cursor.alloc(8, st));
+    CUDA_TRY(cudaMemsetAsync(cursor.p, 0, 8, st));
+    k_distinct_pairs<<<static_cast<int>((threads + 255) / 256), 256, 0, st>>>(id_a.as<uint32_t>(), bits_a.as<uint64_t>(), n, id_b.as<uint32_t>(),
+                                                                           bits_b.as<uint64_t>(), cursor.as<unsigned long long>());
+    CUDA_TRY(cudaGetLastError());
+    unsigned long long d = 0;
+    CUDA_TRY(cudaMemcpyAsync(&d, cursor.p, 8, cudaMemcpyDeviceToHost, st));
+    id_a.reset(); bits_a.reset(); tmp.reset();
+    CUDA_TRY(cudaStreamSynchronize(st));
+    PA_TRY(g->cd_id.alloc(std::max<uint64_t>(d, 1) * 4, st));
+    PA_TRY(g->cd_bits.alloc(std::max<uint64_t>(d, 1) * 8, st));
+    if (d) {
+      CUDA_TRY(cudaMemcpyAsync(g->cd_id.p, id_b.p, d * 4, cudaMemcpyDeviceToDevice, st));
+      CUDA_TRY(cudaMemcpyAsync(g->cd_bits.p, bits_b.p, d * 8, cudaMemcpyDeviceToDevice, st));
+    }
+    g->cd_n = d;
   }
+  g->cd_have = true;
   k_distinct_emit<<<(G + 255) / 256, 256, 0, st>>>(distinct.as<unsigned long long>(), G, o.values.as<int64_t>());
   CUDA_TRY(cudaGetLastError());
-  g->last_launches += 5;
+  g->last_launches += 6;
   CUDA_TRY(cudaEventRecord(g->ev[4], st));
   return PA_OK;
 }
@@ -2035,6 +2065,11 @@ static int aggregate_entry(pa_groupby* g, const struct ArrowDeviceArray* values,
   // the stage-2 terms of an earlier aggregate do not belong to this one (run_stage2 sets them again)
   g->s2_ext = 0;
   if (!ext) { g->s2_m2.reset(); g->s2_prod.reset(); }
+  // ... nor do its distinct pairs (run_count_distinct keeps this one's)
+  g->cd_have = false;
+  g->cd_n = 0;
+  g->cd_id.reset(); g->cd_bits.reset();
+  g->dp_parts_n = 0;
   PA_TRY(aggregate_impl(g, &val, agg_mask, deferred));
   if (g->pending) return PA_OK;
   if (had && prev_G != g->G) return set_err(PA_ERR_STATE, "group count changed between passes (%u vs %u)", prev_G, g->G);
@@ -3004,6 +3039,84 @@ int pa_groupby_partials_export_stage2(pa_groupby* g, int32_t n_parts, void* dev_
   return partials_export(g, n_parts, dev_records, capacity_records, REC_WORDS_STAGE2);
 }
 
+// ---- count_distinct across shards: distinct-pair records (distinct.cuh) ----
+static_assert(DP_WORDS == PA_DISTINCT_PAIR_WORDS && DPF_KEY_NULL == 1, "public distinct-pair record");
+
+static int pairs_check(pa_groupby* g, int32_t n_parts) {
+  if (n_parts < 1 || n_parts > 64) return set_err(PA_ERR_INVALID, "bad argument (1 <= n_parts <= 64)");
+  PA_TRY(finish_pending(g));
+  if (g->merged) return set_err(PA_ERR_STATE, "distinct pairs come from a local aggregate, not from a merged handle");
+  if (g->keys.size() != 1 && !g->resample) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of composite keys");
+  if (!g->resample && g->keys[0].is_str) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of utf8 keys: dictionary-encode the column against a shared dictionary");
+  if (!g->cd_have) return set_err(PA_ERR_STATE, "the last aggregate computed no count_distinct: no distinct pairs to export");
+  return ensure_device(g);
+}
+
+static PairsArgs pairs_args(pa_groupby* g, int32_t n_parts) {
+  PairsArgs a{};
+  a.r = g->res;
+  a.id = g->cd_id.as<uint32_t>();
+  a.bits = g->cd_bits.as<uint64_t>();
+  a.n = g->cd_n;
+  a.nparts = static_cast<uint32_t>(n_parts);
+  return a;
+}
+
+// Stream ordered: pairs per owner added into d_counts[0 .. n_parts).
+static int pairs_count_async(pa_groupby* g, int32_t n_parts, unsigned long long* d_counts) {
+  PairsArgs a = pairs_args(g, n_parts);
+  a.counts = d_counts;
+  if (a.n) {
+    k_pairs_count<<<static_cast<unsigned>((a.n + 255) / 256), 256, 0, g->stream>>>(a);
+    CUDA_TRY(cudaGetLastError());
+  }
+  return PA_OK;
+}
+
+// The pairs grouped by owner (counts per owner as pa_groupby_distinct_pairs_count gave them); complete on return.
+static int pairs_export(pa_groupby* g, int32_t n_parts, const int64_t* counts, void* dev_pairs, DevBuf* d_cursor) {
+  cudaStream_t st = g->stream;
+  std::vector<uint64_t> prefix(static_cast<size_t>(n_parts), 0);
+  for (int i = 1; i < n_parts; ++i) prefix[i] = prefix[i - 1] + static_cast<uint64_t>(counts[i - 1]);
+  PA_TRY(d_cursor->alloc(sizeof(uint64_t) * n_parts, st));
+  CUDA_TRY(cudaMemcpyAsync(d_cursor->p, prefix.data(), sizeof(uint64_t) * n_parts, cudaMemcpyHostToDevice, st));
+  PairsArgs a = pairs_args(g, n_parts);
+  a.cursor = d_cursor->as<unsigned long long>();
+  a.out = static_cast<uint64_t*>(dev_pairs);
+  if (a.n) {
+    k_pairs_scatter<<<static_cast<unsigned>((a.n + 255) / 256), 256, 0, st>>>(a);
+    CUDA_TRY(cudaGetLastError());
+  }
+  CUDA_TRY(cudaStreamSynchronize(st));   // `prefix` dies here
+  return PA_OK;
+}
+
+int pa_groupby_distinct_pairs_count(pa_groupby* g, int32_t n_parts, int64_t* counts_host) {
+  if (!g || !counts_host) return set_err(PA_ERR_INVALID, "null argument");
+  PA_TRY(pairs_check(g, n_parts));
+  cudaStream_t st = g->stream;
+  DevBuf counts;
+  PA_TRY(counts.alloc(sizeof(uint64_t) * n_parts, st));
+  CUDA_TRY(cudaMemsetAsync(counts.p, 0, sizeof(uint64_t) * n_parts, st));
+  PA_TRY(pairs_count_async(g, n_parts, counts.as<unsigned long long>()));
+  std::vector<uint64_t> h(static_cast<size_t>(n_parts));
+  CUDA_TRY(cudaMemcpyAsync(h.data(), counts.p, sizeof(uint64_t) * n_parts, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaStreamSynchronize(st));
+  g->dp_parts_n = n_parts;
+  g->dp_counts.assign(h.begin(), h.end());
+  for (int i = 0; i < n_parts; ++i) counts_host[i] = static_cast<int64_t>(h[i]);
+  return PA_OK;
+}
+
+int pa_groupby_distinct_pairs_export(pa_groupby* g, int32_t n_parts, void* dev_pairs, int64_t capacity_pairs) {
+  if (!g || !dev_pairs) return set_err(PA_ERR_INVALID, "null argument");
+  PA_TRY(pairs_check(g, n_parts));
+  if (g->dp_parts_n != n_parts) return set_err(PA_ERR_STATE, "call pa_groupby_distinct_pairs_count(n_parts=%d) first", n_parts);
+  if (capacity_pairs < 0 || static_cast<uint64_t>(capacity_pairs) < g->cd_n) return set_err(PA_ERR_INVALID, "pair buffer too small");
+  DevBuf cursor;
+  return pairs_export(g, n_parts, g->dp_counts.data(), dev_pairs, &cursor);
+}
+
 // Common part of the two merge entry points.  `d_off` = device array [n_sources + 1], exclusive prefix
 // of the per-source record counts (the exact total is d_off[n_sources]); nrec_max = host-side upper bound.
 // Scratch of one merge (key table, per-source index, compaction / sort buffers).  A communicator keeps one between
@@ -3081,7 +3194,11 @@ static int merge_build(pa_groupby* g, const void* dev_records, const uint64_t* d
   }
   const uint32_t G = h_status[ST_COUNTER];
   g->G = G;
-  const bool wide = is_wide(agg_mask, g->last_vc);
+  // all / any: folded as min / max of the 0 / 1 bytes and the count, which is what k_emit_bool reads
+  const uint32_t extb = agg_mask & (PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY);
+  const uint32_t fold_mask = (agg_mask & (PA_AGG_ALL | PA_AGG_STAGE2)) |
+                             (extb ? (PA_AGG_COUNT | ((extb & PA_AGG_BOOL_ALL) ? PA_AGG_MIN : 0u) | ((extb & PA_AGG_BOOL_ANY) ? PA_AGG_MAX : 0u)) : 0u);
+  const bool wide = is_wide(fold_mask, g->last_vc);
   g->last_wide = wide;
   PA_TRY(alloc_result(g, G, true, true));
   PA_TRY(g->m_count64.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
@@ -3125,10 +3242,15 @@ static int merge_build(pa_groupby* g, const void* dev_records, const uint64_t* d
   g->have_groups = true;
   g->last_launches = 4;
   g->last_path = 4;
-  PA_TRY(run_emit(g, nullptr, agg_mask));
+  PA_TRY(run_emit(g, nullptr, fold_mask));
   if (ext) {
     PA_TRY(emit_stage2(g, g->last_vc, ext));
     g->last_launches += 1;
+  }
+  if (extb) {
+    // (the helper min / max / count outputs are bytes and counts nobody asked for)
+    g->outs.erase(std::remove_if(g->outs.begin(), g->outs.end(), [&](const AggOut& o) { return (o.bit & agg_mask) == 0; }), g->outs.end());
+    PA_TRY(run_bool_emit(g, extb));
   }
   CUDA_TRY(cudaEventRecord(g->ev[4], st));
   CUDA_TRY(cudaStreamSynchronize(st));   // local scratch (table, idx, sort buffers) is released after this point
@@ -3140,7 +3262,10 @@ static int merge_build(pa_groupby* g, const void* dev_records, const uint64_t* d
 int pa_merge_create(const void* dev_records, const int64_t* counts_by_source, int32_t n_sources, uint32_t agg_mask,
                     const char* value_format, const char* key_format, const pa_options* opt, pa_groupby** out) {
   if (!counts_by_source || n_sources < 1 || !value_format || !key_format || !out) return set_err(PA_ERR_INVALID, "null argument");
-  if (agg_mask & ~(PA_AGG_ALL | PA_AGG_STAGE2)) return set_err(PA_ERR_INVALID, "bad aggregate mask");
+  // (count_distinct does not travel in partial records: pa_merge_distinct_pairs adds it to the merged handle)
+  if (agg_mask & ~(PA_AGG_ALL | PA_AGG_STAGE2 | PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY)) return set_err(PA_ERR_INVALID, "bad aggregate mask");
+  if ((agg_mask & (PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY)) && strcmp(value_format, "b") != 0)
+    return set_err(PA_ERR_INVALID, "all / any need a boolean column (arrow::compute has no kernel for other types)");
   HandlePtr g(new pa_groupby());
   PA_TRY(handle_init(g.get(), opt));
   cudaStream_t st = g->stream;
@@ -3160,6 +3285,78 @@ int pa_merge_create(const void* dev_records, const int64_t* counts_by_source, in
                      static_cast<uint64_t>(*std::max_element(counts_by_source, counts_by_source + n_sources))));
   *out = g.release();
   return PA_OK;
+}
+
+// Owner-side count_distinct of a merged handle from n_pairs received distinct-pair records (any order): every pair is
+// mapped to its merged group through the key lookup table of build_row_lookup, inserted into a set of (bits, group) of
+// 2^k >= 2 n_pairs 16-byte slots (kept in *keep between calls when given), and counted when it was new.  Replaces an
+// earlier PA_AGG_COUNT_DISTINCT output.  `set_slots`: the set's size.
+static int merge_distinct(pa_groupby* g, const void* dev_pairs, uint64_t n_pairs, DevBuf* keep, uint64_t* set_slots) {
+  cudaStream_t st = g->stream;
+  const uint32_t G = g->G;
+  g->outs.erase(std::remove_if(g->outs.begin(), g->outs.end(), [](const AggOut& o) { return o.bit == PA_AGG_COUNT_DISTINCT; }), g->outs.end());
+  uint64_t cap = 1024;
+  while (cap < 2 * n_pairs) cap <<= 1;
+  DevBuf local_set, distinct, flag;
+  DevBuf& set = keep ? *keep : local_set;
+  PA_TRY(distinct.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
+  CUDA_TRY(cudaMemsetAsync(distinct.p, 0, static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
+  PA_TRY(flag.alloc(4, st));
+  CUDA_TRY(cudaMemsetAsync(flag.p, 0, 4, st));
+  RowLookup lk;
+  if (n_pairs) {
+    PA_TRY(set.alloc(cap * sizeof(DistinctSlot), st));
+    CUDA_TRY(cudaMemsetAsync(set.p, 0xFF, cap * sizeof(DistinctSlot), st));
+    PA_TRY(build_row_lookup(g, &lk));
+    DistinctMergeArgs a{};
+    a.ids = lk.a;
+    a.pairs = static_cast<const uint64_t*>(dev_pairs);
+    a.n = n_pairs;
+    a.set = set.as<DistinctSlot>();
+    a.cap_mask = cap - 1;
+    a.distinct = distinct.as<unsigned long long>();
+    a.G = G;
+    a.no_group = flag.as<uint32_t>();
+    const int grid = static_cast<int>(std::min<uint64_t>((n_pairs + DM_THREADS - 1) / DM_THREADS, static_cast<uint64_t>(g->num_sms) * 8));
+    if (G <= DM_SMEM_GROUPS) k_distinct_merge<true><<<grid, DM_THREADS, static_cast<size_t>(std::max<uint32_t>(G, 1)) * 4, st>>>(a);
+    else k_distinct_merge<false><<<grid, DM_THREADS, 0, st>>>(a);
+    CUDA_TRY(cudaGetLastError());
+  }
+  g->outs.emplace_back();
+  AggOut& o = g->outs.back();
+  o.bit = PA_AGG_COUNT_DISTINCT;
+  o.format = "l";
+  o.width = 8;
+  o.nullable = false;
+  PA_TRY(o.values.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
+  if (G) {
+    k_distinct_emit<<<(G + 255) / 256, 256, 0, st>>>(distinct.as<unsigned long long>(), G, o.values.as<int64_t>());
+    CUDA_TRY(cudaGetLastError());
+  }
+  uint32_t h_flag = 0;
+  CUDA_TRY(cudaMemcpyAsync(&h_flag, flag.p, 4, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaStreamSynchronize(st));   // the lookup table and the local set are released after this point
+  if (set_slots) *set_slots = n_pairs ? cap : 0;
+  if (h_flag) {
+    g->outs.pop_back();
+    return set_err(PA_ERR_STATE, "a distinct pair names a key that no merged record carried (inconsistent exchange)");
+  }
+  return PA_OK;
+}
+
+int pa_merge_distinct_pairs(pa_groupby* merged, const void* dev_pairs, const int64_t* counts_by_source, int32_t n_sources) {
+  if (!merged || !counts_by_source || n_sources < 1) return set_err(PA_ERR_INVALID, "null argument");
+  PA_TRY(finish_pending(merged));
+  if (!merged->merged || !merged->have_groups) return set_err(PA_ERR_STATE, "distinct pairs merge into a handle made by pa_merge_create");
+  uint64_t total = 0;
+  for (int i = 0; i < n_sources; ++i) {
+    if (counts_by_source[i] < 0) return set_err(PA_ERR_INVALID, "negative pair count");
+    total += static_cast<uint64_t>(counts_by_source[i]);
+  }
+  if (total > 0xFFFFFFFEull) return set_err(PA_ERR_INVALID, "more than 2^32 - 2 distinct pairs in one merge");
+  if (total && !dev_pairs) return set_err(PA_ERR_INVALID, "null pair buffer");
+  PA_TRY(ensure_device(merged));
+  return merge_distinct(merged, dev_pairs, total, nullptr, nullptr);
 }
 
 int pa_groupby_partials_export_padded(pa_groupby* g, int32_t n_parts, void* dev_blocks, int64_t block_records) {
@@ -3298,13 +3495,15 @@ int merge_padded_general(pa_groupby* g, const void* dev_blocks, int32_t n_source
 // columns is copied (staged, §h2d_copy), aggregated with row_base = its first row, and exported as partial records;
 // the owner-side merge then joins the chunks' records exactly as it joins ranks' — sources folded in chunk (= row)
 // order, groups ordered by global first row.  Device memory in use: one chunk of keys and values + the records.
-// Product / variance / stddev: every chunk's two-pass terms travel in stage-2 records (merge.cuh).
+// Product / variance / stddev: every chunk's two-pass terms travel in stage-2 records (merge.cuh).  All / any: in the
+// min / max words of the ordinary record.
 int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const struct ArrowSchema* key_schema,
                                  const struct ArrowDeviceArray* values, const struct ArrowSchema* value_schema,
                                  uint32_t agg_mask, int64_t chunk_rows, const pa_options* opt, pa_groupby** merged_out) {
   if (!keys || !key_schema || !values || !value_schema || !merged_out) return set_err(PA_ERR_INVALID, "null argument");
-  if (agg_mask == 0 || (agg_mask & ~(PA_AGG_ALL | PA_AGG_STAGE2)))
-    return set_err(PA_ERR_NOT_IMPLEMENTED, "chunked aggregates: sum / mean / count / min / max / first / last / product / variance / stddev");
+  if (agg_mask == 0 || (agg_mask & ~(PA_AGG_ALL | PA_AGG_STAGE2 | PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY)))
+    return set_err(PA_ERR_NOT_IMPLEMENTED, "chunked aggregates: sum / mean / count / min / max / first / last / product / variance / stddev / "
+                                           "all / any (count_distinct is not available across chunks)");
   const bool stage2 = (agg_mask & PA_AGG_STAGE2) != 0;
   const size_t RW = stage2 ? PA_PARTIAL_WORDS_STAGE2 : PA_PARTIAL_WORDS;
   if (keys->device_type == ARROW_DEVICE_CUDA || values->device_type == ARROW_DEVICE_CUDA)
@@ -3363,12 +3562,14 @@ struct pa_comm {
   int world = 1, rank = 0, device = 0;
   bool own = false;
   DevBuf send, recv, d_counts, d_all, d_cursor;     // kept between steps (grow only)
+  DevBuf psend, precv, pset;                        // count_distinct: distinct pairs sent / received, the owner's set
   MergeScratch merge;
   double phase_ms[5] = {0, 0, 0, 0, 0};   // last step: local pass, count + export, exchange, merge, total
   cudaEvent_t ev[6] = {};
   uint64_t h_bound = 0;                   // end of this rank's row shard (staging for the async copy)
   int last_record_bytes = 0, last_unordered = 0;   // pa_comm_last_exchange
   int64_t last_table_slots = 0;
+  int64_t last_pairs_sent = 0, last_pairs_received = 0, last_set_slots = 0;   // pa_comm_last_distinct
 };
 
 #define NCCL_TRY(expr)                                                                                          \
@@ -3388,8 +3589,8 @@ int pa_comm_unique_id(void* out_id, int64_t capacity_bytes) {
 static int comm_finish(pa_comm* c) {
   // The communicator outlives the handles (and their streams) it is used with: its scratch does not belong to any
   // stream's allocation order.
-  for (DevBuf* b : {&c->send, &c->recv, &c->d_counts, &c->d_all, &c->d_cursor, &c->merge.tkeys, &c->merge.idx, &c->merge.m_first, &c->merge.m_slot,
-                    &c->merge.s_first, &c->merge.s_slot, &c->merge.cub_tmp})
+  for (DevBuf* b : {&c->send, &c->recv, &c->d_counts, &c->d_all, &c->d_cursor, &c->psend, &c->precv, &c->pset, &c->merge.tkeys, &c->merge.idx,
+                    &c->merge.m_first, &c->merge.m_slot, &c->merge.s_first, &c->merge.s_slot, &c->merge.cub_tmp})
     b->plain = true;
   for (auto& e : c->ev) CUDA_TRY(cudaEventCreate(&e));
   return PA_OK;
@@ -3436,6 +3637,14 @@ int pa_comm_last_exchange(pa_comm* c, int32_t* record_bytes, int32_t* unordered_
   return PA_OK;
 }
 
+int pa_comm_last_distinct(pa_comm* c, int64_t* pairs_sent, int64_t* pairs_received, int64_t* set_slots) {
+  if (!c) return set_err(PA_ERR_INVALID, "null argument");
+  if (pairs_sent) *pairs_sent = c->last_pairs_sent;
+  if (pairs_received) *pairs_received = c->last_pairs_received;
+  if (set_slots) *set_slots = c->last_set_slots;
+  return PA_OK;
+}
+
 int pa_comm_last_phases(pa_comm* c, double phase_ms[5]) {
   if (!c || !phase_ms) return set_err(PA_ERR_INVALID, "null argument");
   for (int i = 0; i < 5; ++i) phase_ms[i] = c->phase_ms[i];
@@ -3448,8 +3657,9 @@ int pa_comm_last_phases(pa_comm* c, double phase_ms[5]) {
 int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDeviceArray* values,
                                  const struct ArrowSchema* value_schema, uint32_t agg_mask, pa_groupby** merged_out) {
   if (!g || !c || !values || !value_schema || !merged_out) return set_err(PA_ERR_INVALID, "null argument");
-  if (agg_mask == 0 || (agg_mask & ~(PA_AGG_ALL | PA_AGG_STAGE2)))
-    return set_err(PA_ERR_NOT_IMPLEMENTED, "sharded aggregates: sum / mean / count / min / max / first / last / product / variance / stddev");
+  if (agg_mask == 0 || (agg_mask & ~(PA_AGG_ALL | PA_AGG_STAGE2 | PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY | PA_AGG_COUNT_DISTINCT)))
+    return set_err(PA_ERR_NOT_IMPLEMENTED, "sharded aggregates: sum / mean / count / min / max / first / last / product / variance / stddev / "
+                                           "all / any / count_distinct");
   if (g->device != c->device) return set_err(PA_ERR_INVALID, "handle lives on device %d, communicator on %d", g->device, c->device);
   if (g->keys.size() != 1 && !g->resample) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of composite keys");
   if (!g->resample && g->keys[0].is_str) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of utf8 keys: dictionary-encode the column against a shared dictionary");
@@ -3460,11 +3670,15 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   // 1. local pass.  sum / mean of floats / count need one 32-byte sector per group (compact records, merge.cuh),
   // everything else the full record; with compact records the bucketed path may hand over its unordered group records
   // as they are (the merge orders by global first row anyway).  Product / variance / stddev: the local pass runs its
-  // second stage too, and the records carry its terms (REC_WORDS_STAGE2).
+  // second stage too, and the records carry its terms (REC_WORDS_STAGE2).  All / any travel in the full record's
+  // min / max words.  Count_distinct: the local pass keeps its distinct pairs, which take a second exchange to their
+  // owners (pairs are counted per owner with the records, exported in [1], sent in [2], deduplicated in [3]).
   int vw_ = 8, vc_ = VC_I;
   PA_TRY(parse_format(value_schema->format, &vw_, &vc_));
   const bool stage2 = (agg_mask & PA_AGG_STAGE2) != 0;
-  const bool compact = !stage2 && !is_wide(agg_mask, vc_) && !(agg_mask & (AGG_FIRST | AGG_LAST));
+  const bool distinct = (agg_mask & PA_AGG_COUNT_DISTINCT) != 0;
+  const bool full_only = stage2 || distinct || (agg_mask & (PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY));
+  const bool compact = !full_only && !is_wide(agg_mask, vc_) && !(agg_mask & (AGG_FIRST | AGG_LAST));
   g->want_unordered = compact && !g->resample;
   const int local_rc = aggregate_entry(g, values, value_schema, agg_mask, false);
   g->want_unordered = false;
@@ -3477,7 +3691,8 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   // 2. counts per owner, all ranks' counts to everybody
   // (every rank also tells the others where its row shard ends: the merge orders by GLOBAL first row and only has
   // to sort the bits below the largest one)
-  const int W1 = W + 1;
+  // (count_distinct: the W pair counts per owner follow, at [W + 1, 2 W + 1), in the same gather)
+  const int W1 = W + 1 + (distinct ? W : 0);
   PA_TRY(c->d_counts.alloc(sizeof(uint64_t) * W1, st));
   PA_TRY(c->d_all.alloc(sizeof(uint64_t) * W1 * W, st));
   CUDA_TRY(cudaMemsetAsync(c->d_counts.p, 0, sizeof(uint64_t) * W1, st));
@@ -3496,18 +3711,31 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
       CUDA_TRY(cudaGetLastError());
     }
   }
+  if (distinct) PA_TRY(pairs_count_async(g, W, c->d_counts.as<unsigned long long>() + W + 1));
   NCCL_TRY(ncclAllGather(c->d_counts.p, c->d_all.p, W1, ncclUint64, c->comm, st));
   std::vector<uint64_t> all(static_cast<size_t>(W1) * W);
   CUDA_TRY(cudaMemcpyAsync(all.data(), c->d_all.p, sizeof(uint64_t) * W1 * W, cudaMemcpyDeviceToHost, st));
   CUDA_TRY(cudaStreamSynchronize(st));
-  std::vector<int64_t> send_cnt(W), recv_cnt(W);
-  uint64_t send_total = 0, recv_total = 0, row_bound = 1;
+  std::vector<int64_t> send_cnt(W), recv_cnt(W), psend_cnt(W, 0), precv_cnt(W, 0);
+  uint64_t send_total = 0, recv_total = 0, row_bound = 1, psend_total = 0, precv_total = 0;
   for (int p = 0; p < W; ++p) {
     send_cnt[p] = static_cast<int64_t>(all[static_cast<size_t>(c->rank) * W1 + p]);
     recv_cnt[p] = static_cast<int64_t>(all[static_cast<size_t>(p) * W1 + c->rank]);
     send_total += send_cnt[p];
     recv_total += recv_cnt[p];
     row_bound = std::max(row_bound, all[static_cast<size_t>(p) * W1 + W]);
+    if (distinct) {
+      psend_cnt[p] = static_cast<int64_t>(all[static_cast<size_t>(c->rank) * W1 + W + 1 + p]);
+      precv_cnt[p] = static_cast<int64_t>(all[static_cast<size_t>(p) * W1 + W + 1 + c->rank]);
+      psend_total += psend_cnt[p];
+      precv_total += precv_cnt[p];
+    }
+  }
+  // (checked for every owner: every rank sees every count, so all ranks fail together before any record is sent)
+  for (int q = 0; distinct && q < W; ++q) {
+    uint64_t to_q = 0;
+    for (int p = 0; p < W; ++p) to_q += all[static_cast<size_t>(p) * W1 + W + 1 + q];
+    if (to_q > 0xFFFFFFFEull) return set_err(PA_ERR_INVALID, "rank %d would receive more than 2^32 - 2 distinct pairs in one merge", q);
   }
   // 3. export the records grouped by owner
   const int words = stage2 ? REC_WORDS_STAGE2 : rec_words(compact);
@@ -3530,6 +3758,12 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
     g->parts_counts.assign(send_cnt.begin(), send_cnt.end());
     PA_TRY(partials_export(g, W, c->send.p, static_cast<int64_t>(std::max<uint64_t>(send_total, g->G)), words));
   }
+  const size_t PW = DP_WORDS;
+  if (distinct) {
+    PA_TRY(c->psend.alloc(std::max<uint64_t>(psend_total, 1) * PW * 8, st));
+    PA_TRY(c->precv.alloc(std::max<uint64_t>(precv_total, 1) * PW * 8, st));
+    PA_TRY(pairs_export(g, W, psend_cnt.data(), c->psend.p, &c->d_cursor));
+  }
   CUDA_TRY(cudaEventRecord(c->ev[2], st));
   // 4. all-to-all of the records
   NCCL_TRY(ncclGroupStart());
@@ -3543,6 +3777,17 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
     }
   }
   NCCL_TRY(ncclGroupEnd());
+  if (distinct) {   // the distinct pairs, grouped by owner, in a second exchange
+    NCCL_TRY(ncclGroupStart());
+    uint64_t so = 0, ro = 0;
+    for (int p = 0; p < W; ++p) {
+      if (psend_cnt[p]) NCCL_TRY(ncclSend(c->psend.as<uint64_t>() + so * PW, static_cast<size_t>(psend_cnt[p]) * PW, ncclUint64, p, c->comm, st));
+      if (precv_cnt[p]) NCCL_TRY(ncclRecv(c->precv.as<uint64_t>() + ro * PW, static_cast<size_t>(precv_cnt[p]) * PW, ncclUint64, p, c->comm, st));
+      so += psend_cnt[p];
+      ro += precv_cnt[p];
+    }
+    NCCL_TRY(ncclGroupEnd());
+  }
   CUDA_TRY(cudaEventRecord(c->ev[3], st));
   // 5. owner-side merge
   const std::string kfmt = g->resample ? g->index_format : g->keys[0].format;
@@ -3559,8 +3804,10 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   CUDA_TRY(cudaMemcpyAsync(d_off.p, off.data(), sizeof(uint64_t) * (W + 1), cudaMemcpyHostToDevice, st));
   CUDA_TRY(cudaMemsetAsync(m->status.p, 0, sizeof(uint32_t) * ST_WORDS, st));
   CUDA_TRY(cudaEventRecord(m->ev[0], st));
-  PA_TRY(merge_build(m.get(), c->recv.p, d_off.as<uint64_t>(), W, recv_total, agg_mask, value_schema->format, kfmt.c_str(), &c->merge, row_bound, compact,
-                      static_cast<uint64_t>(*std::max_element(recv_cnt.begin(), recv_cnt.end()))));
+  PA_TRY(merge_build(m.get(), c->recv.p, d_off.as<uint64_t>(), W, recv_total, agg_mask & ~PA_AGG_COUNT_DISTINCT, value_schema->format, kfmt.c_str(),
+                     &c->merge, row_bound, compact, static_cast<uint64_t>(*std::max_element(recv_cnt.begin(), recv_cnt.end()))));
+  uint64_t set_slots = 0;
+  if (distinct) PA_TRY(merge_distinct(m.get(), c->precv.p, precv_total, &c->pset, &set_slots));
   CUDA_TRY(cudaEventRecord(c->ev[4], st));
   CUDA_TRY(cudaEventSynchronize(c->ev[4]));
   float t = 0;
@@ -3570,6 +3817,9 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   c->last_record_bytes = static_cast<int>(RW * 8);
   c->last_unordered = unordered ? 1 : 0;
   c->last_table_slots = static_cast<int64_t>(c->merge.last_slots);
+  c->last_pairs_sent = static_cast<int64_t>(psend_total);
+  c->last_pairs_received = static_cast<int64_t>(precv_total);
+  c->last_set_slots = static_cast<int64_t>(set_slots);
   *merged_out = m.release();
   return PA_OK;
 }

@@ -43,6 +43,23 @@ __global__ void __launch_bounds__(256) k_rowid_build(RowIdArgs a) {
   }
 }
 
+// Group id of a (non-null) key value, 0xFFFFFFFF if no group has it.
+__device__ __forceinline__ uint32_t key_lookup(const RowIdArgs& a, uint64_t key) {
+  if (key == kEmptyKey) return a.special[1];
+  uint64_t s = gtable_home(key, a.shift);
+  for (;;) {
+    const uint64_t k = __ldg(a.tkeys + s);
+    if (k == key) return __ldg(a.tranks + s);
+    if (k == kEmptyKey) return 0xFFFFFFFFu;
+    s = (s + 1) & a.cap_mask;
+  }
+}
+
+// Group id of a key given by value and null flag instead of by row (merge of distinct pairs, distinct.cuh).
+__device__ __forceinline__ uint32_t group_of_key(const RowIdArgs& a, uint64_t key, bool is_null) {
+  return is_null ? a.special[0] : key_lookup(a, key);
+}
+
 // Group id of row i (0xFFFFFFFF if its key was never aggregated — cannot happen for a finished handle).
 __device__ __forceinline__ uint32_t rowid_lookup(const RowIdArgs& a, int64_t i) {
   uint64_t key = load_key_rt(a.keys, i, a.kw);
@@ -55,14 +72,7 @@ __device__ __forceinline__ uint32_t rowid_lookup(const RowIdArgs& a, int64_t i) 
     if (b < 0) return 0xFFFFFFFFu;
     key = static_cast<uint64_t>(rs_label(a.rs, b));
   }
-  if (key == kEmptyKey) return a.special[1];
-  uint64_t s = gtable_home(key, a.shift);
-  for (;;) {
-    const uint64_t k = __ldg(a.tkeys + s);
-    if (k == key) return __ldg(a.tranks + s);
-    if (k == kEmptyKey) return 0xFFFFFFFFu;
-    s = (s + 1) & a.cap_mask;
-  }
+  return key_lookup(a, key);
 }
 
 __global__ void __launch_bounds__(256) k_rowid_scan(RowIdArgs a) {

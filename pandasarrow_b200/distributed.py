@@ -6,7 +6,9 @@
       -> merge by key in source-rank order + order by global first row   (CUDA, pa_merge_create)
 
 Product / variance / stddev take the counted exchange with PA_PARTIAL_WORDS_STAGE2-word records, which also carry every
-shard's two-pass terms (M2 and product); the merge combines them in source-rank order.
+shard's two-pass terms (M2 and product); the merge combines them in source-rank order.  All / any take the counted
+exchange too (min / max of the 0 / 1 values).  Count_distinct needs a second exchange: every shard's distinct
+(key, value) pairs, PA_DISTINCT_PAIR_WORDS words each, go to the key's owner, which counts them without duplicates.
 
 Each rank ends up owning the groups with hash(key) % world == rank; `gather_result` concatenates
 the owners' results on every rank and restores global first-appearance order.
@@ -20,7 +22,7 @@ from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 
-from ._lib import PA_AGG, PA_AGG_STAGE2, PA_PARTIAL_WORDS, PA_PARTIAL_WORDS_STAGE2
+from ._lib import PA_AGG, PA_AGG_STAGE2, PA_DISTINCT_PAIR_WORDS, PA_PARTIAL_WORDS, PA_PARTIAL_WORDS_STAGE2
 
 REC_KEY, REC_FLAGS, REC_SUM, REC_DSUM, REC_COUNT, REC_FIRST_ROW = 0, 1, 2, 3, 4, 5
 
@@ -52,8 +54,8 @@ def owner_of(keys: np.ndarray, world: int, is_null: Optional[np.ndarray] = None)
 
 
 def exchange_records(send, send_counts: Sequence[int], group=None, words: int = PA_PARTIAL_WORDS):
-    """All-to-all of fixed-size records.  `send`: int64 tensor [sum(send_counts), words] (PA_PARTIAL_WORDS, or
-    PA_PARTIAL_WORDS_STAGE2 for stage-2 records), grouped by destination rank.  Returns (recv tensor grouped by source
+    """All-to-all of fixed-size records.  `send`: int64 tensor [sum(send_counts), words] (PA_PARTIAL_WORDS,
+    PA_PARTIAL_WORDS_STAGE2 for stage-2 records, PA_DISTINCT_PAIR_WORDS for distinct pairs), grouped by destination rank.  Returns (recv tensor grouped by source
     rank, recv_counts)."""
     import torch
     import torch.distributed as dist
@@ -130,6 +132,14 @@ class Comm:
         _check(self._L.pa_comm_last_exchange(self._h, C.byref(rb), C.byref(un), C.byref(slots)))
         return {"record_bytes": rb.value, "unordered_export": bool(un.value), "merge_table_slots": slots.value}
 
+    def distinct_info(self) -> Dict[str, int]:
+        """count_distinct exchange of the last step (pa_comm_last_distinct); zeros when it computed none."""
+        import ctypes as C
+        from .groupby import _check
+        sent, recv, slots = C.c_int64(), C.c_int64(), C.c_int64()
+        _check(self._L.pa_comm_last_distinct(self._h, C.byref(sent), C.byref(recv), C.byref(slots)))
+        return {"pairs_sent": sent.value, "pairs_received": recv.value, "set_slots": slots.value}
+
     def close(self):
         if getattr(self, "_h", None) and self._h.value:
             self._L.pa_comm_destroy(self._h)
@@ -170,7 +180,9 @@ def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_fo
     it (and raises PaError if a rank had overflowed: rerun that step with wait=True).
 
     product / variance / stddev in `aggs`: always the counted exchange (the padded blocks hold PA_PARTIAL_WORDS-word
-    records only), with stage-2 records.
+    records only), with stage-2 records.  all / any / count_distinct: the counted exchange as well; count_distinct then
+    exchanges every shard's distinct pairs (exchange_records with words=PA_DISTINCT_PAIR_WORDS) and merges them into the
+    owner's handle.
 
     tail_stream (a torch.cuda.Stream, padded path only): the exchange and the merge run on it, behind an event recorded
     after the export — the handle's own stream is free for the next step's local pass while this step's records travel
@@ -181,9 +193,10 @@ def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_fo
     world = dist.get_world_size(group)
     dev = torch.device("cuda", torch.cuda.current_device())
     stage2 = any(PA_AGG[a] & PA_AGG_STAGE2 for a in aggs)
+    distinct = "count_distinct" in aggs
     if padded is None:
         padded = stream is not None and stream == torch.cuda.current_stream(dev).cuda_stream
-    padded = padded and not stage2
+    padded = padded and not stage2 and not any(a in ("all", "any", "count_distinct") for a in aggs)
     # padded path: the local pass is only queued (no status read-back); export, exchange and merge are queued
     # behind it, so the host never waits before the merge's own result read.  A local pass that did not fit
     # the optimistic path makes the export send overflow markers, and everything is redone synchronously below.
@@ -220,8 +233,16 @@ def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_fo
     gb.partials_export(world, send.data_ptr(), send.shape[0], stage2=stage2)
     recv, recv_counts = exchange_records(send[:sum(counts)], counts, group, words=words)
     torch.cuda.synchronize()
-    merged = MergedGroupBy(recv.data_ptr(), recv_counts, aggs, value_format, key_format, device=dev.index, stream=stream)
+    merged = MergedGroupBy(recv.data_ptr(), recv_counts, [a for a in aggs if a != "count_distinct"], value_format, key_format,
+                           device=dev.index, stream=stream)
     merged._keep = (send, recv)
+    if distinct:
+        pcounts = gb.distinct_pairs_count(world)
+        psend = torch.empty((max(sum(pcounts), 1), PA_DISTINCT_PAIR_WORDS), dtype=torch.int64, device=dev)
+        gb.distinct_pairs_export(world, psend.data_ptr(), psend.shape[0])
+        precv, precv_counts = exchange_records(psend[:sum(pcounts)], pcounts, group, words=PA_DISTINCT_PAIR_WORDS)
+        torch.cuda.synchronize()
+        merged.merge_distinct_pairs(precv.data_ptr(), precv_counts)
     return merged
 
 

@@ -343,6 +343,17 @@ class GroupBy:
     def partials_export_padded(self, n_parts: int, blocks_ptr: int, block_records: int):
         _check(self._L.pa_groupby_partials_export_padded(self._h, n_parts, blocks_ptr, block_records))
 
+    def distinct_pairs_count(self, n_parts: int) -> List[int]:
+        """count_distinct across shards: this handle's distinct (key, value) pairs owned by each of n_parts ranks (the
+        last aggregate must have computed count_distinct)."""
+        counts = (C.c_int64 * n_parts)()
+        _check(self._L.pa_groupby_distinct_pairs_count(self._h, n_parts, counts))
+        return list(counts)
+
+    def distinct_pairs_export(self, n_parts: int, pairs_ptr: int, capacity_pairs: int):
+        """PA_DISTINCT_PAIR_WORDS-word pair records, grouped by owner, into device memory (after distinct_pairs_count)."""
+        _check(self._L.pa_groupby_distinct_pairs_export(self._h, n_parts, pairs_ptr, capacity_pairs))
+
     def timing(self) -> dict:
         total = C.c_double()
         st = (C.c_double * 4)()
@@ -419,6 +430,11 @@ class MergedGroupBy(GroupBy):
         counts = (C.c_int64 * len(counts_by_source))(*[int(c) for c in counts_by_source])
         _check(self._L.pa_merge_create(records_ptr, counts, len(counts_by_source), mask, value_format.encode(),
                                        key_format.encode(), C.byref(opt), C.byref(self._h)))
+
+    def merge_distinct_pairs(self, pairs_ptr: int, counts_by_source: Sequence[int]):
+        """Adds count_distinct (fetch("count_distinct")) from the received distinct-pair records, grouped by source."""
+        counts = (C.c_int64 * len(counts_by_source))(*[int(c) for c in counts_by_source])
+        _check(self._L.pa_merge_distinct_pairs(self._h, pairs_ptr, counts, len(counts_by_source)))
 
 
 def _merged_from_handle(h) -> "MergedGroupBy":
