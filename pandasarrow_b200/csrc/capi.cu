@@ -1402,6 +1402,25 @@ int run_bool_emit(pa_groupby* g, uint32_t extb) {
   return PA_OK;
 }
 
+// all / any: the aggregates k_emit_bool reads (min / max of the 0 / 1 bytes, and the count)
+uint32_t bool_helper_mask(uint32_t extb) {
+  return extb ? (PA_AGG_COUNT | ((extb & PA_AGG_BOOL_ALL) ? PA_AGG_MIN : 0u) | ((extb & PA_AGG_BOOL_ANY) ? PA_AGG_MAX : 0u)) : 0u;
+}
+
+void keep_outputs(pa_groupby* g, uint32_t mask) {   // drops the outputs whose bit is not in `mask`
+  g->outs.erase(std::remove_if(g->outs.begin(), g->outs.end(), [&](const AggOut& o) { return (o.bit & mask) == 0; }), g->outs.end());
+}
+
+// Aggregates the local pass, partial records (pa_merge_create, chunked) and the sharded step (records + distinct pairs) take
+constexpr uint32_t LOCAL_AGGS = PA_AGG_ALL | PA_AGG_STAGE2 | PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY | PA_AGG_COUNT_DISTINCT;
+constexpr uint32_t RECORD_AGGS = PA_AGG_ALL | PA_AGG_STAGE2 | PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY;
+constexpr uint32_t SHARDED_AGGS = RECORD_AGGS | PA_AGG_COUNT_DISTINCT;
+
+// Partial-record width (merge.cuh) of an aggregate set; `compact`: the sharded step's one-sector record
+int record_words(uint32_t agg_mask, bool compact) {
+  return compact ? REC_WORDS_COMPACT : ((agg_mask & PA_AGG_STAGE2) ? REC_WORDS_STAGE2 : REC_WORDS);
+}
+
 // count_distinct (distinct.cuh): ids + value bits -> two stable radix sorts -> boundary count.  Appends to g->outs.
 int run_count_distinct(pa_groupby* g, const Column* val) {
   cudaStream_t st = g->stream;
@@ -1705,11 +1724,195 @@ int aggregate_impl_raw(pa_groupby* g, const Column* val, uint32_t mask, bool def
   return PA_OK;
 }
 
+// ---- owner-side merge of partial records (merge.cuh) ----
+int set_merged_formats(pa_groupby* g, const char* value_format, const char* key_format) {
+  g->merged = true;
+  g->keys.resize(1);
+  int kw = 8, kvc = VC_I;
+  PA_TRY(parse_format(key_format, &kw, &kvc));
+  g->keys[0].format = key_format;
+  g->keys[0].width = kw;
+  g->fields.assign(1, KeyField{});
+  g->fields[0].width = kw;
+  g->index_format = key_format;
+  PA_TRY(parse_format(value_format, &g->last_vw, &g->last_vc));
+  g->last_vfmt = value_format;
+  return PA_OK;
+}
+
+// GroupResult and fold outputs (64-bit counts, first / last values, global first rows) for `cap` groups, as outputs of `a`
+template <typename Args>
+int alloc_merged_result(pa_groupby* g, uint32_t cap, Args* a) {
+  cudaStream_t st = g->stream;
+  PA_TRY(alloc_result(g, cap, true, true));
+  const size_t n = std::max<uint32_t>(cap, 1);
+  PA_TRY(g->m_count64.alloc(n * 8, st));
+  g->res.count64 = g->m_count64.as<uint64_t>();
+  PA_TRY(g->m_first_val.alloc(n * 8, st));
+  PA_TRY(g->m_first_row_g.alloc(n * 8, st));
+  PA_TRY(g->m_last_val.alloc(n * 8, st));
+  PA_TRY(g->m_first_valid.alloc(n, st));
+  PA_TRY(g->m_last_valid.alloc(n, st));
+  a->out = g->res;
+  a->o_first_val = g->m_first_val.as<uint64_t>(); a->o_last_val = g->m_last_val.as<uint64_t>();
+  a->o_first_valid = g->m_first_valid.as<uint8_t>(); a->o_last_valid = g->m_last_valid.as<uint8_t>();
+  a->o_first_row_g = g->m_first_row_g.as<uint64_t>();
+  return PA_OK;
+}
+
+// Scratch of one merge (key table, per-source index, compaction / sort buffers).  A communicator keeps one between
+// steps (pa_groupby_sharded_aggregate) so that a step allocates nothing but its result.
+struct MergeScratch { DevBuf tkeys, idx, m_first, m_slot, s_first, s_slot, cub_tmp; uint64_t last_slots = 0; };
+
+// Common part of the merge entry points.  `d_off` = device array [n_sources + 1], exclusive prefix
+// of the per-source record counts (the exact total is d_off[n_sources]); nrec_max = host-side upper bound.
+int merge_build(pa_groupby* g, const void* dev_records, const uint64_t* d_off, int32_t n_sources, uint64_t nrec_max,
+                uint32_t agg_mask, const char* value_format, const char* key_format, MergeScratch* keep = nullptr,
+                uint64_t row_bound = 0, bool compact = false, uint64_t distinct_hint = 0) {
+  cudaStream_t st = g->stream;
+  PA_TRY(set_merged_formats(g, value_format, key_format));
+  if (nrec_max >= 0xFFFFFFFFull) return set_err(PA_ERR_NOT_IMPLEMENTED, "more than 2^32-1 partial records per rank");
+  MergeScratch local_scratch;
+  MergeScratch& ms = keep ? *keep : local_scratch;
+  DevBuf &tkeys = ms.tkeys, &idx = ms.idx, &m_first = ms.m_first, &m_slot = ms.m_slot, &s_first = ms.s_first, &s_slot = ms.s_slot, &cub_tmp = ms.cub_tmp;
+  PA_TRY(m_first.alloc(std::max<uint64_t>(nrec_max, 1) * 8, st));
+  PA_TRY(m_slot.alloc(std::max<uint64_t>(nrec_max, 1) * 4, st));
+  MergeArgs a{};
+  a.records = static_cast<const uint64_t*>(dev_records);
+  a.src_offset = d_off;
+  const uint32_t ext = agg_mask & PA_AGG_STAGE2;
+  a.nsrc = n_sources; a.nrec = nrec_max;
+  a.words = record_words(agg_mask, compact);
+  a.status = g->status.as<uint32_t>();
+  a.m_first_row = m_first.as<uint64_t>(); a.m_slot = m_slot.as<uint32_t>();
+  a.vc = g->last_vc;
+  // Join table: 2^k >= 2 x the number of distinct keys.  A source holds every key at most once, so the count lies
+  // between the largest source and the sum; sources that saw (nearly) the same keys — row-range shards of one column —
+  // are the common case, so the table is sized by `distinct_hint` (the largest source; 0 = unknown) first: 8 sources of
+  // 12.5 M records fill 2^25 slots instead of 2^28 (index array 1 GB instead of 8.6 GB per step).  Too small shows as a
+  // probe sequence beyond max_probe; then the merge is redone with the table every key set fits.
+  uint32_t h_status[ST_WORDS];
+  uint64_t sized_for = distinct_hint ? std::min<uint64_t>(std::max<uint64_t>(distinct_hint + distinct_hint / 4, 512), std::max<uint64_t>(nrec_max, 512)) : std::max<uint64_t>(nrec_max, 512);
+  for (;;) {
+    uint64_t cap = 1024;
+    while (cap < sized_for * 2) cap <<= 1;
+    const uint64_t nslots = cap + 2;
+    ms.last_slots = nslots;
+    PA_TRY(tkeys.alloc(nslots * 8, st));
+    PA_TRY(idx.alloc(nslots * n_sources * 4, st));
+    const int fgrid = static_cast<int>(std::min<uint64_t>((nslots + 255) / 256, static_cast<uint64_t>(g->num_sms) * 16));
+    k_fill_u64<<<fgrid, 256, 0, st>>>(tkeys.as<unsigned long long>(), nslots, kEmptyKey);
+    CUDA_TRY(cudaMemsetAsync(idx.p, 0xFF, nslots * n_sources * 4, st));
+    a.tkeys = tkeys.as<unsigned long long>(); a.cap_mask = cap - 1; a.idx = idx.as<uint32_t>();
+    a.max_probe = sized_for >= nrec_max ? cap : std::min<uint64_t>(cap, 2048);
+    CUDA_TRY(cudaEventRecord(g->ev[1], st));
+    if (nrec_max) {
+      k_merge_insert<<<static_cast<int>((nrec_max + 255) / 256), 256, 0, st>>>(a);
+      CUDA_TRY(cudaGetLastError());
+    }
+    k_merge_compact<<<static_cast<int>((nslots + MC_THREADS - 1) / MC_THREADS), MC_THREADS, 0, st>>>(a);
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaEventRecord(g->ev[2], st));
+    CUDA_TRY(cudaMemcpyAsync(h_status, g->status.p, sizeof h_status, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    if (h_status[ST_PEER_OVERFLOW]) return set_err(PA_ERR_STATE, "a source rank had more groups than a padded block holds; use the counted exchange");
+    if (h_status[ST_OVERFLOW] && sized_for < nrec_max) {   // the hint was too small: every key set fits a table sized by the record count
+      sized_for = nrec_max;
+      CUDA_TRY(cudaMemsetAsync(a.status + ST_OVERFLOW, 0, sizeof(uint32_t), st));
+      CUDA_TRY(cudaMemsetAsync(a.status + ST_COUNTER, 0, sizeof(uint32_t), st));
+      continue;
+    }
+    if (h_status[ST_OVERFLOW]) return set_err(PA_ERR_CUDA, "merge table overflow");
+    break;
+  }
+  const uint32_t G = h_status[ST_COUNTER];
+  g->G = G;
+  // all / any: folded as min / max of the 0 / 1 bytes and the count, which is what k_emit_bool reads
+  const uint32_t extb = agg_mask & (PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY);
+  const uint32_t fold_mask = (agg_mask & (PA_AGG_ALL | PA_AGG_STAGE2)) | bool_helper_mask(extb);
+  const bool wide = is_wide(fold_mask, g->last_vc);
+  g->last_wide = wide;
+  PA_TRY(alloc_merged_result(g, G, &a));
+  if (ext & (AGG_VARIANCE | AGG_STDDEV)) PA_TRY(g->s2_m2.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
+  if (ext & AGG_PRODUCT) PA_TRY(g->s2_prod.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
+  uint32_t h_no_terms = 0;
+  if (G) {
+    PA_TRY(s_first.alloc(static_cast<size_t>(G) * 8, st));
+    PA_TRY(s_slot.alloc(static_cast<size_t>(G) * 4, st));
+    size_t tmp_bytes = 0;
+    // (global first rows are below row_bound when the caller knows the shards: sort only the bits that can differ)
+    int end_bit = 64;
+    if (row_bound) { end_bit = 1; while (end_bit < 64 && (row_bound >> end_bit)) ++end_bit; }
+    CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, m_first.as<uint64_t>(), s_first.as<uint64_t>(), m_slot.as<uint32_t>(), s_slot.as<uint32_t>(), static_cast<int>(G), 0, end_bit, st));
+    PA_TRY(cub_tmp.alloc(tmp_bytes, st));
+    CUDA_TRY(cub::DeviceRadixSort::SortPairs(cub_tmp.p, tmp_bytes, m_first.as<uint64_t>(), s_first.as<uint64_t>(), m_slot.as<uint32_t>(), s_slot.as<uint32_t>(), static_cast<int>(G), 0, end_bit, st));
+    a.order = s_slot.as<uint32_t>();
+    a.G = G;
+    if (ext) {
+      a.o_m2 = (ext & (AGG_VARIANCE | AGG_STDDEV)) ? g->s2_m2.as<double>() : nullptr;
+      a.o_prod = (ext & AGG_PRODUCT) ? g->s2_prod.as<unsigned long long>() : nullptr;
+      k_merge_fold<true><<<(G + 255) / 256, 256, 0, st>>>(a);
+      CUDA_TRY(cudaGetLastError());
+      CUDA_TRY(cudaMemcpyAsync(&h_no_terms, a.status + ST_NO_TERMS, sizeof h_no_terms, cudaMemcpyDeviceToHost, st));
+    } else {
+      k_merge_fold<false><<<(G + 255) / 256, 256, 0, st>>>(a);
+      CUDA_TRY(cudaGetLastError());
+    }
+  }
+  CUDA_TRY(cudaEventRecord(g->ev[3], st));
+  g->have_groups = true;
+  g->last_launches = 4;
+  g->last_path = 4;
+  PA_TRY(run_emit(g, nullptr, fold_mask));
+  if (ext) {
+    PA_TRY(emit_stage2(g, g->last_vc, ext));
+    g->last_launches += 1;
+  }
+  if (extb) {
+    // (the helper min / max / count outputs are bytes and counts nobody asked for)
+    keep_outputs(g, agg_mask);
+    PA_TRY(run_bool_emit(g, extb));
+  }
+  CUDA_TRY(cudaEventRecord(g->ev[4], st));
+  CUDA_TRY(cudaStreamSynchronize(st));   // local scratch (table, idx, sort buffers) is released after this point
+  if (h_no_terms) return set_err(PA_ERR_STATE, "partial records carry no variance / product terms for this aggregate mask "
+                                               "(export them with pa_groupby_partials_export_stage2 after an aggregate that computes them)");
+  return PA_OK;
+}
+
+// Merge of records whose per-source counts the host knows: offsets to the device, the table sized by the largest source.
+int merge_counted(pa_groupby* g, const void* dev_records, const int64_t* counts, int32_t n_sources, uint32_t agg_mask,
+                  const char* value_format, const char* key_format, MergeScratch* keep, uint64_t row_bound, bool compact) {
+  cudaStream_t st = g->stream;
+  std::vector<uint64_t> off(n_sources + 1, 0);
+  for (int i = 0; i < n_sources; ++i) off[i + 1] = off[i] + static_cast<uint64_t>(counts[i]);
+  if (off[n_sources] && !dev_records) return set_err(PA_ERR_INVALID, "null record buffer");
+  DevBuf d_off;
+  PA_TRY(d_off.alloc(sizeof(uint64_t) * (n_sources + 1), st));
+  CUDA_TRY(cudaMemcpyAsync(d_off.p, off.data(), sizeof(uint64_t) * (n_sources + 1), cudaMemcpyHostToDevice, st));
+  CUDA_TRY(cudaMemsetAsync(g->status.p, 0, sizeof(uint32_t) * ST_WORDS, st));
+  CUDA_TRY(cudaEventRecord(g->ev[0], st));
+  return merge_build(g, dev_records, d_off.as<uint64_t>(), n_sources, off[n_sources], agg_mask, value_format, key_format, keep,
+                     row_bound, compact, static_cast<uint64_t>(*std::max_element(counts, counts + n_sources)));
+}
+
+int merge_padded_general(pa_groupby* g, const void* dev_blocks, int32_t n_sources, int64_t block_records, uint32_t agg_mask,
+                         const char* value_format, const char* key_format) {
+  cudaStream_t st = g->stream;
+  const uint64_t nrec_max = static_cast<uint64_t>(n_sources) * static_cast<uint64_t>(block_records);
+  DevBuf d_off, records;
+  PA_TRY(d_off.alloc(sizeof(uint64_t) * (n_sources + 1), st));
+  PA_TRY(records.alloc(nrec_max * PA_PARTIAL_WORDS * 8, st));
+  CUDA_TRY(cudaMemsetAsync(g->status.p, 0, sizeof(uint32_t) * ST_WORDS, st));
+  k_merge_unpad<<<n_sources, 256, 0, st>>>(static_cast<const uint64_t*>(dev_blocks), static_cast<uint32_t>(n_sources),
+                                           static_cast<uint64_t>(block_records), records.as<uint64_t>(), d_off.as<uint64_t>(),
+                                           g->status.as<uint32_t>());
+  CUDA_TRY(cudaGetLastError());
+  return merge_build(g, records.p, d_off.as<uint64_t>(), n_sources, nrec_max, agg_mask, value_format, key_format);
+}
+
 // Completes a deferred aggregate: reads the status words; on success only the group count was missing, otherwise
 // the pass is redone synchronously from the stage that failed.
-int merge_padded_general(pa_groupby* g, const void* dev_blocks, int32_t n_sources, int64_t block_records, uint32_t agg_mask,
-                         const char* value_format, const char* key_format);
-
 int finish_pending(pa_groupby* g) {
   if (g->pending_merge) {
     g->pending_merge = false;
@@ -2013,7 +2216,7 @@ int pa_groupby_unique(pa_groupby* g, int32_t key_i, struct ArrowArray* out, stru
 static int aggregate_entry(pa_groupby* g, const struct ArrowDeviceArray* values, const struct ArrowSchema* value_schema,
                            uint32_t agg_mask, bool deferred) {
   if (!g || !values || !value_schema) return set_err(PA_ERR_INVALID, "null argument");
-  if (agg_mask == 0 || (agg_mask & ~(PA_AGG_ALL | PA_AGG_STAGE2 | PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY | PA_AGG_COUNT_DISTINCT))) return set_err(PA_ERR_INVALID, "bad aggregate mask 0x%x", agg_mask);
+  if (agg_mask == 0 || (agg_mask & ~LOCAL_AGGS)) return set_err(PA_ERR_INVALID, "bad aggregate mask 0x%x", agg_mask);
   const uint32_t requested = agg_mask;
   const uint32_t extb = agg_mask & (PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY);
   const bool want_distinct = (agg_mask & PA_AGG_COUNT_DISTINCT) != 0;
@@ -2025,8 +2228,7 @@ static int aggregate_entry(pa_groupby* g, const struct ArrowDeviceArray* values,
   if (ext || extb || want_distinct) {
     deferred = false;
     // all = (min over the 0 / 1 bytes) != 0, any = (max) != 0: the ordinary pass delivers both
-    agg_mask = (agg_mask & PA_AGG_ALL) | PA_AGG_COUNT | ((ext & (PA_AGG_VARIANCE | PA_AGG_STDDEV)) ? PA_AGG_MEAN : 0u) |
-               ((extb & PA_AGG_BOOL_ALL) ? PA_AGG_MIN : 0u) | ((extb & PA_AGG_BOOL_ANY) ? PA_AGG_MAX : 0u);
+    agg_mask = (agg_mask & PA_AGG_ALL) | PA_AGG_COUNT | ((ext & (PA_AGG_VARIANCE | PA_AGG_STDDEV)) ? PA_AGG_MEAN : 0u) | bool_helper_mask(extb);
   }
   PA_TRY(ensure_device(g));
   Column val;
@@ -2077,7 +2279,7 @@ static int aggregate_entry(pa_groupby* g, const struct ArrowDeviceArray* values,
   if (want_distinct) PA_TRY(run_count_distinct(g, &val));
   if (val.is_bool) {
     // the helper min / max columns are bytes, not Arrow booleans: only what was asked for stays fetchable
-    g->outs.erase(std::remove_if(g->outs.begin(), g->outs.end(), [&](const AggOut& o) { return (o.bit & requested) == 0; }), g->outs.end());
+    keep_outputs(g, requested);
     if (extb) PA_TRY(run_bool_emit(g, extb));
   }
   // `val` may own device copies of host data: make sure the kernels reading them are done
@@ -2963,29 +3165,68 @@ int pa_sort_indices(pa_groupby* g, struct ArrowArray* out, struct ArrowSchema* o
 }
 
 // ---- multi-GPU partial export / merge ----
-int pa_groupby_partials_count(pa_groupby* g, int32_t n_parts, int64_t* counts_host) {
-  if (!g || !counts_host || n_parts < 1 || n_parts > 64) return set_err(PA_ERR_INVALID, "bad argument (1 <= n_parts <= 64)");
-  PA_TRY(finish_pending(g));
-  if (!g->have_groups || g->merged) return set_err(PA_ERR_STATE, "partials need a finished local aggregate");
+static int check_shardable(const pa_groupby* g) {   // keys the exchange routes: one fixed-width column or a resample index
   if (g->keys.size() != 1 && !g->resample) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of composite keys");
   if (!g->resample && g->keys[0].is_str) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of utf8 keys: dictionary-encode the column against a shared dictionary");
-  PA_TRY(ensure_device(g));
+  return PA_OK;
+}
+
+// The groups of the last aggregate and the values its records carry (records of any width)
+static PartialsArgs partials_args(pa_groupby* g, int32_t n_parts) {
+  PartialsArgs a{};
+  a.r = g->res; a.G = g->G; a.nparts = n_parts; a.row_base = g->opt.row_base;
+  a.vw = g->last_vw; a.wide = g->last_wide;
+  for (auto& o : g->outs) {
+    if (o.bit == AGG_FIRST) { a.first_vals = o.values.p; a.first_valid = o.valid.as<uint32_t>(); }
+    if (o.bit == AGG_LAST) { a.last_vals = o.values.p; a.last_valid = o.valid.as<uint32_t>(); }
+  }
+  return a;
+}
+
+// Stream ordered: groups per owner added into d_counts[0 .. n_parts).
+static int partials_count_async(pa_groupby* g, int32_t n_parts, unsigned long long* d_counts) {
+  PartialsArgs a = partials_args(g, n_parts);
+  a.counts = d_counts;
+  if (g->G) {
+    k_partials_count<<<(g->G + 255) / 256, 256, 0, g->stream>>>(a);
+    CUDA_TRY(cudaGetLastError());
+  }
+  return PA_OK;
+}
+
+// counts_host[0 .. n_parts) = what `count_async` (partials_count_async, pairs_count_async) counts per owner.
+static int owner_counts(pa_groupby* g, int32_t n_parts, int (*count_async)(pa_groupby*, int32_t, unsigned long long*), int64_t* counts_host) {
   cudaStream_t st = g->stream;
   DevBuf counts;
   PA_TRY(counts.alloc(sizeof(uint64_t) * n_parts, st));
   CUDA_TRY(cudaMemsetAsync(counts.p, 0, sizeof(uint64_t) * n_parts, st));
-  PartialsArgs a{};
-  a.r = g->res; a.G = g->G; a.nparts = n_parts; a.counts = counts.as<unsigned long long>();
-  if (g->G) {
-    k_partials_count<<<(g->G + 255) / 256, 256, 0, st>>>(a);
-    CUDA_TRY(cudaGetLastError());
-  }
-  std::vector<uint64_t> h(n_parts);
+  PA_TRY(count_async(g, n_parts, counts.as<unsigned long long>()));
+  std::vector<uint64_t> h(static_cast<size_t>(n_parts));
   CUDA_TRY(cudaMemcpyAsync(h.data(), counts.p, sizeof(uint64_t) * n_parts, cudaMemcpyDeviceToHost, st));
   CUDA_TRY(cudaStreamSynchronize(st));
-  g->parts_n = n_parts;
-  g->parts_counts.assign(h.begin(), h.end());
   for (int i = 0; i < n_parts; ++i) counts_host[i] = static_cast<int64_t>(h[i]);
+  return PA_OK;
+}
+
+// Write cursors of a scatter grouped by owner: the exclusive prefix of the per-owner counts, copied to *cursor in stream
+// order (from pageable memory: the copy has read `prefix` when it returns).
+static int owner_cursors(cudaStream_t st, const int64_t* counts, int32_t n_parts, DevBuf* cursor) {
+  std::vector<uint64_t> prefix(static_cast<size_t>(n_parts), 0);
+  for (int i = 1; i < n_parts; ++i) prefix[i] = prefix[i - 1] + static_cast<uint64_t>(counts[i - 1]);
+  PA_TRY(cursor->alloc(sizeof(uint64_t) * n_parts, st));
+  CUDA_TRY(cudaMemcpyAsync(cursor->p, prefix.data(), sizeof(uint64_t) * n_parts, cudaMemcpyHostToDevice, st));
+  return PA_OK;
+}
+
+int pa_groupby_partials_count(pa_groupby* g, int32_t n_parts, int64_t* counts_host) {
+  if (!g || !counts_host || n_parts < 1 || n_parts > 64) return set_err(PA_ERR_INVALID, "bad argument (1 <= n_parts <= 64)");
+  PA_TRY(finish_pending(g));
+  if (!g->have_groups || g->merged) return set_err(PA_ERR_STATE, "partials need a finished local aggregate");
+  PA_TRY(check_shardable(g));
+  PA_TRY(ensure_device(g));
+  PA_TRY(owner_counts(g, n_parts, partials_count_async, counts_host));
+  g->parts_n = n_parts;
+  g->parts_counts.assign(counts_host, counts_host + n_parts);
   return PA_OK;
 }
 
@@ -2999,14 +3240,9 @@ static int partials_export(pa_groupby* g, int32_t n_parts, void* dev_records, in
   if (capacity_records < static_cast<int64_t>(g->G)) return set_err(PA_ERR_INVALID, "record buffer too small");
   PA_TRY(ensure_device(g));
   cudaStream_t st = g->stream;
-  std::vector<uint64_t> prefix(n_parts, 0);
-  for (int i = 1; i < n_parts; ++i) prefix[i] = prefix[i - 1] + static_cast<uint64_t>(g->parts_counts[i - 1]);
   DevBuf cursor;
-  PA_TRY(cursor.alloc(sizeof(uint64_t) * n_parts, st));
-  CUDA_TRY(cudaMemcpyAsync(cursor.p, prefix.data(), sizeof(uint64_t) * n_parts, cudaMemcpyHostToDevice, st));
-  PartialsArgs a{};
-  a.r = g->res; a.G = g->G; a.nparts = n_parts; a.row_base = g->opt.row_base;
-  a.vw = g->last_vw; a.wide = g->last_wide;
+  PA_TRY(owner_cursors(st, g->parts_counts.data(), n_parts, &cursor));
+  PartialsArgs a = partials_args(g, n_parts);
   a.words = words;
   if (words == REC_WORDS_STAGE2) {
     if (!g->s2_ext) return set_err(PA_ERR_STATE, "the last aggregate computed no product / variance / stddev: nothing for stage-2 records");
@@ -3016,17 +3252,13 @@ static int partials_export(pa_groupby* g, int32_t n_parts, void* dev_records, in
     a.m2 = (g->s2_ext & (AGG_VARIANCE | AGG_STDDEV)) ? g->s2_m2.as<double>() : nullptr;
     a.prod = (g->s2_ext & AGG_PRODUCT) ? g->s2_prod.as<unsigned long long>() : nullptr;
   }
-  for (auto& o : g->outs) {
-    if (o.bit == AGG_FIRST) { a.first_vals = o.values.p; a.first_valid = o.valid.as<uint32_t>(); }
-    if (o.bit == AGG_LAST) { a.last_vals = o.values.p; a.last_valid = o.valid.as<uint32_t>(); }
-  }
   a.cursor = cursor.as<unsigned long long>();
   a.records = static_cast<uint64_t*>(dev_records);
   if (g->G) {
     k_partials_scatter<<<(g->G + 255) / 256, 256, 0, st>>>(a);
     CUDA_TRY(cudaGetLastError());
   }
-  CUDA_TRY(cudaStreamSynchronize(st));   // `prefix` and `cursor` die here; records are complete for the caller's collective
+  CUDA_TRY(cudaStreamSynchronize(st));   // `cursor` dies here; records are complete for the caller's collective
   return PA_OK;
 }
 
@@ -3046,8 +3278,7 @@ static int pairs_check(pa_groupby* g, int32_t n_parts) {
   if (n_parts < 1 || n_parts > 64) return set_err(PA_ERR_INVALID, "bad argument (1 <= n_parts <= 64)");
   PA_TRY(finish_pending(g));
   if (g->merged) return set_err(PA_ERR_STATE, "distinct pairs come from a local aggregate, not from a merged handle");
-  if (g->keys.size() != 1 && !g->resample) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of composite keys");
-  if (!g->resample && g->keys[0].is_str) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of utf8 keys: dictionary-encode the column against a shared dictionary");
+  PA_TRY(check_shardable(g));
   if (!g->cd_have) return set_err(PA_ERR_STATE, "the last aggregate computed no count_distinct: no distinct pairs to export");
   return ensure_device(g);
 }
@@ -3076,10 +3307,7 @@ static int pairs_count_async(pa_groupby* g, int32_t n_parts, unsigned long long*
 // The pairs grouped by owner (counts per owner as pa_groupby_distinct_pairs_count gave them); complete on return.
 static int pairs_export(pa_groupby* g, int32_t n_parts, const int64_t* counts, void* dev_pairs, DevBuf* d_cursor) {
   cudaStream_t st = g->stream;
-  std::vector<uint64_t> prefix(static_cast<size_t>(n_parts), 0);
-  for (int i = 1; i < n_parts; ++i) prefix[i] = prefix[i - 1] + static_cast<uint64_t>(counts[i - 1]);
-  PA_TRY(d_cursor->alloc(sizeof(uint64_t) * n_parts, st));
-  CUDA_TRY(cudaMemcpyAsync(d_cursor->p, prefix.data(), sizeof(uint64_t) * n_parts, cudaMemcpyHostToDevice, st));
+  PA_TRY(owner_cursors(st, counts, n_parts, d_cursor));
   PairsArgs a = pairs_args(g, n_parts);
   a.cursor = d_cursor->as<unsigned long long>();
   a.out = static_cast<uint64_t*>(dev_pairs);
@@ -3087,24 +3315,16 @@ static int pairs_export(pa_groupby* g, int32_t n_parts, const int64_t* counts, v
     k_pairs_scatter<<<static_cast<unsigned>((a.n + 255) / 256), 256, 0, st>>>(a);
     CUDA_TRY(cudaGetLastError());
   }
-  CUDA_TRY(cudaStreamSynchronize(st));   // `prefix` dies here
+  CUDA_TRY(cudaStreamSynchronize(st));
   return PA_OK;
 }
 
 int pa_groupby_distinct_pairs_count(pa_groupby* g, int32_t n_parts, int64_t* counts_host) {
   if (!g || !counts_host) return set_err(PA_ERR_INVALID, "null argument");
   PA_TRY(pairs_check(g, n_parts));
-  cudaStream_t st = g->stream;
-  DevBuf counts;
-  PA_TRY(counts.alloc(sizeof(uint64_t) * n_parts, st));
-  CUDA_TRY(cudaMemsetAsync(counts.p, 0, sizeof(uint64_t) * n_parts, st));
-  PA_TRY(pairs_count_async(g, n_parts, counts.as<unsigned long long>()));
-  std::vector<uint64_t> h(static_cast<size_t>(n_parts));
-  CUDA_TRY(cudaMemcpyAsync(h.data(), counts.p, sizeof(uint64_t) * n_parts, cudaMemcpyDeviceToHost, st));
-  CUDA_TRY(cudaStreamSynchronize(st));
+  PA_TRY(owner_counts(g, n_parts, pairs_count_async, counts_host));
   g->dp_parts_n = n_parts;
-  g->dp_counts.assign(h.begin(), h.end());
-  for (int i = 0; i < n_parts; ++i) counts_host[i] = static_cast<int64_t>(h[i]);
+  g->dp_counts.assign(counts_host, counts_host + n_parts);
   return PA_OK;
 }
 
@@ -3117,172 +3337,18 @@ int pa_groupby_distinct_pairs_export(pa_groupby* g, int32_t n_parts, void* dev_p
   return pairs_export(g, n_parts, g->dp_counts.data(), dev_pairs, &cursor);
 }
 
-// Common part of the two merge entry points.  `d_off` = device array [n_sources + 1], exclusive prefix
-// of the per-source record counts (the exact total is d_off[n_sources]); nrec_max = host-side upper bound.
-// Scratch of one merge (key table, per-source index, compaction / sort buffers).  A communicator keeps one between
-// steps (pa_groupby_sharded_aggregate) so that a step allocates nothing but its result.
-struct MergeScratch { DevBuf tkeys, idx, m_first, m_slot, s_first, s_slot, cub_tmp; uint64_t last_slots = 0; };
-
-static int merge_build(pa_groupby* g, const void* dev_records, const uint64_t* d_off, int32_t n_sources, uint64_t nrec_max,
-                       uint32_t agg_mask, const char* value_format, const char* key_format, MergeScratch* keep = nullptr,
-                       uint64_t row_bound = 0, bool compact = false, uint64_t distinct_hint = 0) {
-  cudaStream_t st = g->stream;
-  g->merged = true;
-  g->keys.resize(1);
-  int kw = 8, kvc = VC_I;
-  PA_TRY(parse_format(key_format, &kw, &kvc));
-  g->keys[0].format = key_format;
-  g->keys[0].width = kw;
-  g->fields.assign(1, KeyField{});
-  g->fields[0].width = kw;
-  g->index_format = key_format;
-  PA_TRY(parse_format(value_format, &g->last_vw, &g->last_vc));
-  g->last_vfmt = value_format;
-  if (nrec_max >= 0xFFFFFFFFull) return set_err(PA_ERR_NOT_IMPLEMENTED, "more than 2^32-1 partial records per rank");
-  MergeScratch local_scratch;
-  MergeScratch& ms = keep ? *keep : local_scratch;
-  DevBuf &tkeys = ms.tkeys, &idx = ms.idx, &m_first = ms.m_first, &m_slot = ms.m_slot, &s_first = ms.s_first, &s_slot = ms.s_slot, &cub_tmp = ms.cub_tmp;
-  PA_TRY(m_first.alloc(std::max<uint64_t>(nrec_max, 1) * 8, st));
-  PA_TRY(m_slot.alloc(std::max<uint64_t>(nrec_max, 1) * 4, st));
-  MergeArgs a{};
-  a.records = static_cast<const uint64_t*>(dev_records);
-  a.src_offset = d_off;
-  const uint32_t ext = agg_mask & PA_AGG_STAGE2;
-  a.nsrc = n_sources; a.nrec = nrec_max;
-  a.words = compact ? REC_WORDS_COMPACT : (ext ? REC_WORDS_STAGE2 : REC_WORDS);
-  a.status = g->status.as<uint32_t>();
-  a.m_first_row = m_first.as<uint64_t>(); a.m_slot = m_slot.as<uint32_t>();
-  a.vc = g->last_vc;
-  // Join table: 2^k >= 2 x the number of distinct keys.  A source holds every key at most once, so the count lies
-  // between the largest source and the sum; sources that saw (nearly) the same keys — row-range shards of one column —
-  // are the common case, so the table is sized by `distinct_hint` (the largest source; 0 = unknown) first: 8 sources of
-  // 12.5 M records fill 2^25 slots instead of 2^28 (index array 1 GB instead of 8.6 GB per step).  Too small shows as a
-  // probe sequence beyond max_probe; then the merge is redone with the table every key set fits.
-  uint32_t h_status[ST_WORDS];
-  uint64_t sized_for = distinct_hint ? std::min<uint64_t>(std::max<uint64_t>(distinct_hint + distinct_hint / 4, 512), std::max<uint64_t>(nrec_max, 512)) : std::max<uint64_t>(nrec_max, 512);
-  for (;;) {
-    uint64_t cap = 1024;
-    while (cap < sized_for * 2) cap <<= 1;
-    const uint64_t nslots = cap + 2;
-    ms.last_slots = nslots;
-    PA_TRY(tkeys.alloc(nslots * 8, st));
-    PA_TRY(idx.alloc(nslots * n_sources * 4, st));
-    const int fgrid = static_cast<int>(std::min<uint64_t>((nslots + 255) / 256, static_cast<uint64_t>(g->num_sms) * 16));
-    k_fill_u64<<<fgrid, 256, 0, st>>>(tkeys.as<unsigned long long>(), nslots, kEmptyKey);
-    CUDA_TRY(cudaMemsetAsync(idx.p, 0xFF, nslots * n_sources * 4, st));
-    a.tkeys = tkeys.as<unsigned long long>(); a.cap_mask = cap - 1; a.idx = idx.as<uint32_t>();
-    a.max_probe = sized_for >= nrec_max ? cap : std::min<uint64_t>(cap, 2048);
-    CUDA_TRY(cudaEventRecord(g->ev[1], st));
-    if (nrec_max) {
-      k_merge_insert<<<static_cast<int>((nrec_max + 255) / 256), 256, 0, st>>>(a);
-      CUDA_TRY(cudaGetLastError());
-    }
-    k_merge_compact<<<static_cast<int>((nslots + MC_THREADS - 1) / MC_THREADS), MC_THREADS, 0, st>>>(a);
-    CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaEventRecord(g->ev[2], st));
-    CUDA_TRY(cudaMemcpyAsync(h_status, g->status.p, sizeof h_status, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
-    if (h_status[ST_PEER_OVERFLOW]) return set_err(PA_ERR_STATE, "a source rank had more groups than a padded block holds; use the counted exchange");
-    if (h_status[ST_OVERFLOW] && sized_for < nrec_max) {   // the hint was too small: every key set fits a table sized by the record count
-      sized_for = nrec_max;
-      CUDA_TRY(cudaMemsetAsync(a.status + ST_OVERFLOW, 0, sizeof(uint32_t), st));
-      CUDA_TRY(cudaMemsetAsync(a.status + ST_COUNTER, 0, sizeof(uint32_t), st));
-      continue;
-    }
-    if (h_status[ST_OVERFLOW]) return set_err(PA_ERR_CUDA, "merge table overflow");
-    break;
-  }
-  const uint32_t G = h_status[ST_COUNTER];
-  g->G = G;
-  // all / any: folded as min / max of the 0 / 1 bytes and the count, which is what k_emit_bool reads
-  const uint32_t extb = agg_mask & (PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY);
-  const uint32_t fold_mask = (agg_mask & (PA_AGG_ALL | PA_AGG_STAGE2)) |
-                             (extb ? (PA_AGG_COUNT | ((extb & PA_AGG_BOOL_ALL) ? PA_AGG_MIN : 0u) | ((extb & PA_AGG_BOOL_ANY) ? PA_AGG_MAX : 0u)) : 0u);
-  const bool wide = is_wide(fold_mask, g->last_vc);
-  g->last_wide = wide;
-  PA_TRY(alloc_result(g, G, true, true));
-  PA_TRY(g->m_count64.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
-  g->res.count64 = g->m_count64.as<uint64_t>();
-  PA_TRY(g->m_first_val.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
-  PA_TRY(g->m_first_row_g.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
-  PA_TRY(g->m_last_val.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
-  PA_TRY(g->m_first_valid.alloc(std::max<uint32_t>(G, 1), st));
-  PA_TRY(g->m_last_valid.alloc(std::max<uint32_t>(G, 1), st));
-  if (ext & (AGG_VARIANCE | AGG_STDDEV)) PA_TRY(g->s2_m2.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
-  if (ext & AGG_PRODUCT) PA_TRY(g->s2_prod.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 8, st));
-  uint32_t h_no_terms = 0;
-  if (G) {
-    PA_TRY(s_first.alloc(static_cast<size_t>(G) * 8, st));
-    PA_TRY(s_slot.alloc(static_cast<size_t>(G) * 4, st));
-    size_t tmp_bytes = 0;
-    // (global first rows are below row_bound when the caller knows the shards: sort only the bits that can differ)
-    int end_bit = 64;
-    if (row_bound) { end_bit = 1; while (end_bit < 64 && (row_bound >> end_bit)) ++end_bit; }
-    CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, m_first.as<uint64_t>(), s_first.as<uint64_t>(), m_slot.as<uint32_t>(), s_slot.as<uint32_t>(), static_cast<int>(G), 0, end_bit, st));
-    PA_TRY(cub_tmp.alloc(tmp_bytes, st));
-    CUDA_TRY(cub::DeviceRadixSort::SortPairs(cub_tmp.p, tmp_bytes, m_first.as<uint64_t>(), s_first.as<uint64_t>(), m_slot.as<uint32_t>(), s_slot.as<uint32_t>(), static_cast<int>(G), 0, end_bit, st));
-    a.order = s_slot.as<uint32_t>();
-    a.G = G;
-    a.out = g->res;
-    a.o_first_val = g->m_first_val.as<uint64_t>(); a.o_last_val = g->m_last_val.as<uint64_t>();
-    a.o_first_valid = g->m_first_valid.as<uint8_t>(); a.o_last_valid = g->m_last_valid.as<uint8_t>();
-    a.o_first_row_g = g->m_first_row_g.as<uint64_t>();
-    if (ext) {
-      a.o_m2 = (ext & (AGG_VARIANCE | AGG_STDDEV)) ? g->s2_m2.as<double>() : nullptr;
-      a.o_prod = (ext & AGG_PRODUCT) ? g->s2_prod.as<unsigned long long>() : nullptr;
-      k_merge_fold<true><<<(G + 255) / 256, 256, 0, st>>>(a);
-      CUDA_TRY(cudaGetLastError());
-      CUDA_TRY(cudaMemcpyAsync(&h_no_terms, a.status + ST_NO_TERMS, sizeof h_no_terms, cudaMemcpyDeviceToHost, st));
-    } else {
-      k_merge_fold<false><<<(G + 255) / 256, 256, 0, st>>>(a);
-      CUDA_TRY(cudaGetLastError());
-    }
-  }
-  CUDA_TRY(cudaEventRecord(g->ev[3], st));
-  g->have_groups = true;
-  g->last_launches = 4;
-  g->last_path = 4;
-  PA_TRY(run_emit(g, nullptr, fold_mask));
-  if (ext) {
-    PA_TRY(emit_stage2(g, g->last_vc, ext));
-    g->last_launches += 1;
-  }
-  if (extb) {
-    // (the helper min / max / count outputs are bytes and counts nobody asked for)
-    g->outs.erase(std::remove_if(g->outs.begin(), g->outs.end(), [&](const AggOut& o) { return (o.bit & agg_mask) == 0; }), g->outs.end());
-    PA_TRY(run_bool_emit(g, extb));
-  }
-  CUDA_TRY(cudaEventRecord(g->ev[4], st));
-  CUDA_TRY(cudaStreamSynchronize(st));   // local scratch (table, idx, sort buffers) is released after this point
-  if (h_no_terms) return set_err(PA_ERR_STATE, "partial records carry no variance / product terms for this aggregate mask "
-                                               "(export them with pa_groupby_partials_export_stage2 after an aggregate that computes them)");
-  return PA_OK;
-}
-
 int pa_merge_create(const void* dev_records, const int64_t* counts_by_source, int32_t n_sources, uint32_t agg_mask,
                     const char* value_format, const char* key_format, const pa_options* opt, pa_groupby** out) {
   if (!counts_by_source || n_sources < 1 || !value_format || !key_format || !out) return set_err(PA_ERR_INVALID, "null argument");
   // (count_distinct does not travel in partial records: pa_merge_distinct_pairs adds it to the merged handle)
-  if (agg_mask & ~(PA_AGG_ALL | PA_AGG_STAGE2 | PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY)) return set_err(PA_ERR_INVALID, "bad aggregate mask");
+  if (agg_mask & ~RECORD_AGGS) return set_err(PA_ERR_INVALID, "bad aggregate mask");
   if ((agg_mask & (PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY)) && strcmp(value_format, "b") != 0)
     return set_err(PA_ERR_INVALID, "all / any need a boolean column (arrow::compute has no kernel for other types)");
   HandlePtr g(new pa_groupby());
   PA_TRY(handle_init(g.get(), opt));
-  cudaStream_t st = g->stream;
-  std::vector<uint64_t> off(n_sources + 1, 0);
-  for (int i = 0; i < n_sources; ++i) {
+  for (int i = 0; i < n_sources; ++i)
     if (counts_by_source[i] < 0) return set_err(PA_ERR_INVALID, "negative record count");
-    off[i + 1] = off[i] + static_cast<uint64_t>(counts_by_source[i]);
-  }
-  const uint64_t nrec = off[n_sources];
-  if (nrec && !dev_records) return set_err(PA_ERR_INVALID, "null record buffer");
-  DevBuf d_off;
-  PA_TRY(d_off.alloc(sizeof(uint64_t) * (n_sources + 1), st));
-  CUDA_TRY(cudaMemcpyAsync(d_off.p, off.data(), sizeof(uint64_t) * (n_sources + 1), cudaMemcpyHostToDevice, st));
-  CUDA_TRY(cudaMemsetAsync(g->status.p, 0, sizeof(uint32_t) * ST_WORDS, st));
-  CUDA_TRY(cudaEventRecord(g->ev[0], st));
-  PA_TRY(merge_build(g.get(), dev_records, d_off.as<uint64_t>(), n_sources, nrec, agg_mask, value_format, key_format, nullptr, 0, false,
-                     static_cast<uint64_t>(*std::max_element(counts_by_source, counts_by_source + n_sources))));
+  PA_TRY(merge_counted(g.get(), dev_records, counts_by_source, n_sources, agg_mask, value_format, key_format, nullptr, 0, false));
   *out = g.release();
   return PA_OK;
 }
@@ -3294,7 +3360,7 @@ int pa_merge_create(const void* dev_records, const int64_t* counts_by_source, in
 static int merge_distinct(pa_groupby* g, const void* dev_pairs, uint64_t n_pairs, DevBuf* keep, uint64_t* set_slots) {
   cudaStream_t st = g->stream;
   const uint32_t G = g->G;
-  g->outs.erase(std::remove_if(g->outs.begin(), g->outs.end(), [](const AggOut& o) { return o.bit == PA_AGG_COUNT_DISTINCT; }), g->outs.end());
+  keep_outputs(g, ~PA_AGG_COUNT_DISTINCT);
   uint64_t cap = 1024;
   while (cap < 2 * n_pairs) cap <<= 1;
   DevBuf local_set, distinct, flag;
@@ -3362,17 +3428,10 @@ int pa_merge_distinct_pairs(pa_groupby* merged, const void* dev_pairs, const int
 int pa_groupby_partials_export_padded(pa_groupby* g, int32_t n_parts, void* dev_blocks, int64_t block_records) {
   if (!g || !dev_blocks || n_parts < 1 || n_parts > 64 || block_records < 1) return set_err(PA_ERR_INVALID, "bad argument (1 <= n_parts <= 64)");
   if (!g->have_groups || g->merged) return set_err(PA_ERR_STATE, "partials need a finished local aggregate");
-  if (g->keys.size() != 1 && !g->resample) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of composite keys");
-  if (!g->resample && g->keys[0].is_str) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of utf8 keys: dictionary-encode the column against a shared dictionary");
+  PA_TRY(check_shardable(g));
   PA_TRY(ensure_device(g));
-  PartialsArgs a{};
-  a.r = g->res; a.G = g->G; a.nparts = n_parts; a.row_base = g->opt.row_base;
-  a.vw = g->last_vw; a.wide = g->last_wide;
+  PartialsArgs a = partials_args(g, n_parts);
   a.words = REC_WORDS;
-  for (auto& o : g->outs) {
-    if (o.bit == AGG_FIRST) { a.first_vals = o.values.p; a.first_valid = o.valid.as<uint32_t>(); }
-    if (o.bit == AGG_LAST) { a.last_vals = o.values.p; a.last_valid = o.valid.as<uint32_t>(); }
-  }
   a.records = static_cast<uint64_t*>(dev_blocks);
   if (g->pending) {   // deferred local aggregate: group count and failure flag are still on the device
     a.G_dev = g->status.as<uint32_t>() + ST_NGROUPS;
@@ -3408,88 +3467,43 @@ int pa_merge_create_padded(const void* dev_blocks, int32_t n_sources, int64_t bl
   CUDA_TRY(cudaMemsetAsync(g->status.p, 0, sizeof(uint32_t) * ST_WORDS, st));
   CUDA_TRY(cudaEventRecord(g->ev[0], st));
   // ---- few records: the whole merge is one single-CTA kernel + emit, one synchronisation ----
-  {
-    pa_groupby* h = g.get();
-    h->merged = true;
-    h->keys.resize(1);
-    int kw = 8, kvc = VC_I;
-    PA_TRY(parse_format(key_format, &kw, &kvc));
-    h->keys[0].format = key_format;
-    h->keys[0].width = kw;
-    h->fields.assign(1, KeyField{});
-    h->fields[0].width = kw;
-    h->index_format = key_format;
-    PA_TRY(parse_format(value_format, &h->last_vw, &h->last_vc));
-    h->last_vfmt = value_format;
-    h->last_wide = is_wide(agg_mask, h->last_vc);
-    const uint32_t cap_out = static_cast<uint32_t>(std::min<uint64_t>(nrec_max, MS_MAX_GROUPS)) + 2;
-    PA_TRY(alloc_result(h, cap_out, true, true));
-    PA_TRY(h->m_count64.alloc(static_cast<size_t>(cap_out) * 8, st));
-    h->res.count64 = h->m_count64.as<uint64_t>();
-    PA_TRY(h->m_first_val.alloc(static_cast<size_t>(cap_out) * 8, st));
-    PA_TRY(h->m_first_row_g.alloc(static_cast<size_t>(cap_out) * 8, st));
-    PA_TRY(h->m_last_val.alloc(static_cast<size_t>(cap_out) * 8, st));
-    PA_TRY(h->m_first_valid.alloc(cap_out, st));
-    PA_TRY(h->m_last_valid.alloc(cap_out, st));
-    MergeSmallArgs m{};
-    m.blocks = static_cast<const uint64_t*>(dev_blocks);
-    m.nsrc = static_cast<uint32_t>(n_sources);
-    m.block_records = static_cast<uint64_t>(block_records);
-    m.vc = h->last_vc;
-    m.out = h->res;
-    m.o_first_val = h->m_first_val.as<uint64_t>(); m.o_last_val = h->m_last_val.as<uint64_t>();
-    m.o_first_valid = h->m_first_valid.as<uint8_t>(); m.o_last_valid = h->m_last_valid.as<uint8_t>();
-    m.o_first_row_g = h->m_first_row_g.as<uint64_t>();
-    m.status = h->status.as<uint32_t>();
-    static bool attr_set[64] = {};
-    if (!attr_set[h->device & 63]) {
-      CUDA_TRY(cudaFuncSetAttribute(k_merge_small, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(MS_SMEM_BYTES)));
-      attr_set[h->device & 63] = true;
-    }
-    CUDA_TRY(cudaEventRecord(h->ev[1], st));
-    k_merge_small<<<1, MS_THREADS, MS_SMEM_BYTES, st>>>(m);
-    CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaEventRecord(h->ev[2], st));
-    CUDA_TRY(cudaEventRecord(h->ev[3], st));
-    h->have_groups = true;
-    h->last_launches = 1;
-    h->last_path = 4;
-    h->G = cap_out;                                     // upper bound for the emit grid and the output buffers
-    h->emit_G_dev = h->status.as<uint32_t>() + ST_COUNTER;
-    PA_TRY(run_emit(h, nullptr, agg_mask));
-    h->emit_G_dev = nullptr;
-    CUDA_TRY(cudaEventRecord(h->ev[4], st));
-    // the status words (group count, overflow markers) are read by the first call that needs them
-    h->pending_merge = true;
-    h->poolable = true;
-    h->pm_blocks = dev_blocks; h->pm_nsrc = n_sources; h->pm_block_records = block_records; h->pm_mask = agg_mask;
-    h->pm_vfmt = value_format; h->pm_kfmt = key_format;
-    *out = g.release();
-    return PA_OK;
+  PA_TRY(set_merged_formats(g.get(), value_format, key_format));
+  g->last_wide = is_wide(agg_mask, g->last_vc);
+  const uint32_t cap_out = static_cast<uint32_t>(std::min<uint64_t>(nrec_max, MS_MAX_GROUPS)) + 2;
+  MergeSmallArgs m{};
+  PA_TRY(alloc_merged_result(g.get(), cap_out, &m));
+  m.blocks = static_cast<const uint64_t*>(dev_blocks);
+  m.nsrc = static_cast<uint32_t>(n_sources);
+  m.block_records = static_cast<uint64_t>(block_records);
+  m.vc = g->last_vc;
+  m.status = g->status.as<uint32_t>();
+  static bool attr_set[64] = {};
+  if (!attr_set[g->device & 63]) {
+    CUDA_TRY(cudaFuncSetAttribute(k_merge_small, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(MS_SMEM_BYTES)));
+    attr_set[g->device & 63] = true;
   }
-}
-
-extern "C++" {
-namespace {
-int merge_padded_general(pa_groupby* g, const void* dev_blocks, int32_t n_sources, int64_t block_records, uint32_t agg_mask,
-                         const char* value_format, const char* key_format) {
-  cudaStream_t st = g->stream;
-  const uint64_t nrec_max = static_cast<uint64_t>(n_sources) * static_cast<uint64_t>(block_records);
-  DevBuf d_off, records;
-  PA_TRY(d_off.alloc(sizeof(uint64_t) * (n_sources + 1), st));
-  PA_TRY(records.alloc(nrec_max * PA_PARTIAL_WORDS * 8, st));
-  CUDA_TRY(cudaMemsetAsync(g->status.p, 0, sizeof(uint32_t) * ST_WORDS, st));
-  k_merge_unpad<<<n_sources, 256, 0, st>>>(static_cast<const uint64_t*>(dev_blocks), static_cast<uint32_t>(n_sources),
-                                           static_cast<uint64_t>(block_records), records.as<uint64_t>(), d_off.as<uint64_t>(),
-                                           g->status.as<uint32_t>());
+  CUDA_TRY(cudaEventRecord(g->ev[1], st));
+  k_merge_small<<<1, MS_THREADS, MS_SMEM_BYTES, st>>>(m);
   CUDA_TRY(cudaGetLastError());
-  return merge_build(g, records.p, d_off.as<uint64_t>(), n_sources, nrec_max, agg_mask, value_format, key_format);
+  CUDA_TRY(cudaEventRecord(g->ev[2], st));
+  CUDA_TRY(cudaEventRecord(g->ev[3], st));
+  g->have_groups = true;
+  g->last_launches = 1;
+  g->last_path = 4;
+  g->G = cap_out;                                     // upper bound for the emit grid and the output buffers
+  g->emit_G_dev = g->status.as<uint32_t>() + ST_COUNTER;
+  PA_TRY(run_emit(g.get(), nullptr, agg_mask));
+  g->emit_G_dev = nullptr;
+  CUDA_TRY(cudaEventRecord(g->ev[4], st));
+  // the status words (group count, overflow markers) are read by the first call that needs them
+  g->pending_merge = true;
+  g->poolable = true;
+  g->pm_blocks = dev_blocks; g->pm_nsrc = n_sources; g->pm_block_records = block_records; g->pm_mask = agg_mask;
+  g->pm_vfmt = value_format; g->pm_kfmt = key_format;
+  *out = g.release();
+  return PA_OK;
 }
-}  // namespace
-}  // extern "C++"
 
-// ---- multi-GPU through the C ABI: communicator + the whole sharded step (SURVEY.md §8b "multi-GPU variants taking a
-// communicator handle", §8e) ----
 // ---- host frames larger than the device (or than 2^32-2 rows): aggregate chunk by chunk, merge the partials ----
 // The row-range shards of the multi-GPU path, executed one after the other on ONE device: every chunk of the host
 // columns is copied (staged, §h2d_copy), aggregated with row_base = its first row, and exported as partial records;
@@ -3501,11 +3515,10 @@ int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const stru
                                  const struct ArrowDeviceArray* values, const struct ArrowSchema* value_schema,
                                  uint32_t agg_mask, int64_t chunk_rows, const pa_options* opt, pa_groupby** merged_out) {
   if (!keys || !key_schema || !values || !value_schema || !merged_out) return set_err(PA_ERR_INVALID, "null argument");
-  if (agg_mask == 0 || (agg_mask & ~(PA_AGG_ALL | PA_AGG_STAGE2 | PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY)))
+  if (agg_mask == 0 || (agg_mask & ~RECORD_AGGS))
     return set_err(PA_ERR_NOT_IMPLEMENTED, "chunked aggregates: sum / mean / count / min / max / first / last / product / variance / stddev / "
                                            "all / any (count_distinct is not available across chunks)");
-  const bool stage2 = (agg_mask & PA_AGG_STAGE2) != 0;
-  const size_t RW = stage2 ? PA_PARTIAL_WORDS_STAGE2 : PA_PARTIAL_WORDS;
+  const int RW = record_words(agg_mask, false);
   if (keys->device_type == ARROW_DEVICE_CUDA || values->device_type == ARROW_DEVICE_CUDA)
     return set_err(PA_ERR_INVALID, "chunked aggregation is for HOST columns (device columns already fit the device)");
   const int64_t n = keys->array.length;
@@ -3546,7 +3559,7 @@ int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const stru
       if (total) CUDA_TRY(cudaMemcpy(bigger.p, records.p, total * RW * 8, cudaMemcpyDeviceToDevice));
       records = std::move(bigger);
     }
-    if (cnt) PA_TRY((stage2 ? pa_groupby_partials_export_stage2 : pa_groupby_partials_export)(h, 1, static_cast<char*>(records.p) + total * RW * 8, cnt));
+    if (cnt) PA_TRY(partials_export(h, 1, static_cast<char*>(records.p) + total * RW * 8, cnt, RW));
     PA_TRY(pa_groupby_sync(h));
     total += static_cast<uint64_t>(cnt);
   }
@@ -3557,6 +3570,8 @@ int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const stru
   return PA_OK;
 }
 
+// ---- multi-GPU through the C ABI: communicator + the whole sharded step (SURVEY.md §8b "multi-GPU variants taking a
+// communicator handle", §8e) ----
 struct pa_comm {
   ncclComm_t comm = nullptr;
   int world = 1, rank = 0, device = 0;
@@ -3651,18 +3666,33 @@ int pa_comm_last_phases(pa_comm* c, double phase_ms[5]) {
   return PA_OK;
 }
 
+// Grouped send / receive of `words`-word records: send_cnt[p] from `send` (grouped by destination) to every rank p,
+// recv_cnt[p] from rank p into `recv` (grouped by source).  Every rank issues the same calls in the same order.
+static int exchange_grouped(pa_comm* c, cudaStream_t st, const uint64_t* send, const int64_t* send_cnt, uint64_t* recv,
+                            const int64_t* recv_cnt, size_t words) {
+  NCCL_TRY(ncclGroupStart());
+  uint64_t so = 0, ro = 0;
+  for (int p = 0; p < c->world; ++p) {
+    if (send_cnt[p]) NCCL_TRY(ncclSend(send + so * words, static_cast<size_t>(send_cnt[p]) * words, ncclUint64, p, c->comm, st));
+    if (recv_cnt[p]) NCCL_TRY(ncclRecv(recv + ro * words, static_cast<size_t>(recv_cnt[p]) * words, ncclUint64, p, c->comm, st));
+    so += send_cnt[p];
+    ro += recv_cnt[p];
+  }
+  NCCL_TRY(ncclGroupEnd());
+  return PA_OK;
+}
+
 // One multi-GPU step for this rank: local stages 1-3 on its row shard -> partial records bucketed by owner =
 // hash(key) % world -> counts (ncclAllGather) and records (grouped ncclSend / ncclRecv: NCCL 2.27 has no all-to-all
 // primitive) over NVLink -> owner-side merge in source-rank order.  Everything runs on the handle's stream.
 int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDeviceArray* values,
                                  const struct ArrowSchema* value_schema, uint32_t agg_mask, pa_groupby** merged_out) {
   if (!g || !c || !values || !value_schema || !merged_out) return set_err(PA_ERR_INVALID, "null argument");
-  if (agg_mask == 0 || (agg_mask & ~(PA_AGG_ALL | PA_AGG_STAGE2 | PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY | PA_AGG_COUNT_DISTINCT)))
+  if (agg_mask == 0 || (agg_mask & ~SHARDED_AGGS))
     return set_err(PA_ERR_NOT_IMPLEMENTED, "sharded aggregates: sum / mean / count / min / max / first / last / product / variance / stddev / "
                                            "all / any / count_distinct");
   if (g->device != c->device) return set_err(PA_ERR_INVALID, "handle lives on device %d, communicator on %d", g->device, c->device);
-  if (g->keys.size() != 1 && !g->resample) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of composite keys");
-  if (!g->resample && g->keys[0].is_str) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of utf8 keys: dictionary-encode the column against a shared dictionary");
+  PA_TRY(check_shardable(g));
   PA_TRY(ensure_device(g));
   cudaStream_t st = g->stream;
   const int W = c->world;
@@ -3704,12 +3734,7 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
       CUDA_TRY(cudaGetLastError());
     }
   } else {
-    PartialsArgs a{};
-    a.r = g->res; a.G = g->G; a.nparts = W; a.counts = c->d_counts.as<unsigned long long>();
-    if (g->G) {
-      k_partials_count<<<(g->G + 255) / 256, 256, 0, st>>>(a);
-      CUDA_TRY(cudaGetLastError());
-    }
+    PA_TRY(partials_count_async(g, W, c->d_counts.as<unsigned long long>()));
   }
   if (distinct) PA_TRY(pairs_count_async(g, W, c->d_counts.as<unsigned long long>() + W + 1));
   NCCL_TRY(ncclAllGather(c->d_counts.p, c->d_all.p, W1, ncclUint64, c->comm, st));
@@ -3738,21 +3763,18 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
     if (to_q > 0xFFFFFFFEull) return set_err(PA_ERR_INVALID, "rank %d would receive more than 2^32 - 2 distinct pairs in one merge", q);
   }
   // 3. export the records grouped by owner
-  const int words = stage2 ? REC_WORDS_STAGE2 : rec_words(compact);
+  const int words = record_words(agg_mask, compact);
   const size_t RW = static_cast<size_t>(words);
   PA_TRY(c->send.alloc(std::max<uint64_t>(send_total, 1) * RW * 8, st));
   PA_TRY(c->recv.alloc(std::max<uint64_t>(recv_total, 1) * RW * 8, st));
   if (unordered) {
-    std::vector<uint64_t> prefix(W, 0);
-    for (int i = 1; i < W; ++i) prefix[i] = prefix[i - 1] + static_cast<uint64_t>(send_cnt[i - 1]);
-    PA_TRY(c->d_cursor.alloc(sizeof(uint64_t) * W, st));
-    CUDA_TRY(cudaMemcpyAsync(c->d_cursor.p, prefix.data(), sizeof(uint64_t) * W, cudaMemcpyHostToDevice, st));
+    PA_TRY(owner_cursors(st, send_cnt.data(), W, &c->d_cursor));
     if (G_local) {
       k_bkrec_scatter<<<(G_local + 255) / 256, 256, 0, st>>>(static_cast<const BkRec32*>(g->unordered_recs), G_local, static_cast<uint32_t>(W),
                                                              g->opt.row_base, c->d_cursor.as<unsigned long long>(), c->send.as<uint64_t>());
       CUDA_TRY(cudaGetLastError());
     }
-    CUDA_TRY(cudaStreamSynchronize(st));   // `prefix` dies here
+    CUDA_TRY(cudaStreamSynchronize(st));
   } else {
     g->parts_n = W;
     g->parts_counts.assign(send_cnt.begin(), send_cnt.end());
@@ -3765,29 +3787,9 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
     PA_TRY(pairs_export(g, W, psend_cnt.data(), c->psend.p, &c->d_cursor));
   }
   CUDA_TRY(cudaEventRecord(c->ev[2], st));
-  // 4. all-to-all of the records
-  NCCL_TRY(ncclGroupStart());
-  {
-    uint64_t so = 0, ro = 0;
-    for (int p = 0; p < W; ++p) {
-      if (send_cnt[p]) NCCL_TRY(ncclSend(c->send.as<uint64_t>() + so * RW, static_cast<size_t>(send_cnt[p]) * RW, ncclUint64, p, c->comm, st));
-      if (recv_cnt[p]) NCCL_TRY(ncclRecv(c->recv.as<uint64_t>() + ro * RW, static_cast<size_t>(recv_cnt[p]) * RW, ncclUint64, p, c->comm, st));
-      so += send_cnt[p];
-      ro += recv_cnt[p];
-    }
-  }
-  NCCL_TRY(ncclGroupEnd());
-  if (distinct) {   // the distinct pairs, grouped by owner, in a second exchange
-    NCCL_TRY(ncclGroupStart());
-    uint64_t so = 0, ro = 0;
-    for (int p = 0; p < W; ++p) {
-      if (psend_cnt[p]) NCCL_TRY(ncclSend(c->psend.as<uint64_t>() + so * PW, static_cast<size_t>(psend_cnt[p]) * PW, ncclUint64, p, c->comm, st));
-      if (precv_cnt[p]) NCCL_TRY(ncclRecv(c->precv.as<uint64_t>() + ro * PW, static_cast<size_t>(precv_cnt[p]) * PW, ncclUint64, p, c->comm, st));
-      so += psend_cnt[p];
-      ro += precv_cnt[p];
-    }
-    NCCL_TRY(ncclGroupEnd());
-  }
+  // 4. all-to-all of the records; the distinct pairs, grouped by owner, in a second exchange
+  PA_TRY(exchange_grouped(c, st, c->send.as<uint64_t>(), send_cnt.data(), c->recv.as<uint64_t>(), recv_cnt.data(), RW));
+  if (distinct) PA_TRY(exchange_grouped(c, st, c->psend.as<uint64_t>(), psend_cnt.data(), c->precv.as<uint64_t>(), precv_cnt.data(), PW));
   CUDA_TRY(cudaEventRecord(c->ev[3], st));
   // 5. owner-side merge
   const std::string kfmt = g->resample ? g->index_format : g->keys[0].format;
@@ -3797,15 +3799,8 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   mo.device = g->device;
   mo.cuda_stream = st;
   PA_TRY(handle_init(m.get(), &mo));
-  std::vector<uint64_t> off(W + 1, 0);
-  for (int i = 0; i < W; ++i) off[i + 1] = off[i] + static_cast<uint64_t>(recv_cnt[i]);
-  DevBuf d_off;
-  PA_TRY(d_off.alloc(sizeof(uint64_t) * (W + 1), st));
-  CUDA_TRY(cudaMemcpyAsync(d_off.p, off.data(), sizeof(uint64_t) * (W + 1), cudaMemcpyHostToDevice, st));
-  CUDA_TRY(cudaMemsetAsync(m->status.p, 0, sizeof(uint32_t) * ST_WORDS, st));
-  CUDA_TRY(cudaEventRecord(m->ev[0], st));
-  PA_TRY(merge_build(m.get(), c->recv.p, d_off.as<uint64_t>(), W, recv_total, agg_mask & ~PA_AGG_COUNT_DISTINCT, value_schema->format, kfmt.c_str(),
-                     &c->merge, row_bound, compact, static_cast<uint64_t>(*std::max_element(recv_cnt.begin(), recv_cnt.end()))));
+  PA_TRY(merge_counted(m.get(), c->recv.p, recv_cnt.data(), W, agg_mask & ~PA_AGG_COUNT_DISTINCT, value_schema->format, kfmt.c_str(),
+                       &c->merge, row_bound, compact));
   uint64_t set_slots = 0;
   if (distinct) PA_TRY(merge_distinct(m.get(), c->precv.p, precv_total, &c->pset, &set_slots));
   CUDA_TRY(cudaEventRecord(c->ev[4], st));

@@ -30,7 +30,6 @@ constexpr uint64_t RF_KEY_NULL = 1, RF_FIRST_VALID = 2, RF_LAST_VALID = 4, RF_HA
 // exchange are this code); the public partial record of pa_groupby_partials_export stays PA_PARTIAL_WORDS wide.
 constexpr int RC_KEY = 0, RC_SUM = 1, RC_COUNT = 2, RC_FIRST_ROW = 3, REC_WORDS_COMPACT = 4;
 constexpr uint64_t RC_KEY_NULL_BIT = 1ull << 63;   // in the count word
-__host__ __device__ __forceinline__ int rec_words(bool compact) { return compact ? REC_WORDS_COMPACT : REC_WORDS; }
 __device__ __forceinline__ bool rec_key_null(const uint64_t* rec, bool compact) {
   return compact ? (rec[RC_COUNT] & RC_KEY_NULL_BIT) != 0 : (rec[REC_FLAGS] & RF_KEY_NULL) != 0;
 }

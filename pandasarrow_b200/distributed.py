@@ -18,6 +18,7 @@ backend, which is what the world_size-2 gloo tests exercise on CPU.
 """
 from __future__ import annotations
 
+import functools
 from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
@@ -226,22 +227,22 @@ def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_fo
         except PaError as e:
             if "padded block" not in str(e):
                 raise
-    counts = gb.partials_count(world)
-    dev = torch.device("cuda", torch.cuda.current_device())
-    words = PA_PARTIAL_WORDS_STAGE2 if stage2 else PA_PARTIAL_WORDS
-    send = torch.empty((max(sum(counts), 1), words), dtype=torch.int64, device=dev)
-    gb.partials_export(world, send.data_ptr(), send.shape[0], stage2=stage2)
-    recv, recv_counts = exchange_records(send[:sum(counts)], counts, group, words=words)
-    torch.cuda.synchronize()
+
+    def counted_exchange(count, export, words):
+        counts = count(world)
+        send = torch.empty((max(sum(counts), 1), words), dtype=torch.int64, device=dev)
+        export(world, send.data_ptr(), send.shape[0])
+        recv, recv_counts = exchange_records(send[:sum(counts)], counts, group, words=words)
+        torch.cuda.synchronize()
+        return send, recv, recv_counts
+
+    send, recv, recv_counts = counted_exchange(gb.partials_count, functools.partial(gb.partials_export, stage2=stage2),
+                                               PA_PARTIAL_WORDS_STAGE2 if stage2 else PA_PARTIAL_WORDS)
     merged = MergedGroupBy(recv.data_ptr(), recv_counts, [a for a in aggs if a != "count_distinct"], value_format, key_format,
                            device=dev.index, stream=stream)
     merged._keep = (send, recv)
     if distinct:
-        pcounts = gb.distinct_pairs_count(world)
-        psend = torch.empty((max(sum(pcounts), 1), PA_DISTINCT_PAIR_WORDS), dtype=torch.int64, device=dev)
-        gb.distinct_pairs_export(world, psend.data_ptr(), psend.shape[0])
-        precv, precv_counts = exchange_records(psend[:sum(pcounts)], pcounts, group, words=PA_DISTINCT_PAIR_WORDS)
-        torch.cuda.synchronize()
+        _, precv, precv_counts = counted_exchange(gb.distinct_pairs_count, gb.distinct_pairs_export, PA_DISTINCT_PAIR_WORDS)
         merged.merge_distinct_pairs(precv.data_ptr(), precv_counts)
     return merged
 
