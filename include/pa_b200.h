@@ -325,7 +325,8 @@ int pa_groupby_partials_export_stage2(pa_groupby* g, int32_t n_parts, void* dev_
  * "b" PA_AGG_BOOL_ALL / PA_AGG_BOOL_ANY bits: those merge the records' min / max and count).  The
  * records are PA_PARTIAL_WORDS_STAGE2 words wide exactly when agg_mask has a PA_AGG_STAGE2 bit (then PA_ERR_STATE if
  * a record lacks the terms asked for), PA_PARTIAL_WORDS otherwise.  value_format / key_format are
- * the Arrow format strings of the value and (single) key column.  PA_AGG_COUNT_DISTINCT is not a record aggregate:
+ * the Arrow format strings of the value and (single) key column; a composite key travels as its packed word: pass "L" and
+ * then pa_merge_set_key_layout.  PA_AGG_COUNT_DISTINCT is not a record aggregate:
  * see pa_merge_distinct_pairs. */
 int pa_merge_create(const void* dev_records, const int64_t* counts_by_source, int32_t n_sources, uint32_t agg_mask,
                     const char* value_format, const char* key_format, const pa_options* opt, pa_groupby** out);
@@ -364,16 +365,59 @@ int pa_groupby_partials_export_padded(pa_groupby* g, int32_t n_parts, void* dev_
 int pa_merge_create_padded(const void* dev_blocks, int32_t n_sources, int64_t block_records, uint32_t agg_mask,
                            const char* value_format, const char* key_format, const pa_options* opt, pa_groupby** out);
 
+/* ---- composite keys across shards ----
+ * A composite key is packed into one 64-bit word per row: column j takes bits[j] value bits, then one null bit when
+ * nullable[j], columns in order from bit 0.  Records, owner routing and the merge treat that word as the key.  A handle
+ * packs with the layout its own data implies: a column carries a null bit only when the column handed to
+ * pa_groupby_create has a validity bitmap and a nonzero null_count, and a dictionary column takes bits_for(dictionary
+ * length) bits.  Shards of one frame can therefore pack the same group into different words.  Before their records
+ * meet, all shards agree on one layout (pa_key_layout_agree over every shard's pa_groupby_key_layout) and repack to it
+ * (pa_groupby_set_key_layout); pa_groupby_sharded_aggregate does both by itself. */
+#define PA_MAX_KEY_COLS 4
+typedef struct pa_key_layout {
+  int32_t n_keys;                               /* 2 .. PA_MAX_KEY_COLS */
+  int32_t width[PA_MAX_KEY_COLS];               /* bytes of the key column: 4 or 8 */
+  int32_t bits[PA_MAX_KEY_COLS];                /* value bits (dictionary: bits for its length) */
+  int32_t nullable[PA_MAX_KEY_COLS];            /* 0 / 1: the field carries a null bit */
+  uint64_t dict_fingerprint[PA_MAX_KEY_COLS];   /* 64-bit hash of the dictionary's values; 0 = not a dictionary */
+} pa_key_layout;
+/* The current layout of a composite (2+ column) key handle.  The dictionary fingerprints hash each dictionary's format,
+ * then every entry's validity and bytes; they are computed on the first call and kept (a dictionary on the device is
+ * copied to the host for that).  PA_ERR_INVALID for a single-key, resample or merged handle. */
+int pa_groupby_key_layout(pa_groupby* g, pa_key_layout* out);
+/* The layout every shard packs with, from all n shards' layouts.  Column count, widths, bits and dictionary
+ * fingerprints must be equal on every input (otherwise PA_ERR_INVALID naming the column; for dictionaries: encode the
+ * column against one dictionary shared by all shards); a column is nullable when it is nullable on any input.
+ * PA_ERR_NOT_IMPLEMENTED when the result needs more than 64 bits.  Every shard that applies this to the same inputs
+ * gets the same answer, so all fail together before any record moves. */
+int pa_key_layout_agree(const pa_key_layout* all, int32_t n, pa_key_layout* out);
+/* Repacks a composite key handle's keys under `layout`, which must dominate its own (same column count, widths, bits
+ * and fingerprints; nullable wherever its own is), else PA_ERR_INVALID.  Completes a pending aggregate first; the
+ * groups, outputs, groupings, distinct pairs and stage-2 terms of earlier aggregates are dropped (the next call
+ * recomputes them; group order and values do not change).  Equal to the current layout: no-op. */
+int pa_groupby_set_key_layout(pa_groupby* g, const pa_key_layout* layout);
+/* Gives a merged handle (pa_merge_create / pa_merge_create_padded with key_format "L", the packed word) the composite
+ * key: pa_groupby_unique(merged, j) then returns column j with format key_formats[j] (a dictionary column: its index
+ * format), null where the null bit is set.  Does not complete a pending padded merge. */
+int pa_merge_set_key_layout(pa_groupby* merged, const pa_key_layout* layout, const char* const* key_formats);
+
 /* Host frames larger than free device memory (or than 2^32-2 rows): the columns are aggregated chunk_rows rows at a
  * time — each chunk copied through the pinned staging pipeline, aggregated with row_base = its first row and exported as
  * partial records — and the chunks' records are merged like ranks' (sources folded in row order, groups in global
  * first-appearance order).  Single key column; sum / mean / count / min / max / first / last / product / variance / stddev
  * (those three travel in PA_PARTIAL_WORDS_STAGE2-word records) and all / any of boolean columns; not count_distinct.
  * `merged_out` answers
- * num_groups / unique / fetch like a merged multi-GPU handle.  At most 64 chunks. */
+ * num_groups / unique / fetch like a merged multi-GPU handle.  At most 64 chunks.
+ * pa_groupby_aggregate_chunked is pa_groupby_aggregate_chunked_keys with n_keys = 1. */
 int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const struct ArrowSchema* key_schema,
                                  const struct ArrowDeviceArray* values, const struct ArrowSchema* value_schema,
                                  uint32_t agg_mask, int64_t chunk_rows, const pa_options* opt, pa_groupby** merged_out);
+/* The same with n_keys key columns (a composite key as pa_groupby_create takes it).  Chunks are views of the same
+ * columns, so every chunk packs with the layout of the whole columns; the merged handle carries that layout and
+ * answers pa_groupby_unique for every key column. */
+int pa_groupby_aggregate_chunked_keys(const struct ArrowDeviceArray* keys, const struct ArrowSchema* key_schemas, int32_t n_keys,
+                                      const struct ArrowDeviceArray* values, const struct ArrowSchema* value_schema,
+                                      uint32_t agg_mask, int64_t chunk_rows, const pa_options* opt, pa_groupby** merged_out);
 
 /* ---- the same exchange driven from C: communicator handle + one call per step (SURVEY.md §8b, §8e).
  * pa_comm wraps an NCCL communicator over the GPUs of one node (NVLink / NVSwitch).  Rank 0 obtains an id with
@@ -387,7 +431,11 @@ int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const stru
  * PA_PARTIAL_WORDS_STAGE2-word records, see pa_groupby_partials_export_stage2), PA_AGG_BOOL_ALL / PA_AGG_BOOL_ANY
  * (boolean columns), and PA_AGG_COUNT_DISTINCT: the pairs are counted per owner before the count gather, which carries
  * both counts, travel in a second grouped send / receive after the records and are deduplicated on the merged handle
- * (pa_merge_distinct_pairs); pair send / receive / set scratch stays on the communicator too. */
+ * (pa_merge_distinct_pairs); pair send / receive / set scratch stays on the communicator too.  A composite key handle
+ * starts every step with one more ncclAllGather, of every rank's pa_key_layout, agrees on a layout
+ * (pa_key_layout_agree; all ranks fail together when the layouts do not agree), repacks when it differs from the
+ * handle's own (pa_groupby_set_key_layout) and hands the merged handle that layout and its key formats.  Single-key
+ * and resample steps issue no extra collective. */
 #define PA_COMM_ID_BYTES 128
 typedef struct pa_comm pa_comm;
 int pa_comm_unique_id(void* out_id, int64_t capacity_bytes);
@@ -405,6 +453,10 @@ int pa_comm_last_exchange(pa_comm* c, int32_t* record_bytes, int32_t* unordered_
 /* The last step's count_distinct exchange: distinct pairs this rank sent and received, and the slots of its owner-side
  * set (all 0 when the step computed no count_distinct). */
 int pa_comm_last_distinct(pa_comm* c, int64_t* pairs_sent, int64_t* pairs_received, int64_t* set_slots);
+/* The last step's composite-key agreement, outside the phases above: device time (ms) of the layout gather (copy in,
+ * ncclAllGather, copy out) and of the repack (0 when the handle already packed with the agreed layout); both 0 for a
+ * single-key or resample step. */
+int pa_comm_last_key_layout(pa_comm* c, double* agree_ms, double* repack_ms);
 
 /* ---- synthetic workload generator (SURVEY.md §8d), used by bench.py and the tests so that the
  * same counter-based splitmix64 streams exist on host and device without PCIe staging.

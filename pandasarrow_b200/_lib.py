@@ -18,6 +18,7 @@ PA_PARTIAL_WORDS = 11
 PA_PARTIAL_WORDS_STAGE2 = 13   # records that also carry the product / variance terms
 PA_AGG_STAGE2 = 128 | 256 | 512
 PA_DISTINCT_PAIR_WORDS = 3     # count_distinct across shards: (key, value bits, flags) records
+PA_MAX_KEY_COLS = 4
 
 # every symbol include/pa_b200.h declares
 EXPORTS = [
@@ -33,6 +34,8 @@ EXPORTS = [
     "pa_synth_validity", "pa_synth_timestamps",
     "pa_comm_unique_id", "pa_comm_create", "pa_comm_adopt", "pa_comm_destroy", "pa_groupby_sharded_aggregate", "pa_comm_last_phases", "pa_comm_last_exchange",
     "pa_comm_last_distinct",
+    "pa_groupby_key_layout", "pa_key_layout_agree", "pa_groupby_set_key_layout", "pa_merge_set_key_layout",
+    "pa_groupby_aggregate_chunked_keys", "pa_comm_last_key_layout",
 ]
 
 
@@ -65,6 +68,12 @@ class PaOptions(C.Structure):
     _fields_ = [("device", C.c_int32), ("path", C.c_int32), ("expected_groups", C.c_int64),
                 ("cuda_stream", C.c_void_p), ("row_base", C.c_int64), ("lowcard_no_dense", C.c_int64),
                 ("no_partition", C.c_int64), ("bucket_bits", C.c_int64), ("sm_reserve", C.c_int64)]
+
+
+class PaKeyLayout(C.Structure):
+    """pa_key_layout: how a composite key packs into one 64-bit word (include/pa_b200.h)."""
+    _fields_ = [("n_keys", C.c_int32), ("width", C.c_int32 * PA_MAX_KEY_COLS), ("bits", C.c_int32 * PA_MAX_KEY_COLS),
+                ("nullable", C.c_int32 * PA_MAX_KEY_COLS), ("dict_fingerprint", C.c_uint64 * PA_MAX_KEY_COLS)]
 
 
 _lib = None
@@ -142,6 +151,13 @@ def load():
                                   C.POINTER(PaOptions), C.POINTER(P)]
     L.pa_groupby_aggregate_chunked.argtypes = [C.POINTER(ArrowDeviceArray), C.POINTER(ArrowSchema), C.POINTER(ArrowDeviceArray), C.POINTER(ArrowSchema),
                                                C.c_uint32, C.c_int64, C.POINTER(PaOptions), C.POINTER(P)]
+    L.pa_groupby_aggregate_chunked_keys.argtypes = [C.POINTER(ArrowDeviceArray), C.POINTER(ArrowSchema), C.c_int32,
+                                                    C.POINTER(ArrowDeviceArray), C.POINTER(ArrowSchema), C.c_uint32, C.c_int64,
+                                                    C.POINTER(PaOptions), C.POINTER(P)]
+    L.pa_groupby_key_layout.argtypes = [P, C.POINTER(PaKeyLayout)]
+    L.pa_key_layout_agree.argtypes = [C.POINTER(PaKeyLayout), C.c_int32, C.POINTER(PaKeyLayout)]
+    L.pa_groupby_set_key_layout.argtypes = [P, C.POINTER(PaKeyLayout)]
+    L.pa_merge_set_key_layout.argtypes = [P, C.POINTER(PaKeyLayout), C.POINTER(C.c_char_p)]
     L.pa_groupby_partials_export_padded.argtypes = [P, C.c_int32, P, C.c_int64]
     L.pa_merge_create_padded.argtypes = [P, C.c_int32, C.c_int64, C.c_uint32, C.c_char_p, C.c_char_p,
                                          C.POINTER(PaOptions), C.POINTER(P)]
@@ -154,6 +170,7 @@ def load():
     L.pa_comm_last_phases.argtypes = [P, C.POINTER(C.c_double)]
     L.pa_comm_last_exchange.argtypes = [P, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int64)]
     L.pa_comm_last_distinct.argtypes = [P, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+    L.pa_comm_last_key_layout.argtypes = [P, C.POINTER(C.c_double), C.POINTER(C.c_double)]
     L.pa_synth_keys_i64.argtypes = [P, C.c_int64, C.c_int64, C.c_uint64, C.c_uint64, P]
     L.pa_synth_vals_f64.argtypes = [P, C.c_int64, C.c_int64, C.c_uint64, P]
     L.pa_synth_validity.argtypes = [P, C.c_int64, C.c_int64, C.c_uint64, C.c_uint32, P]

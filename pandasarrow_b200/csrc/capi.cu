@@ -123,6 +123,11 @@ struct Column {
   bool is_dict = false;
   bool is_bool = false;             // Arrow boolean (bit-packed) unpacked to one byte per value in own_data
   int64_t dict_len = 0;
+  // dictionary key column: the (borrowed) dictionary and its fingerprint (dict_fingerprint), computed on first need
+  const ArrowArray* dict = nullptr;
+  const ArrowSchema* dict_schema = nullptr;
+  bool dict_on_dev = false;
+  uint64_t dict_fp = 0;
   DevBuf own_data, own_valid;       // set when the input lived on the host (or was unpacked)
   DevBuf own_bits;                  // boolean host input: the packed bits on the device
   // utf8 / large_utf8 KEY columns (strkeys.cuh): `data` is the per-row 64-bit hash, the strings stay reachable here
@@ -270,6 +275,9 @@ int load_column(const ArrowDeviceArray* da, const ArrowSchema* sc, cudaStream_t 
   out->format = sc->format;
   out->is_dict = sc->dictionary != nullptr;
   out->dict_len = (a.dictionary != nullptr) ? a.dictionary->length : 0;
+  out->dict = a.dictionary;
+  out->dict_schema = sc->dictionary;
+  out->dict_on_dev = da->device_type == ARROW_DEVICE_CUDA;
   out->n = a.length;
   const bool has_nulls = a.null_count != 0 && a.buffers[0] != nullptr;
   const char* values = static_cast<const char*>(a.buffers[1]);
@@ -1584,36 +1592,154 @@ int bits_for(uint64_t n_values) {  // bits needed to represent values 0..n_value
   return b;
 }
 
-int setup_keys(pa_groupby* g) {
-  const int nk = static_cast<int>(g->keys.size());
-  g->fields.assign(nk, KeyField{});
-  if (nk == 1) {
-    const Column& k = g->keys[0];
-    if (k.width != 4 && k.width != 8) return set_err(PA_ERR_INVALID, "key columns must be 32- or 64-bit (format '%s')", k.format.c_str());
-    g->packed = false;
-    g->key_data = k.data;
-    g->key_valid = k.valid;
-    g->key_bit_off = k.bit_off;
-    g->key_width = k.width;
-    g->fields[0].width = k.width;
+// ---- composite keys: the packing layout (pa_key_layout) ----
+static_assert(PA_MAX_KEY_COLS == kMaxKeyCols, "public key column limit");
+
+// Value bits of a composite key's column: a dictionary column needs only enough for its codes
+int key_bits(int width, bool is_dict, int64_t dict_len) {
+  return (is_dict && dict_len > 0) ? bits_for(static_cast<uint64_t>(dict_len)) : width * 8;
+}
+
+// The one place the packing order is decided: column j at the bits after columns 0 .. j-1, value bits then null bit.
+int layout_fields(const pa_key_layout& l, std::vector<KeyField>* fields) {
+  fields->assign(l.n_keys, KeyField{});
+  int shift = 0;
+  for (int j = 0; j < l.n_keys; ++j) {
+    KeyField& f = (*fields)[j];
+    f.width = l.width[j]; f.bits = l.bits[j]; f.nullable = l.nullable[j];
+    f.shift = shift;
+    shift += f.bits + f.nullable;
+  }
+  if (shift > 64) return set_err(PA_ERR_NOT_IMPLEMENTED, "composite key needs %d bits; only keys that pack into 64 bits are supported", shift);
+  return PA_OK;
+}
+
+// A layout from outside (caller, peer rank): `which` names it in the message
+int check_layout(const pa_key_layout& l, int which) {
+  if (l.n_keys < 2 || l.n_keys > PA_MAX_KEY_COLS)
+    return set_err(PA_ERR_INVALID, "key layout %d: %d key columns (a composite key has 2 .. %d)", which, l.n_keys, PA_MAX_KEY_COLS);
+  for (int j = 0; j < l.n_keys; ++j) {
+    if ((l.width[j] != 4 && l.width[j] != 8) || l.bits[j] < 1 || l.bits[j] > l.width[j] * 8 || (l.nullable[j] != 0 && l.nullable[j] != 1))
+      return set_err(PA_ERR_INVALID, "key layout %d, key column %d: width %d, bits %d, nullable %d is not a packable field", which, j,
+                     l.width[j], l.bits[j], l.nullable[j]);
+  }
+  return PA_OK;
+}
+
+// The layout a local handle's key columns imply on their own: a null bit where the column has a validity bitmap
+// (load_column keeps one only when null_count != 0).  Fingerprints stay 0 (fill_fingerprints).
+void column_layout(const pa_groupby* g, pa_key_layout* l) {
+  *l = pa_key_layout{};
+  l->n_keys = static_cast<int32_t>(g->keys.size());
+  for (int j = 0; j < l->n_keys; ++j) {
+    const Column& k = g->keys[j];
+    l->width[j] = k.width;
+    l->bits[j] = key_bits(k.width, k.is_dict, k.dict_len);
+    l->nullable[j] = k.valid != nullptr;
+  }
+}
+
+// The layout the handle packs with now (its fields)
+void fields_layout(const pa_groupby* g, pa_key_layout* l) {
+  *l = pa_key_layout{};
+  l->n_keys = static_cast<int32_t>(g->fields.size());
+  for (int j = 0; j < l->n_keys; ++j) {
+    l->width[j] = g->fields[j].width; l->bits[j] = g->fields[j].bits; l->nullable[j] = g->fields[j].nullable;
+  }
+}
+
+// Bytes [off, off + bytes) of an Arrow buffer on the host (copied from the device when it lives there)
+int host_bytes(const void* buf, size_t off, size_t bytes, bool on_dev, std::vector<uint8_t>* out) {
+  out->resize(bytes);
+  if (!bytes) return PA_OK;
+  if (!buf) return set_err(PA_ERR_INVALID, "dictionary buffer is null");
+  const char* p = static_cast<const char*>(buf) + off;
+  if (on_dev) CUDA_TRY(cudaMemcpy(out->data(), p, bytes, cudaMemcpyDeviceToHost));
+  else memcpy(out->data(), p, bytes);
+  return PA_OK;
+}
+
+uint64_t fnv1a(uint64_t h, const void* p, size_t n) {
+  const uint8_t* b = static_cast<const uint8_t*>(p);
+  for (size_t i = 0; i < n; ++i) { h ^= b[i]; h *= 0x100000001B3ull; }
+  return h;
+}
+
+// 64-bit hash of a dictionary's logical values: its format, its length, then for every entry its validity and (when
+// valid) its bytes, length-prefixed for utf8 / binary.  Computed once per column; never 0 (0 = not a dictionary).
+int dict_fingerprint(Column* k) {
+  if (!k->is_dict || k->dict_fp) return PA_OK;
+  const ArrowArray* d = k->dict;
+  const ArrowSchema* s = k->dict_schema;
+  if (!d || !s || !s->format) return set_err(PA_ERR_INVALID, "dictionary key column without its dictionary");
+  const char* f = s->format;
+  const bool var = (f[0] == 'u' || f[0] == 'U' || f[0] == 'z' || f[0] == 'Z') && f[1] == 0;
+  const bool wide_off = f[0] == 'U' || f[0] == 'Z';
+  int width = 0, vc = VC_I;
+  if (!var) {
+    if (f[0] == 'b') return set_err(PA_ERR_NOT_IMPLEMENTED, "dictionary of booleans in a composite key");
+    PA_TRY(parse_format(f, &width, &vc));
+  }
+  if (d->n_buffers < (var ? 3 : 2)) return set_err(PA_ERR_INVALID, "dictionary of format '%s' has %lld buffers", f, (long long)d->n_buffers);
+  const int64_t len = d->length, off = d->offset;
+  std::vector<uint8_t> valid, vals, offs;
+  const bool has_valid = d->null_count != 0 && d->buffers[0] != nullptr;
+  if (has_valid) PA_TRY(host_bytes(d->buffers[0], static_cast<size_t>(off / 8), static_cast<size_t>((off + len + 7) / 8 - off / 8), k->dict_on_dev, &valid));
+  int64_t first = 0;
+  if (var) {
+    const size_t ow = wide_off ? 8 : 4;
+    PA_TRY(host_bytes(d->buffers[1], static_cast<size_t>(off) * ow, static_cast<size_t>(len + 1) * ow, k->dict_on_dev, &offs));
+    auto at = [&](int64_t i) -> int64_t {
+      if (wide_off) { int64_t v; memcpy(&v, offs.data() + i * 8, 8); return v; }
+      int32_t v; memcpy(&v, offs.data() + i * 4, 4); return v;
+    };
+    first = at(0);
+    const int64_t last = at(len);
+    if (last < first) return set_err(PA_ERR_INVALID, "dictionary offsets are not ascending");
+    PA_TRY(host_bytes(d->buffers[2], static_cast<size_t>(first), static_cast<size_t>(last - first), k->dict_on_dev, &vals));
+    uint64_t h = fnv1a(0xCBF29CE484222325ull, f, strlen(f) + 1);
+    h = fnv1a(h, &len, sizeof len);
+    for (int64_t i = 0; i < len; ++i) {
+      const uint8_t ok = has_valid ? ((valid[static_cast<size_t>((off % 8 + i) / 8)] >> ((off % 8 + i) % 8)) & 1) : 1;
+      h = fnv1a(h, &ok, 1);
+      if (!ok) continue;
+      const int64_t b = at(i) - first, n = at(i + 1) - at(i);
+      h = fnv1a(h, &n, sizeof n);
+      h = fnv1a(h, vals.data() + b, static_cast<size_t>(n));
+    }
+    k->dict_fp = h ? h : 1;
     return PA_OK;
   }
-  if (nk > kMaxKeyCols) return set_err(PA_ERR_INVALID, "at most %d key columns", kMaxKeyCols);
-  int shift = 0;
+  PA_TRY(host_bytes(d->buffers[1], static_cast<size_t>(off) * width, static_cast<size_t>(len) * width, k->dict_on_dev, &vals));
+  uint64_t h = fnv1a(0xCBF29CE484222325ull, f, strlen(f) + 1);
+  h = fnv1a(h, &len, sizeof len);
+  for (int64_t i = 0; i < len; ++i) {
+    const uint8_t ok = has_valid ? ((valid[static_cast<size_t>((off % 8 + i) / 8)] >> ((off % 8 + i) % 8)) & 1) : 1;
+    h = fnv1a(h, &ok, 1);
+    if (ok) h = fnv1a(h, vals.data() + i * width, static_cast<size_t>(width));
+  }
+  k->dict_fp = h ? h : 1;
+  return PA_OK;
+}
+
+int fill_fingerprints(pa_groupby* g, pa_key_layout* l) {
+  for (int j = 0; j < l->n_keys; ++j) {
+    PA_TRY(dict_fingerprint(&g->keys[j]));
+    l->dict_fingerprint[j] = g->keys[j].dict_fp;
+  }
+  return PA_OK;
+}
+
+// Packs the handle's key columns under g->fields into one 64-bit word per row
+int pack_keys(pa_groupby* g) {
+  const int nk = static_cast<int>(g->keys.size());
   KeyPackArgs a{};
   for (int j = 0; j < nk; ++j) {
     const Column& k = g->keys[j];
-    if (k.width != 4 && k.width != 8) return set_err(PA_ERR_INVALID, "key columns must be 32- or 64-bit (format '%s')", k.format.c_str());
-    KeyField& f = g->fields[j];
-    f.width = k.width;
-    f.bits = (k.is_dict && k.dict_len > 0) ? bits_for(static_cast<uint64_t>(k.dict_len)) : k.width * 8;
-    f.nullable = k.valid != nullptr;
-    f.shift = shift;
-    shift += f.bits + f.nullable;
+    const KeyField& f = g->fields[j];
     a.col[j] = k.data; a.valid[j] = k.valid; a.off[j] = k.bit_off; a.width[j] = k.width;
     a.bits[j] = f.bits; a.shift[j] = f.shift; a.nullable[j] = f.nullable;
   }
-  if (shift > 64) return set_err(PA_ERR_NOT_IMPLEMENTED, "composite key needs %d bits; only keys that pack into 64 bits are supported", shift);
   PA_TRY(g->packed_keys.alloc(static_cast<size_t>(g->n) * 8, g->stream));
   a.n_cols = nk;
   a.n = g->n;
@@ -1626,6 +1752,48 @@ int setup_keys(pa_groupby* g) {
   g->key_valid = nullptr;
   g->key_bit_off = 0;
   g->key_width = 8;
+  return PA_OK;
+}
+
+int setup_keys(pa_groupby* g) {
+  const int nk = static_cast<int>(g->keys.size());
+  if (nk == 1) {
+    const Column& k = g->keys[0];
+    if (k.width != 4 && k.width != 8) return set_err(PA_ERR_INVALID, "key columns must be 32- or 64-bit (format '%s')", k.format.c_str());
+    g->fields.assign(1, KeyField{});
+    g->packed = false;
+    g->key_data = k.data;
+    g->key_valid = k.valid;
+    g->key_bit_off = k.bit_off;
+    g->key_width = k.width;
+    g->fields[0].width = k.width;
+    return PA_OK;
+  }
+  if (nk > kMaxKeyCols) return set_err(PA_ERR_INVALID, "at most %d key columns", kMaxKeyCols);
+  for (const Column& k : g->keys)
+    if (k.width != 4 && k.width != 8) return set_err(PA_ERR_INVALID, "key columns must be 32- or 64-bit (format '%s')", k.format.c_str());
+  pa_key_layout own;
+  column_layout(g, &own);
+  PA_TRY(layout_fields(own, &g->fields));
+  return pack_keys(g);
+}
+
+// A merged handle's composite key: the records carry the packed word, pa_groupby_unique unpacks column j of it
+int set_merged_layout(pa_groupby* g, const pa_key_layout& l, const char* const* key_formats) {
+  std::vector<KeyField> fields;
+  PA_TRY(layout_fields(l, &fields));
+  std::vector<Column> keys(static_cast<size_t>(l.n_keys));
+  for (int j = 0; j < l.n_keys; ++j) {
+    if (!key_formats[j]) return set_err(PA_ERR_INVALID, "key_formats[%d] is null", j);
+    int w = 8, vc = VC_I;
+    PA_TRY(parse_format(key_formats[j], &w, &vc));
+    if (w != l.width[j]) return set_err(PA_ERR_INVALID, "key_formats[%d] '%s' is %d bytes wide, the layout says %d", j, key_formats[j], w, l.width[j]);
+    keys[j].format = key_formats[j];
+    keys[j].width = w;
+  }
+  g->keys = std::move(keys);
+  g->fields = std::move(fields);
+  g->packed = true;
   return PA_OK;
 }
 
@@ -1727,6 +1895,7 @@ int aggregate_impl_raw(pa_groupby* g, const Column* val, uint32_t mask, bool def
 // ---- owner-side merge of partial records (merge.cuh) ----
 int set_merged_formats(pa_groupby* g, const char* value_format, const char* key_format) {
   g->merged = true;
+  g->packed = false;   // (pa_merge_set_key_layout makes it composite; a recycled handle may have been)
   g->keys.resize(1);
   int kw = 8, kvc = VC_I;
   PA_TRY(parse_format(key_format, &kw, &kvc));
@@ -1932,7 +2101,17 @@ int finish_pending(pa_groupby* g) {
     g->outs.clear();                                    // too many records / groups for one CTA: general merge
     g->have_groups = false;
     g->poolable = false;
-    return merge_padded_general(g, g->pm_blocks, g->pm_nsrc, g->pm_block_records, g->pm_mask, g->pm_vfmt.c_str(), g->pm_kfmt.c_str());
+    if (!g->packed)
+      return merge_padded_general(g, g->pm_blocks, g->pm_nsrc, g->pm_block_records, g->pm_mask, g->pm_vfmt.c_str(), g->pm_kfmt.c_str());
+    // composite key (pa_merge_set_key_layout): the general merge sets the key format anew, the layout stays
+    pa_key_layout l;
+    fields_layout(g, &l);
+    std::vector<std::string> kf;
+    for (const Column& k : g->keys) kf.push_back(k.format);
+    PA_TRY(merge_padded_general(g, g->pm_blocks, g->pm_nsrc, g->pm_block_records, g->pm_mask, g->pm_vfmt.c_str(), g->pm_kfmt.c_str()));
+    std::vector<const char*> kp;
+    for (const std::string& s : kf) kp.push_back(s.c_str());
+    return set_merged_layout(g, l, kp.data());
   }
   if (!g->pending) return PA_OK;
   g->pending = false;
@@ -3165,10 +3344,93 @@ int pa_sort_indices(pa_groupby* g, struct ArrowArray* out, struct ArrowSchema* o
 }
 
 // ---- multi-GPU partial export / merge ----
-static int check_shardable(const pa_groupby* g) {   // keys the exchange routes: one fixed-width column or a resample index
-  if (g->keys.size() != 1 && !g->resample) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of composite keys");
+// keys the exchange routes: one fixed-width column, a packed composite key or a resample index
+static int check_shardable(const pa_groupby* g) {
   if (!g->resample && g->keys[0].is_str) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of utf8 keys: dictionary-encode the column against a shared dictionary");
   return PA_OK;
+}
+
+static int check_composite_local(const pa_groupby* g) {
+  if (g->resample || g->merged || !g->packed) return set_err(PA_ERR_INVALID, "key layouts describe the composite key (2+ columns) of a pa_groupby_create handle");
+  return PA_OK;
+}
+
+// The current layout with its dictionary fingerprints
+static int key_layout_of(pa_groupby* g, pa_key_layout* out) {
+  PA_TRY(check_composite_local(g));
+  fields_layout(g, out);
+  return fill_fingerprints(g, out);
+}
+
+int pa_groupby_key_layout(pa_groupby* g, pa_key_layout* out) {
+  if (!g || !out) return set_err(PA_ERR_INVALID, "null argument");
+  return key_layout_of(g, out);
+}
+
+int pa_key_layout_agree(const pa_key_layout* all, int32_t n, pa_key_layout* out) {
+  if (!all || !out || n < 1) return set_err(PA_ERR_INVALID, "bad argument (n >= 1 layouts)");
+  for (int i = 0; i < n; ++i) PA_TRY(check_layout(all[i], i));
+  pa_key_layout r = all[0];
+  for (int i = 1; i < n; ++i) {
+    const pa_key_layout& l = all[i];
+    if (l.n_keys != r.n_keys) return set_err(PA_ERR_INVALID, "key layouts differ in their number of key columns (%d vs %d)", r.n_keys, l.n_keys);
+    for (int j = 0; j < r.n_keys; ++j) {
+      if (l.width[j] != r.width[j]) return set_err(PA_ERR_INVALID, "key column %d: widths differ across shards (%d vs %d bytes)", j, r.width[j], l.width[j]);
+      // (before the bits: dictionaries of different lengths are a dictionary mismatch too)
+      if (l.dict_fingerprint[j] != r.dict_fingerprint[j])
+        return set_err(PA_ERR_INVALID, "key column %d: dictionaries differ across shards; encode the column against one dictionary shared by all shards", j);
+      if (l.bits[j] != r.bits[j]) return set_err(PA_ERR_INVALID, "key column %d: value bits differ across shards (%d vs %d)", j, r.bits[j], l.bits[j]);
+      r.nullable[j] |= l.nullable[j];
+    }
+  }
+  std::vector<KeyField> fields;
+  PA_TRY(layout_fields(r, &fields));
+  *out = r;
+  return PA_OK;
+}
+
+int pa_groupby_set_key_layout(pa_groupby* g, const pa_key_layout* layout) {
+  if (!g || !layout) return set_err(PA_ERR_INVALID, "null argument");
+  PA_TRY(check_composite_local(g));
+  PA_TRY(check_layout(*layout, 0));
+  PA_TRY(ensure_device(g));
+  PA_TRY(finish_pending(g));
+  pa_key_layout own;
+  column_layout(g, &own);
+  PA_TRY(fill_fingerprints(g, &own));
+  if (layout->n_keys != own.n_keys) return set_err(PA_ERR_INVALID, "the layout has %d key columns, the handle %d", layout->n_keys, own.n_keys);
+  for (int j = 0; j < own.n_keys; ++j) {
+    if (layout->width[j] != own.width[j]) return set_err(PA_ERR_INVALID, "key column %d: the layout says %d bytes, the column has %d", j, layout->width[j], own.width[j]);
+    if (layout->dict_fingerprint[j] != own.dict_fingerprint[j])
+      return set_err(PA_ERR_INVALID, "key column %d: the layout's dictionary differs from the column's; encode the column against one dictionary shared by all shards", j);
+    if (layout->bits[j] != own.bits[j]) return set_err(PA_ERR_INVALID, "key column %d: the layout says %d value bits, the column needs %d", j, layout->bits[j], own.bits[j]);
+    if (own.nullable[j] && !layout->nullable[j]) return set_err(PA_ERR_INVALID, "key column %d has nulls, the layout gives it no null bit", j);
+  }
+  pa_key_layout cur;
+  fields_layout(g, &cur);
+  bool same = true;
+  for (int j = 0; j < own.n_keys; ++j) same = same && cur.nullable[j] == layout->nullable[j];
+  if (same) return PA_OK;
+  std::vector<KeyField> fields;
+  PA_TRY(layout_fields(*layout, &fields));
+  g->fields = std::move(fields);
+  PA_TRY(pack_keys(g));
+  // everything below was computed from the old key words
+  g->have_groups = false; g->bk_have_hist = false; g->G = 0; g->outs.clear();
+  g->have_groupings = false;
+  g->parts_n = 0;
+  g->s2_ext = 0; g->s2_m2.reset(); g->s2_prod.reset();
+  g->cd_have = false; g->cd_n = 0; g->cd_id.reset(); g->cd_bits.reset(); g->dp_parts_n = 0;
+  return PA_OK;
+}
+
+int pa_merge_set_key_layout(pa_groupby* merged, const pa_key_layout* layout, const char* const* key_formats) {
+  if (!merged || !layout || !key_formats) return set_err(PA_ERR_INVALID, "null argument");
+  if (!merged->merged || merged->resample) return set_err(PA_ERR_STATE, "a merged key layout applies to a handle made by pa_merge_create / pa_merge_create_padded");
+  if (!merged->packed && merged->keys[0].format != "L")
+    return set_err(PA_ERR_INVALID, "composite keys travel as their packed word: merge with key format \"L\", not '%s'", merged->keys[0].format.c_str());
+  PA_TRY(check_layout(*layout, 0));
+  return set_merged_layout(merged, *layout, key_formats);
 }
 
 // The groups of the last aggregate and the values its records carry (records of any width)
@@ -3514,15 +3776,38 @@ int pa_merge_create_padded(const void* dev_blocks, int32_t n_sources, int64_t bl
 int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const struct ArrowSchema* key_schema,
                                  const struct ArrowDeviceArray* values, const struct ArrowSchema* value_schema,
                                  uint32_t agg_mask, int64_t chunk_rows, const pa_options* opt, pa_groupby** merged_out) {
-  if (!keys || !key_schema || !values || !value_schema || !merged_out) return set_err(PA_ERR_INVALID, "null argument");
+  return pa_groupby_aggregate_chunked_keys(keys, key_schema, 1, values, value_schema, agg_mask, chunk_rows, opt, merged_out);
+}
+
+// Composite keys: every chunk is a view of the same columns (same dictionaries, and a chunk of a column with nulls keeps
+// the bitmap), so each chunk packs with the layout of the whole columns; that layout goes to the merged handle.
+int pa_groupby_aggregate_chunked_keys(const struct ArrowDeviceArray* keys, const struct ArrowSchema* key_schemas, int32_t n_keys,
+                                      const struct ArrowDeviceArray* values, const struct ArrowSchema* value_schema,
+                                      uint32_t agg_mask, int64_t chunk_rows, const pa_options* opt, pa_groupby** merged_out) {
+  if (!keys || !key_schemas || n_keys < 1 || !values || !value_schema || !merged_out) return set_err(PA_ERR_INVALID, "null argument");
   if (agg_mask == 0 || (agg_mask & ~RECORD_AGGS))
     return set_err(PA_ERR_NOT_IMPLEMENTED, "chunked aggregates: sum / mean / count / min / max / first / last / product / variance / stddev / "
                                            "all / any (count_distinct is not available across chunks)");
   const int RW = record_words(agg_mask, false);
-  if (keys->device_type == ARROW_DEVICE_CUDA || values->device_type == ARROW_DEVICE_CUDA)
-    return set_err(PA_ERR_INVALID, "chunked aggregation is for HOST columns (device columns already fit the device)");
+  for (int j = 0; j < n_keys; ++j)
+    if (keys[j].device_type == ARROW_DEVICE_CUDA || values->device_type == ARROW_DEVICE_CUDA)
+      return set_err(PA_ERR_INVALID, "chunked aggregation is for HOST columns (device columns already fit the device)");
   const int64_t n = keys->array.length;
   if (values->array.length != n) return set_err(PA_ERR_INVALID, "key and value columns differ in length");
+  for (int j = 1; j < n_keys; ++j)
+    if (keys[j].array.length != n) return set_err(PA_ERR_INVALID, "key columns differ in length");
+  const bool composite = n_keys > 1;
+  pa_key_layout whole{};   // composite: the layout of the whole columns (as load_column + column_layout see them)
+  if (composite && n_keys <= PA_MAX_KEY_COLS) {
+    whole.n_keys = n_keys;
+    for (int j = 0; j < n_keys; ++j) {
+      int w = 8, vc = VC_I;
+      if (parse_format(key_schemas[j].format, &w, &vc) != PA_OK) break;   // (pa_groupby_create reports it)
+      whole.width[j] = w;
+      whole.bits[j] = key_bits(w, key_schemas[j].dictionary != nullptr, keys[j].array.dictionary ? keys[j].array.dictionary->length : 0);
+      whole.nullable[j] = keys[j].array.null_count != 0 && keys[j].array.buffers[0] != nullptr;
+    }
+  }
   if (chunk_rows <= 0) chunk_rows = 1ll << 30;
   if (chunk_rows >= 0xFFFFFFFEll) return set_err(PA_ERR_INVALID, "chunk_rows must be below 2^32 - 2");
   const int64_t n_chunks = std::max<int64_t>(1, (n + chunk_rows - 1) / chunk_rows);
@@ -3536,16 +3821,27 @@ int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const stru
   uint64_t total = 0;
   for (int64_t c = 0; c < n_chunks; ++c) {
     const int64_t lo = c * chunk_rows, len = std::min(chunk_rows, n - lo);
-    ArrowDeviceArray kc = *keys, vc = *values;           // views: same buffers, shifted window
-    kc.array.offset += lo; kc.array.length = len;
+    std::vector<ArrowDeviceArray> kc(keys, keys + n_keys);   // views: same buffers, shifted window
+    ArrowDeviceArray vc = *values;
+    for (ArrowDeviceArray& k : kc) {
+      k.array.offset += lo; k.array.length = len;
+      if (k.array.null_count > 0) k.array.null_count = -1;
+      k.array.release = nullptr;
+    }
     vc.array.offset += lo; vc.array.length = len;
-    if (kc.array.null_count > 0) kc.array.null_count = -1;
     if (vc.array.null_count > 0) vc.array.null_count = -1;
-    kc.array.release = nullptr; vc.array.release = nullptr;
+    vc.array.release = nullptr;
     o.row_base = base0 + lo;
     pa_groupby* h = nullptr;
-    PA_TRY(pa_groupby_create(&kc, key_schema, 1, &o, &h));
+    PA_TRY(pa_groupby_create(kc.data(), key_schemas, n_keys, &o, &h));
     HandlePtr guard(h);
+    if (composite) {
+      pa_key_layout mine;
+      fields_layout(h, &mine);
+      for (int j = 0; j < n_keys; ++j)
+        if (mine.width[j] != whole.width[j] || mine.bits[j] != whole.bits[j] || mine.nullable[j] != whole.nullable[j])
+          return set_err(PA_ERR_STATE, "chunk %lld packs key column %d differently from the whole column", (long long)c, j);
+    }
     PA_TRY(pa_groupby_aggregate(h, &vc, value_schema, agg_mask));
     int64_t cnt = 0;
     PA_TRY(pa_groupby_partials_count(h, 1, &cnt));
@@ -3564,9 +3860,17 @@ int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const stru
     total += static_cast<uint64_t>(cnt);
   }
   o.row_base = base0;
-  const std::string kfmt = key_schema->format;
-  PA_TRY(pa_merge_create(records.p, counts.data(), static_cast<int32_t>(n_chunks), agg_mask, value_schema->format, kfmt.c_str(), &o, merged_out));
+  const std::string kfmt = composite ? "L" : key_schemas->format;
+  pa_groupby* m = nullptr;
+  PA_TRY(pa_merge_create(records.p, counts.data(), static_cast<int32_t>(n_chunks), agg_mask, value_schema->format, kfmt.c_str(), &o, &m));
+  HandlePtr merged(m);
+  if (composite) {
+    std::vector<const char*> kf;
+    for (int j = 0; j < n_keys; ++j) kf.push_back(key_schemas[j].format);
+    PA_TRY(set_merged_layout(m, whole, kf.data()));
+  }
   CUDA_TRY(cudaDeviceSynchronize());   // `records` is released on return
+  *merged_out = merged.release();
   return PA_OK;
 }
 
@@ -3579,8 +3883,10 @@ struct pa_comm {
   DevBuf send, recv, d_counts, d_all, d_cursor;     // kept between steps (grow only)
   DevBuf psend, precv, pset;                        // count_distinct: distinct pairs sent / received, the owner's set
   MergeScratch merge;
+  DevBuf layouts;                                   // composite keys: this rank's pa_key_layout, then all ranks'
   double phase_ms[5] = {0, 0, 0, 0, 0};   // last step: local pass, count + export, exchange, merge, total
-  cudaEvent_t ev[6] = {};
+  double agree_ms = 0, repack_ms = 0;     // last step: key layout gather, repack (pa_comm_last_key_layout)
+  cudaEvent_t ev[8] = {};
   uint64_t h_bound = 0;                   // end of this rank's row shard (staging for the async copy)
   int last_record_bytes = 0, last_unordered = 0;   // pa_comm_last_exchange
   int64_t last_table_slots = 0;
@@ -3604,7 +3910,7 @@ int pa_comm_unique_id(void* out_id, int64_t capacity_bytes) {
 static int comm_finish(pa_comm* c) {
   // The communicator outlives the handles (and their streams) it is used with: its scratch does not belong to any
   // stream's allocation order.
-  for (DevBuf* b : {&c->send, &c->recv, &c->d_counts, &c->d_all, &c->d_cursor, &c->psend, &c->precv, &c->pset, &c->merge.tkeys, &c->merge.idx,
+  for (DevBuf* b : {&c->send, &c->recv, &c->d_counts, &c->d_all, &c->d_cursor, &c->psend, &c->precv, &c->pset, &c->layouts, &c->merge.tkeys, &c->merge.idx,
                     &c->merge.m_first, &c->merge.m_slot, &c->merge.s_first, &c->merge.s_slot, &c->merge.cub_tmp})
     b->plain = true;
   for (auto& e : c->ev) CUDA_TRY(cudaEventCreate(&e));
@@ -3660,6 +3966,13 @@ int pa_comm_last_distinct(pa_comm* c, int64_t* pairs_sent, int64_t* pairs_receiv
   return PA_OK;
 }
 
+int pa_comm_last_key_layout(pa_comm* c, double* agree_ms, double* repack_ms) {
+  if (!c) return set_err(PA_ERR_INVALID, "null argument");
+  if (agree_ms) *agree_ms = c->agree_ms;
+  if (repack_ms) *repack_ms = c->repack_ms;
+  return PA_OK;
+}
+
 int pa_comm_last_phases(pa_comm* c, double phase_ms[5]) {
   if (!c || !phase_ms) return set_err(PA_ERR_INVALID, "null argument");
   for (int i = 0; i < 5; ++i) phase_ms[i] = c->phase_ms[i];
@@ -3696,6 +4009,41 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   PA_TRY(ensure_device(g));
   cudaStream_t st = g->stream;
   const int W = c->world;
+  // 0. composite key: every rank's key layout to everybody, one agreed layout, repack when it differs from this
+  // handle's.  On every step (never cached): a rank that skipped the gather while another ran it would hang the step.
+  // A rank that cannot describe its layout still takes part (with n_keys = 0), so that every rank fails together.
+  const bool composite = g->packed && !g->resample;
+  pa_key_layout agreed{};
+  c->agree_ms = 0; c->repack_ms = 0;
+  if (composite) {
+    pa_key_layout mine{};
+    const int mine_rc = key_layout_of(g, &mine);
+    const std::string mine_err = mine_rc != PA_OK ? g_err : std::string();
+    if (mine_rc != PA_OK) mine = pa_key_layout{};
+    const size_t LB = sizeof(pa_key_layout);
+    PA_TRY(c->layouts.alloc(LB * (W + 1), st));
+    CUDA_TRY(cudaEventRecord(c->ev[5], st));
+    CUDA_TRY(cudaMemcpyAsync(c->layouts.p, &mine, LB, cudaMemcpyHostToDevice, st));
+    NCCL_TRY(ncclAllGather(c->layouts.p, c->layouts.as<char>() + LB, LB, ncclUint8, c->comm, st));
+    std::vector<pa_key_layout> all(static_cast<size_t>(W));
+    CUDA_TRY(cudaMemcpyAsync(all.data(), c->layouts.as<char>() + LB, LB * W, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaEventRecord(c->ev[6], st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    if (mine_rc != PA_OK) return set_err(mine_rc, "%s", mine_err.c_str());
+    PA_TRY(pa_key_layout_agree(all.data(), W, &agreed));
+    bool repack = false;
+    for (int j = 0; j < agreed.n_keys; ++j) repack = repack || agreed.nullable[j] != mine.nullable[j];
+    PA_TRY(pa_groupby_set_key_layout(g, &agreed));
+    float t = 0;
+    CUDA_TRY(cudaEventElapsedTime(&t, c->ev[5], c->ev[6]));
+    c->agree_ms = t;
+    if (repack) {
+      CUDA_TRY(cudaEventRecord(c->ev[7], st));
+      CUDA_TRY(cudaEventSynchronize(c->ev[7]));
+      CUDA_TRY(cudaEventElapsedTime(&t, c->ev[6], c->ev[7]));
+      c->repack_ms = t;
+    }
+  }
   CUDA_TRY(cudaEventRecord(c->ev[0], st));
   // 1. local pass.  sum / mean of floats / count need one 32-byte sector per group (compact records, merge.cuh),
   // everything else the full record; with compact records the bucketed path may hand over its unordered group records
@@ -3792,7 +4140,7 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   if (distinct) PA_TRY(exchange_grouped(c, st, c->psend.as<uint64_t>(), psend_cnt.data(), c->precv.as<uint64_t>(), precv_cnt.data(), PW));
   CUDA_TRY(cudaEventRecord(c->ev[3], st));
   // 5. owner-side merge
-  const std::string kfmt = g->resample ? g->index_format : g->keys[0].format;
+  const std::string kfmt = g->resample ? g->index_format : composite ? "L" : g->keys[0].format;
   HandlePtr m(new pa_groupby());
   pa_options mo;
   pa_options_init(&mo);
@@ -3801,6 +4149,11 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   PA_TRY(handle_init(m.get(), &mo));
   PA_TRY(merge_counted(m.get(), c->recv.p, recv_cnt.data(), W, agg_mask & ~PA_AGG_COUNT_DISTINCT, value_schema->format, kfmt.c_str(),
                        &c->merge, row_bound, compact));
+  if (composite) {
+    std::vector<const char*> kf;
+    for (const Column& k : g->keys) kf.push_back(k.format.c_str());
+    PA_TRY(set_merged_layout(m.get(), agreed, kf.data()));
+  }
   uint64_t set_slots = 0;
   if (distinct) PA_TRY(merge_distinct(m.get(), c->precv.p, precv_total, &c->pset, &set_slots));
   CUDA_TRY(cudaEventRecord(c->ev[4], st));

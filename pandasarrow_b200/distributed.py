@@ -13,6 +13,14 @@ exchange too (min / max of the 0 / 1 values).  Count_distinct needs a second exc
 Each rank ends up owning the groups with hash(key) % world == rank; `gather_result` concatenates
 the owners' results on every rank and restores global first-appearance order.
 
+Composite keys (group_by(["k1", "k2"])) travel as their packed 64-bit word.  How a shard packs depends on its data: a
+column carries a null bit only when the shard's slice of it has nulls, and a dictionary column is packed as its codes.
+So before the local pass every shard agrees on one layout (agree_key_layout: the null bits of all shards, identical
+widths and dictionaries) and repacks to it; then the same group is the same word, and has the same owner, everywhere.
+A utf8 column in a sharded composite key must therefore be dictionary-encoded ONCE, over the whole column, before it
+is sliced into shards: per-shard `dictionary_encode()` gives every shard its own codes, and the agreement fails with a
+dictionary-fingerprint error instead of merging different strings into one group.
+
 torch.distributed is plumbing only (rendezvous + the collective); the exchange helpers work on any
 backend, which is what the world_size-2 gloo tests exercise on CPU.
 """
@@ -74,6 +82,49 @@ def exchange_records(send, send_counts: Sequence[int], group=None, words: int = 
     return recv, recv_counts
 
 
+def agree_key_layout(gb, group=None):
+    """All-gather the composite key layout of every shard's GroupBy (any torch.distributed backend), agree on one
+    (pa_key_layout_agree: nullable wherever any shard has nulls; widths, bits and dictionaries must match, else PaError
+    on every rank) and repack `gb` to it.  Returns the agreed PaKeyLayout."""
+    import torch
+    import torch.distributed as dist
+    from ._lib import PaKeyLayout
+    from .groupby import PaError
+    world = dist.get_world_size(group)
+    err = None
+    try:
+        mine = gb.key_layout()
+    except PaError as e:          # still take part in the gather (n_keys = 0): every rank then fails together
+        err, mine = e, PaKeyLayout()
+    t = torch.tensor(list(bytes(mine)), dtype=torch.uint8)
+    if dist.get_backend(group) == "nccl":
+        t = t.cuda()
+    parts = [torch.empty_like(t) for _ in range(world)]
+    dist.all_gather(parts, t, group=group)
+    if err is not None:
+        raise err
+    agreed = agree_layouts([PaKeyLayout.from_buffer_copy(bytes(p.cpu().tolist())) for p in parts])
+    gb.set_key_layout(agreed)
+    return agreed
+
+
+def agree_layouts(layouts):
+    """pa_key_layout_agree over every shard's PaKeyLayout: the one layout all of them pack with (PaError when they
+    cannot agree)."""
+    import ctypes as C
+    from . import _lib
+    from ._lib import PaKeyLayout
+    from .groupby import _check
+    all_ = (PaKeyLayout * len(layouts))(*layouts)
+    agreed = PaKeyLayout()
+    _check(_lib.load().pa_key_layout_agree(all_, len(layouts), C.byref(agreed)))
+    return agreed
+
+
+def _composite(gb) -> bool:
+    return len(getattr(gb, "key_names", ())) > 1
+
+
 class Comm:
     """pa_comm (include/pa_b200.h): an NCCL communicator owned by libpa_b200.so.  The unique id travels over the
     already initialised torch.distributed group (any backend); after that the whole sharded step — local pass, owner
@@ -116,7 +167,19 @@ class Comm:
             _check(self._L.pa_groupby_sharded_aggregate(gb._h, self._h, C.byref(arg.dev), C.byref(arg.schema), mask, C.byref(h)))
         finally:
             arg.close()
-        return MergedGroupBy._from_handle(h)
+        m = MergedGroupBy._from_handle(h)
+        if _composite(gb):
+            m._adopt_keys(gb.key_names, gb._dicts)
+        return m
+
+    def key_layout_info(self) -> Dict[str, float]:
+        """Composite-key agreement of the last step (pa_comm_last_key_layout): device ms of the layout gather and of the
+        repack (0 when none happened)."""
+        import ctypes as C
+        from .groupby import _check
+        a, r = C.c_double(), C.c_double()
+        _check(self._L.pa_comm_last_key_layout(self._h, C.byref(a), C.byref(r)))
+        return {"agree_ms": a.value, "repack_ms": r.value}
 
     def phases(self) -> Dict[str, float]:
         import ctypes as C
@@ -166,10 +229,13 @@ def exchange_padded(send_blocks, group=None):
     return recv
 
 
-def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_format: str, group=None, stream=None,
+def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_format, group=None, stream=None,
                       padded: Optional[bool] = None, wait: bool = True, tail_stream=None):
     """Run the whole multi-GPU step for this rank.  `gb` is this rank's GroupBy over its row shard
     (created with row_base = first global row of the shard).  Returns the owner-side MergedGroupBy.
+
+    Composite key: the shards first agree on one key layout (agree_key_layout, one all-gather); `key_format` may then
+    be the list of key column formats, or None to take them (and the dictionaries unique() wraps) from `gb`.
 
     With few groups (<= PADDED_BLOCK_RECORDS on this rank) the partials travel in fixed-size blocks: one
     stream-ordered export kernel, one equal-split all-to-all, one merge — no host round trip in between.  A rank
@@ -198,6 +264,16 @@ def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_fo
     if padded is None:
         padded = stream is not None and stream == torch.cuda.current_stream(dev).cuda_stream
     padded = padded and not stage2 and not any(a in ("all", "any", "count_distinct") for a in aggs)
+    composite = _composite(gb)
+    if composite:
+        layout = agree_key_layout(gb, group)
+        key_formats = list(key_format) if isinstance(key_format, (list, tuple)) else gb.key_formats
+        key_format = "L"            # the records carry the packed word
+
+    def adopt(merged):
+        if composite:
+            merged.set_composite_key(layout, key_formats, gb.key_names, gb._dicts)
+        return merged
     # padded path: the local pass is only queued (no status read-back); export, exchange and merge are queued
     # behind it, so the host never waits before the merge's own result read.  A local pass that did not fit
     # the optimistic path makes the export send overflow markers, and everything is redone synchronously below.
@@ -209,8 +285,8 @@ def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_fo
         try:
             if tail_stream is None:
                 recv = exchange_padded(send, group)
-                merged = MergedGroupBy(recv.data_ptr(), [0] * world, aggs, value_format, key_format, device=dev.index,
-                                       stream=stream, padded_block_records=cap)
+                merged = adopt(MergedGroupBy(recv.data_ptr(), [0] * world, aggs, value_format, key_format, device=dev.index,
+                                             stream=stream, padded_block_records=cap))
             else:
                 done = torch.cuda.Event()
                 done.record(torch.cuda.current_stream(dev))
@@ -218,8 +294,8 @@ def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_fo
                 with torch.cuda.stream(tail_stream):
                     tail_stream.wait_event(done)
                     recv = exchange_padded(send, group)
-                    merged = MergedGroupBy(recv.data_ptr(), [0] * world, aggs, value_format, key_format, device=dev.index,
-                                           stream=tail_stream.cuda_stream, padded_block_records=cap)
+                    merged = adopt(MergedGroupBy(recv.data_ptr(), [0] * world, aggs, value_format, key_format, device=dev.index,
+                                                 stream=tail_stream.cuda_stream, padded_block_records=cap))
             merged._keep = (send, recv)
             if wait:
                 merged.groupSize()          # completes the merge; raises if any rank sent the overflow marker
@@ -238,8 +314,8 @@ def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_fo
 
     send, recv, recv_counts = counted_exchange(gb.partials_count, functools.partial(gb.partials_export, stage2=stage2),
                                                PA_PARTIAL_WORDS_STAGE2 if stage2 else PA_PARTIAL_WORDS)
-    merged = MergedGroupBy(recv.data_ptr(), recv_counts, [a for a in aggs if a != "count_distinct"], value_format, key_format,
-                           device=dev.index, stream=stream)
+    merged = adopt(MergedGroupBy(recv.data_ptr(), recv_counts, [a for a in aggs if a != "count_distinct"], value_format, key_format,
+                                 device=dev.index, stream=stream))
     merged._keep = (send, recv)
     if distinct:
         _, precv, precv_counts = counted_exchange(gb.distinct_pairs_count, gb.distinct_pairs_export, PA_DISTINCT_PAIR_WORDS)

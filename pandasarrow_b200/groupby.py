@@ -18,7 +18,7 @@ import pyarrow as pa
 
 from . import _lib
 from ._lib import (ARROW_DEVICE_CPU, ARROW_DEVICE_CUDA, PA_AGG, ArrowArray, ArrowDeviceArray, ArrowSchema,
-                   PaOptions)
+                   PaKeyLayout, PaOptions)
 
 _RELEASE_ARRAY = C.CFUNCTYPE(None, C.POINTER(ArrowArray))
 _RELEASE_SCHEMA = C.CFUNCTYPE(None, C.POINTER(ArrowSchema))
@@ -193,6 +193,7 @@ class GroupBy:
         key_arrays = [self._normalise_key(k) for k in key_arrays]
         args, devs, schemas = _pack_args(key_arrays)
         self._key_args = args          # keys are borrowed until destroy
+        self.key_formats = [a.schema.format.decode() for a in args]   # (dictionary columns: the index format)
         opt = _options(expected_groups, path, device, stream, row_base, no_dense, no_partition, bucket_bits, sm_reserve)
         try:
             _check(self._L.pa_groupby_create(devs, schemas, len(args), C.byref(opt), C.byref(self._h)))
@@ -256,6 +257,17 @@ class GroupBy:
         if d is not None:
             out = pa.DictionaryArray.from_arrays(out, d)
         return out
+
+    def key_layout(self) -> PaKeyLayout:
+        """pa_groupby_key_layout: how this composite key packs into 64 bits (with its dictionaries' fingerprints)."""
+        out = PaKeyLayout()
+        _check(self._L.pa_groupby_key_layout(self._h, C.byref(out)))
+        return out
+
+    def set_key_layout(self, layout: PaKeyLayout):
+        """pa_groupby_set_key_layout: repack the composite key under `layout` (one that all shards agreed on, see
+        distributed.agree_key_layout); groups and results of earlier aggregates are dropped."""
+        _check(self._L.pa_groupby_set_key_layout(self._h, C.byref(layout)))
 
     def first_rows(self) -> pa.Array:
         """Global row number of the first row of every group (result order)."""
@@ -431,6 +443,18 @@ class MergedGroupBy(GroupBy):
         _check(self._L.pa_merge_create(records_ptr, counts, len(counts_by_source), mask, value_format.encode(),
                                        key_format.encode(), C.byref(opt), C.byref(self._h)))
 
+    def set_composite_key(self, layout: PaKeyLayout, key_formats: Sequence[str], key_names: Optional[Sequence[str]] = None,
+                          dictionaries: Optional[Sequence[Optional[pa.Array]]] = None):
+        """pa_merge_set_key_layout: the records were merged by their packed composite key (key format "L"); unique(j)
+        then returns key column j (`key_formats[j]`: a dictionary column's index format, wrapped with
+        dictionaries[j])."""
+        fmts = (C.c_char_p * len(key_formats))(*[f.encode() for f in key_formats])
+        _check(self._L.pa_merge_set_key_layout(self._h, C.byref(layout), fmts))
+        self._adopt_keys(key_names or [f"key{j}" for j in range(len(key_formats))], dictionaries or [None] * len(key_formats))
+
+    def _adopt_keys(self, key_names, dictionaries):
+        self.key_names, self._dicts = list(key_names), list(dictionaries)
+
     def merge_distinct_pairs(self, pairs_ptr: int, counts_by_source: Sequence[int]):
         """Adds count_distinct (fetch("count_distinct")) from the received distinct-pair records, grouped by source."""
         counts = (C.c_int64 * len(counts_by_source))(*[int(c) for c in counts_by_source])
@@ -448,22 +472,37 @@ def _merged_from_handle(h) -> "MergedGroupBy":
 MergedGroupBy._from_handle = staticmethod(_merged_from_handle)
 
 
-def aggregate_chunked(keys: pa.Array, values: pa.Array, aggs: Sequence[str], chunk_rows: int, *, device: Optional[int] = None,
+def aggregate_chunked(keys, values: pa.Array, aggs: Sequence[str], chunk_rows: int, *, device: Optional[int] = None,
                       row_base: int = 0) -> "MergedGroupBy":
     """Host columns larger than the device (or than 2^32-2 rows): pa_groupby_aggregate_chunked — the columns are
-    aggregated `chunk_rows` rows at a time and the chunks' partial records merged like ranks'."""
+    aggregated `chunk_rows` rows at a time and the chunks' partial records merged like ranks'.  `keys`: one key array,
+    or a list of them (a composite key: utf8 members are dictionary-encoded once over the whole column; unique(j)
+    returns a DictionaryArray for dictionary columns)."""
     mask = 0
     for a in aggs:
         mask |= PA_AGG[a]
-    ka, va = _CArg(keys), _CArg(values)
+    composite = isinstance(keys, (list, tuple))
+    key_list = list(keys) if composite else [keys]
+    if composite:
+        key_list = [k.combine_chunks() if isinstance(k, pa.ChunkedArray) else k for k in key_list]
+        key_list = [k.dictionary_encode() if isinstance(k, pa.Array) and (pa.types.is_string(k.type) or pa.types.is_large_string(k.type))
+                    else k for k in key_list]
+    args, devs, schemas = _pack_args(key_list)
+    va = _CArg(values)
     h = C.c_void_p()
     opt = _options(0, "auto", device, None, row_base=row_base)
     try:
-        _check(_lib.load().pa_groupby_aggregate_chunked(C.byref(ka.dev), C.byref(ka.schema), C.byref(va.dev), C.byref(va.schema),
-                                                        mask, int(chunk_rows), C.byref(opt), C.byref(h)))
+        _check(_lib.load().pa_groupby_aggregate_chunked_keys(devs, schemas, len(args), C.byref(va.dev), C.byref(va.schema),
+                                                             mask, int(chunk_rows), C.byref(opt), C.byref(h)))
     finally:
-        ka.close(); va.close()
-    return MergedGroupBy._from_handle(h)
+        for a in args:
+            a.close()
+        va.close()
+    m = MergedGroupBy._from_handle(h)
+    if composite:
+        m._adopt_keys([f"key{j}" for j in range(len(key_list))],
+                      [k.dictionary if isinstance(k, pa.DictionaryArray) else None for k in key_list])
+    return m
 
 
 class Resampler(GroupBy):
