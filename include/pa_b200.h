@@ -340,7 +340,7 @@ int pa_merge_create(const void* dev_records, const int64_t* counts_by_source, in
 #define PA_DISTINCT_PAIR_WORDS 3
 /* Number of this handle's distinct pairs owned by each of n_parts ranks (1 <= n_parts <= 64), routed like the group
  * records (the null key goes to rank 0).  PA_ERR_STATE when the last aggregate did not compute count_distinct or the
- * handle is merged; composite and utf8 keys as pa_groupby_partials_count. */
+ * handle is merged.  Pairs of a utf8 key carry its hash: merge them after pa_merge_key_strings. */
 int pa_groupby_distinct_pairs_count(pa_groupby* g, int32_t n_parts, int64_t* counts_host);
 /* Writes the pairs, grouped by owner rank in ascending order, into caller-provided DEVICE memory (capacity_pairs >= sum of
  * counts).  Must follow pa_groupby_distinct_pairs_count with the same n_parts. */
@@ -364,6 +364,44 @@ int pa_merge_distinct_pairs(pa_groupby* merged, const void* dev_pairs, const int
 int pa_groupby_partials_export_padded(pa_groupby* g, int32_t n_parts, void* dev_blocks, int64_t block_records);
 int pa_merge_create_padded(const void* dev_blocks, int32_t n_sources, int64_t block_records, uint32_t agg_mask,
                            const char* value_format, const char* key_format, const pa_options* opt, pa_groupby** out);
+
+/* ---- utf8 / large_utf8 keys across shards ----
+ * A single utf8 key is grouped by a seeded 64-bit hash of its bytes, and its records carry that hash as their key word.
+ * Two things make the records alone unsafe across shards: a handle whose own byte check found two strings under one
+ * hash re-hashes with the next seed (so shards may hash one string differently), and two strings of different shards
+ * may share a hash (which no shard can see).  So every record travels with its group's key bytes, all shards hash with
+ * one seed, and the owner compares the bytes of every record of a merged group with those of its representative (the
+ * record carrying the group's global first row: the first string in row order).  The plain pa_groupby_partials_count /
+ * _export / _export_stage2 / _export_padded and pa_merge_create_padded refuse utf8 keys.
+ *
+ * The hash seed of a handle with one utf8 / large_utf8 key (0 at creation, raised by the handle's own check on a
+ * collision); PA_ERR_INVALID for any other handle. */
+int pa_groupby_key_hash_seed(pa_groupby* g, uint64_t* seed);
+/* Re-hashes the key column with `seed` (the largest seed of all shards, see pa_merge_key_strings).  Completes a pending
+ * aggregate first; groups, outputs, groupings, distinct pairs and stage-2 terms are dropped like pa_groupby_set_key_layout
+ * does, and the next aggregate checks the grouping byte for byte again (which may raise the seed once more).  Equal to
+ * the current seed: no-op.  PA_ERR_INVALID for a handle that is not a single utf8 key. */
+int pa_groupby_set_key_hash_seed(pa_groupby* g, uint64_t seed);
+/* Records (as pa_groupby_partials_count) and key bytes owned by each of n_parts ranks, after an aggregate. */
+int pa_groupby_partials_count_utf8(pa_groupby* g, int32_t n_parts, int64_t* records_host, int64_t* bytes_host);
+/* Writes the records (PA_PARTIAL_WORDS words, or PA_PARTIAL_WORDS_STAGE2 when stage2 != 0, as
+ * pa_groupby_partials_export / _export_stage2), one uint32 key length per record (0 for the null key) and the key
+ * bytes, all grouped by owner rank in the same order, into caller-provided DEVICE memory (capacity_records >= the
+ * records, capacity_bytes >= the key bytes of pa_groupby_partials_count_utf8, which must come first with the same
+ * n_parts).  Record i's bytes follow those of records 0 .. i-1. */
+int pa_groupby_partials_export_utf8(pa_groupby* g, int32_t n_parts, int32_t stage2, void* dev_records, int64_t capacity_records,
+                                    void* dev_lengths, void* dev_bytes, int64_t capacity_bytes);
+/* Owner side, on a handle made by pa_merge_create with key_format "u" / "U" from utf8 records (whose record buffer must
+ * still be alive): attaches the merged groups' key strings from the received lengths and bytes (DEVICE memory, grouped
+ * by source like the records; records_by_source as given to pa_merge_create, bytes_by_source and every source's hash
+ * seed on the host).  Every record's bytes are compared with its group's representative's; when two different strings
+ * share a merged group, *collided = 1, no strings are attached, and the caller's ranks agree a retry with the next seed
+ * (4 seeds at most).  Otherwise *collided = 0 and pa_groupby_unique(merged, 0) returns utf8 (key_format "u") or
+ * large_utf8 ("U"); before that it returns PA_ERR_STATE, and so does pa_merge_distinct_pairs.  The merged handle keeps
+ * only its G representative strings.  PA_ERR_INVALID when the seeds differ: hashes of one string under two seeds are
+ * two groups, which nothing after the merge can detect. */
+int pa_merge_key_strings(pa_groupby* merged, const void* dev_lengths, const void* dev_bytes, const int64_t* records_by_source,
+                         const int64_t* bytes_by_source, const uint64_t* seed_by_source, int32_t n_sources, int32_t* collided);
 
 /* ---- composite keys across shards ----
  * A composite key is packed into one 64-bit word per row: column j takes bits[j] value bits, then one null bit when
@@ -406,6 +444,9 @@ int pa_merge_set_key_layout(pa_groupby* merged, const pa_key_layout* layout, con
  * partial records — and the chunks' records are merged like ranks' (sources folded in row order, groups in global
  * first-appearance order).  Single key column; sum / mean / count / min / max / first / last / product / variance / stddev
  * (those three travel in PA_PARTIAL_WORDS_STAGE2-word records) and all / any of boolean columns; not count_distinct.
+ * A utf8 / large_utf8 key: every chunk hashes with one seed and exports its key bytes next to its records; a chunk
+ * whose own check raises the seed, or a merge that finds two strings under one hash, redoes the chunks with the next
+ * seed (4 at most).
  * `merged_out` answers
  * num_groups / unique / fetch like a merged multi-GPU handle.  At most 64 chunks.
  * pa_groupby_aggregate_chunked is pa_groupby_aggregate_chunked_keys with n_keys = 1. */
@@ -434,8 +475,12 @@ int pa_groupby_aggregate_chunked_keys(const struct ArrowDeviceArray* keys, const
  * (pa_merge_distinct_pairs); pair send / receive / set scratch stays on the communicator too.  A composite key handle
  * starts every step with one more ncclAllGather, of every rank's pa_key_layout, agrees on a layout
  * (pa_key_layout_agree; all ranks fail together when the layouts do not agree), repacks when it differs from the
- * handle's own (pa_groupby_set_key_layout) and hands the merged handle that layout and its key formats.  Single-key
- * and resample steps issue no extra collective. */
+ * handle's own (pa_groupby_set_key_layout) and hands the merged handle that layout and its key formats.  A utf8 key
+ * handle adds its hash seed and its key bytes per owner to the count gather; when the seeds differ every rank re-hashes
+ * with the largest and redoes the step.  The key lengths and bytes follow the records in one more grouped send /
+ * receive, the owner checks them (pa_merge_key_strings), and one ncclAllReduce (max) of the collision word follows;
+ * after a collision every rank redoes the step with the next seed.  Four seeds at most, then PA_ERR_STATE on every rank.
+ * Other single-key and resample steps issue no extra collective. */
 #define PA_COMM_ID_BYTES 128
 typedef struct pa_comm pa_comm;
 int pa_comm_unique_id(void* out_id, int64_t capacity_bytes);
@@ -457,6 +502,9 @@ int pa_comm_last_distinct(pa_comm* c, int64_t* pairs_sent, int64_t* pairs_receiv
  * ncclAllGather, copy out) and of the repack (0 when the handle already packed with the agreed layout); both 0 for a
  * single-key or resample step. */
 int pa_comm_last_key_layout(pa_comm* c, double* agree_ms, double* repack_ms);
+/* The last step's utf8 key exchange: key bytes this rank sent and received, the seed all ranks hashed with, and the
+ * number of attempts the step took (1 without a seed change); all 0 for a step without a utf8 key. */
+int pa_comm_last_key_strings(pa_comm* c, int64_t* bytes_sent, int64_t* bytes_received, uint64_t* seed, int32_t* attempts);
 
 /* ---- synthetic workload generator (SURVEY.md §8d), used by bench.py and the tests so that the
  * same counter-based splitmix64 streams exist on host and device without PCIe staging.

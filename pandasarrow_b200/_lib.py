@@ -36,6 +36,8 @@ EXPORTS = [
     "pa_comm_last_distinct",
     "pa_groupby_key_layout", "pa_key_layout_agree", "pa_groupby_set_key_layout", "pa_merge_set_key_layout",
     "pa_groupby_aggregate_chunked_keys", "pa_comm_last_key_layout",
+    "pa_groupby_key_hash_seed", "pa_groupby_set_key_hash_seed", "pa_groupby_partials_count_utf8", "pa_groupby_partials_export_utf8",
+    "pa_merge_key_strings", "pa_comm_last_key_strings",
 ]
 
 
@@ -171,6 +173,13 @@ def load():
     L.pa_comm_last_exchange.argtypes = [P, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int64)]
     L.pa_comm_last_distinct.argtypes = [P, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
     L.pa_comm_last_key_layout.argtypes = [P, C.POINTER(C.c_double), C.POINTER(C.c_double)]
+    L.pa_groupby_key_hash_seed.argtypes = [P, C.POINTER(C.c_uint64)]
+    L.pa_groupby_set_key_hash_seed.argtypes = [P, C.c_uint64]
+    L.pa_groupby_partials_count_utf8.argtypes = [P, C.c_int32, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+    L.pa_groupby_partials_export_utf8.argtypes = [P, C.c_int32, C.c_int32, P, C.c_int64, P, P, C.c_int64]
+    L.pa_merge_key_strings.argtypes = [P, P, P, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_uint64), C.c_int32,
+                                       C.POINTER(C.c_int32)]
+    L.pa_comm_last_key_strings.argtypes = [P, C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_uint64), C.POINTER(C.c_int32)]
     L.pa_synth_keys_i64.argtypes = [P, C.c_int64, C.c_int64, C.c_uint64, C.c_uint64, P]
     L.pa_synth_vals_f64.argtypes = [P, C.c_int64, C.c_int64, C.c_uint64, P]
     L.pa_synth_validity.argtypes = [P, C.c_int64, C.c_int64, C.c_uint64, C.c_uint32, P]

@@ -2,6 +2,7 @@
 // marshalling from the Arrow C Data Interface, path selection, kernel launches, result export.
 // No computation happens on the host and there is no CPU fallback.
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 #include <cuda_runtime.h>
 #include <nccl.h>
 
@@ -344,13 +345,22 @@ int load_column(const ArrowDeviceArray* da, const ArrowSchema* sc, cudaStream_t 
   return PA_OK;
 }
 
+// Collision hook for tests (PA_TEST_STR_HASH_BITS=b): hashes made under seed 0 keep only their low b bits, so that
+// different strings share a hash on demand.  Unset: every bit is kept.
+uint64_t test_hash_keep(uint64_t seed) {
+  static const char* bits = getenv("PA_TEST_STR_HASH_BITS");
+  if (!bits || seed != 0) return ~0ull;
+  const int b = atoi(bits);
+  return b <= 0 ? 0ull : b >= 64 ? ~0ull : (1ull << b) - 1;
+}
+
 // utf8 / large_utf8 key column: offsets + bytes onto the device (or borrowed), then one 64-bit hash per row.
 int hash_string_key(Column* out, cudaStream_t st, int num_sms) {
   PA_TRY(out->own_data.alloc(static_cast<size_t>(std::max<int64_t>(out->n, 1)) * 8, st));
   if (out->n > 0) {
     const int grid = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((out->n + 255) / 256, static_cast<int64_t>(num_sms) * 16)));
     k_str_hash<<<grid, 256, 0, st>>>(out->str, out->valid, out->bit_off, out->n, 0x5851F42D4C957F2Dull + out->str_seed * 0x9E3779B97F4A7C15ull,
-                                     out->own_data.as<uint64_t>());
+                                     test_hash_keep(out->str_seed), out->own_data.as<uint64_t>());
     CUDA_TRY(cudaGetLastError());
   }
   out->data = out->own_data.p;
@@ -475,7 +485,15 @@ struct pa_groupby {
   // multi-GPU
   int parts_n = 0;
   std::vector<int64_t> parts_counts;
+  std::vector<int64_t> ks_counts;         // utf8 key: key bytes per owner (pa_groupby_partials_count_utf8)
   bool merged = false;
+  // merged handle of a utf8 key (key format "u" / "U"): its G representative strings once pa_merge_key_strings has
+  // attached them — int64 offsets, bytes, and rows 0 .. G-1 for unique_strings
+  bool ks_str = false, ks_have = false;
+  DevBuf ks_off, ks_bytes, ks_rows;
+  const void* ks_recs = nullptr;          // pa_merge_create's records (the caller's buffer), ks_nrec of ks_words words
+  int ks_words = 0;
+  uint64_t ks_nrec = 0;
   DevBuf m_count64, m_first_val, m_last_val, m_first_valid, m_last_valid, m_first_row_g;
   // bookkeeping
   DevBuf status;
@@ -1898,7 +1916,11 @@ int set_merged_formats(pa_groupby* g, const char* value_format, const char* key_
   g->packed = false;   // (pa_merge_set_key_layout makes it composite; a recycled handle may have been)
   g->keys.resize(1);
   int kw = 8, kvc = VC_I;
-  PA_TRY(parse_format(key_format, &kw, &kvc));
+  // utf8 key: the records' key word is the hash; the strings come with pa_merge_key_strings
+  g->ks_str = (key_format[0] == 'u' || key_format[0] == 'U') && key_format[1] == 0;
+  g->ks_have = false;
+  g->ks_off.reset(); g->ks_bytes.reset(); g->ks_rows.reset();
+  if (!g->ks_str) PA_TRY(parse_format(key_format, &kw, &kvc));
   g->keys[0].format = key_format;
   g->keys[0].width = kw;
   g->fields.assign(1, KeyField{});
@@ -2361,7 +2383,8 @@ int pa_groupby_num_groups(pa_groupby* g, int64_t* out) {
   return PA_OK;
 }
 
-static int unique_strings(pa_groupby* g, struct ArrowArray* out, struct ArrowSchema* out_schema);
+static int unique_strings(pa_groupby* g, const StrCol& col, const uint32_t* rows, bool large, struct ArrowArray* out,
+                          struct ArrowSchema* out_schema);
 
 int pa_groupby_unique(pa_groupby* g, int32_t key_i, struct ArrowArray* out, struct ArrowSchema* out_schema) {
   if (!g || !out || !out_schema) return set_err(PA_ERR_INVALID, "null argument");
@@ -2369,7 +2392,13 @@ int pa_groupby_unique(pa_groupby* g, int32_t key_i, struct ArrowArray* out, stru
   PA_TRY(ensure_device(g));
   if (!g->resample && !g->merged && g->keys.size() == 1 && g->keys[0].is_str) {
     if (key_i != 0) return set_err(PA_ERR_INVALID, "key index %d out of range", key_i);
-    return unique_strings(g, out, out_schema);
+    return unique_strings(g, g->keys[0].str, g->res.first_row, g->keys[0].str.wide != 0, out, out_schema);
+  }
+  if (g->merged && g->ks_str) {
+    if (key_i != 0) return set_err(PA_ERR_INVALID, "key index %d out of range", key_i);
+    if (!g->ks_have) return set_err(PA_ERR_STATE, "utf8 merged handle without its key strings: call pa_merge_key_strings first");
+    const StrCol col{g->ks_off.p, g->ks_bytes.as<uint8_t>(), 1};
+    return unique_strings(g, col, g->ks_rows.as<uint32_t>(), g->keys[0].format == "U", out, out_schema);
   }
   if (g->resample) {
     if (key_i != 0) return set_err(PA_ERR_INVALID, "key index %d out of range", key_i);
@@ -2638,15 +2667,16 @@ int ensure_groupings(pa_groupby* g) {
 }
 }  // namespace
 
-// unique() of a utf8 / large_utf8 key: the bytes of every group's first row, in group order (int32 offsets; a result
-// of more than 2 GiB of distinct strings is refused).
-static int unique_strings(pa_groupby* g, struct ArrowArray* out, struct ArrowSchema* out_schema) {
+// unique() of a utf8 / large_utf8 key: the bytes of col's row rows[g] for every group g, in group order — a local
+// handle's first rows in its key column, or a merged handle's compacted representatives — as utf8 (large: large_utf8)
+// with int32 offsets (a result of more than 2 GiB of distinct strings is refused).
+static int unique_strings(pa_groupby* g, const StrCol& col, const uint32_t* rows, bool large, struct ArrowArray* out,
+                          struct ArrowSchema* out_schema) {
   cudaStream_t st = g->stream;
   const uint32_t G = g->G;
-  const Column& k = g->keys[0];
   DevBuf offs, tile_sums, bytes, valid;
   PA_TRY(offs.alloc(static_cast<size_t>(G + 1) * 4, st));
-  k_str_lengths<<<(G + 1 + 255) / 256, 256, 0, st>>>(k.str, g->res.first_row, g->res.key_kind, G, offs.as<uint32_t>());
+  k_str_lengths<<<(G + 1 + 255) / 256, 256, 0, st>>>(col, rows, g->res.key_kind, G, offs.as<uint32_t>());
   CUDA_TRY(cudaGetLastError());
   uint64_t total64 = 0;
   {
@@ -2663,7 +2693,7 @@ static int unique_strings(pa_groupby* g, struct ArrowArray* out, struct ArrowSch
   PA_TRY(bytes.alloc(std::max<uint64_t>(total64, 1), st));
   PA_TRY(valid.alloc(((static_cast<size_t>(G) + 31) / 32 + 1) * 4, st));
   if (G) {
-    k_str_gather<<<(static_cast<uint64_t>(G) * 32 + 255) / 256, 256, 0, st>>>(k.str, g->res.first_row, g->res.key_kind, G, offs.as<uint32_t>(), bytes.as<uint8_t>());
+    k_str_gather<<<(static_cast<uint64_t>(G) * 32 + 255) / 256, 256, 0, st>>>(col, rows, g->res.key_kind, G, offs.as<uint32_t>(), bytes.as<uint8_t>());
     CUDA_TRY(cudaGetLastError());
     k_kind_validity<<<(G + 31) / 32 * 32 / 256 + 1, 256, 0, st>>>(g->res.key_kind, G, valid.as<uint32_t>());
     CUDA_TRY(cudaGetLastError());
@@ -2685,8 +2715,7 @@ static int unique_strings(pa_groupby* g, struct ArrowArray* out, struct ArrowSch
   for (size_t i = 0; i < words; ++i) set += __builtin_popcount(static_cast<const uint32_t*>(priv->bufs[0])[i]);
   const int64_t null_count = static_cast<int64_t>(G) - set;
   if (null_count == 0) { free(priv->bufs[0]); priv->bufs[0] = nullptr; }
-  const bool large = k.str.wide != 0;      // large_utf8 in, large_utf8 out (int64 offsets, widened on the host: G + 1 numbers)
-  if (large) {
+  if (large) {   // large_utf8 in, large_utf8 out (int64 offsets, widened on the host: G + 1 numbers)
     int64_t* wide = static_cast<int64_t*>(malloc(std::max<size_t>((static_cast<size_t>(G) + 1) * 8, 64)));
     for (size_t i = 0; i <= G; ++i) wide[i] = static_cast<const uint32_t*>(priv->bufs[1])[i];
     free(priv->bufs[1]);
@@ -3344,9 +3373,34 @@ int pa_sort_indices(pa_groupby* g, struct ArrowArray* out, struct ArrowSchema* o
 }
 
 // ---- multi-GPU partial export / merge ----
-// keys the exchange routes: one fixed-width column, a packed composite key or a resample index
+// keys the plain record exchange routes: one fixed-width column, a packed composite key or a resample index.  A utf8
+// key's record carries a hash the owner cannot check without the key bytes: the _utf8 entry points export both.
 static int check_shardable(const pa_groupby* g) {
-  if (!g->resample && g->keys[0].is_str) return set_err(PA_ERR_NOT_IMPLEMENTED, "multi-GPU merge of utf8 keys: dictionary-encode the column against a shared dictionary");
+  if (!g->resample && g->keys[0].is_str)
+    return set_err(PA_ERR_NOT_IMPLEMENTED, "partial records of utf8 keys need their key bytes: use pa_groupby_partials_count_utf8 / "
+                                           "pa_groupby_partials_export_utf8 (the padded exchange does not take utf8 keys)");
+  return PA_OK;
+}
+
+static bool is_str_key(const pa_groupby* g) { return !g->resample && !g->merged && g->keys.size() == 1 && g->keys[0].is_str; }
+
+// Drops everything computed from the handle's key words (after a repack or a rehash)
+static void drop_results(pa_groupby* g) {
+  g->have_groups = false; g->bk_have_hist = false; g->G = 0; g->outs.clear();
+  g->have_groupings = false;
+  g->parts_n = 0;
+  g->s2_ext = 0; g->s2_m2.reset(); g->s2_prod.reset();
+  g->cd_have = false; g->cd_n = 0; g->cd_id.reset(); g->cd_bits.reset(); g->dp_parts_n = 0;
+}
+
+// utf8 key: rehash the column with hash seed `seed` (strkeys.cuh); the next aggregate groups and checks anew
+static int set_str_seed(pa_groupby* g, uint64_t seed) {
+  if (g->keys[0].str_seed == seed) return PA_OK;
+  g->keys[0].str_seed = seed;
+  PA_TRY(hash_string_key(&g->keys[0], g->stream, g->num_sms));
+  g->key_data = g->keys[0].data;
+  g->str_verified = false;
+  drop_results(g);
   return PA_OK;
 }
 
@@ -3415,12 +3469,7 @@ int pa_groupby_set_key_layout(pa_groupby* g, const pa_key_layout* layout) {
   PA_TRY(layout_fields(*layout, &fields));
   g->fields = std::move(fields);
   PA_TRY(pack_keys(g));
-  // everything below was computed from the old key words
-  g->have_groups = false; g->bk_have_hist = false; g->G = 0; g->outs.clear();
-  g->have_groupings = false;
-  g->parts_n = 0;
-  g->s2_ext = 0; g->s2_m2.reset(); g->s2_prod.reset();
-  g->cd_have = false; g->cd_n = 0; g->cd_id.reset(); g->cd_bits.reset(); g->dp_parts_n = 0;
+  drop_results(g);
   return PA_OK;
 }
 
@@ -3540,7 +3589,6 @@ static int pairs_check(pa_groupby* g, int32_t n_parts) {
   if (n_parts < 1 || n_parts > 64) return set_err(PA_ERR_INVALID, "bad argument (1 <= n_parts <= 64)");
   PA_TRY(finish_pending(g));
   if (g->merged) return set_err(PA_ERR_STATE, "distinct pairs come from a local aggregate, not from a merged handle");
-  PA_TRY(check_shardable(g));
   if (!g->cd_have) return set_err(PA_ERR_STATE, "the last aggregate computed no count_distinct: no distinct pairs to export");
   return ensure_device(g);
 }
@@ -3611,6 +3659,12 @@ int pa_merge_create(const void* dev_records, const int64_t* counts_by_source, in
   for (int i = 0; i < n_sources; ++i)
     if (counts_by_source[i] < 0) return set_err(PA_ERR_INVALID, "negative record count");
   PA_TRY(merge_counted(g.get(), dev_records, counts_by_source, n_sources, agg_mask, value_format, key_format, nullptr, 0, false));
+  if (g->ks_str) {   // (pa_merge_key_strings maps these records to their groups; the caller keeps them alive until then)
+    g->ks_recs = dev_records;
+    g->ks_words = record_words(agg_mask, false);
+    g->ks_nrec = 0;
+    for (int i = 0; i < n_sources; ++i) g->ks_nrec += static_cast<uint64_t>(counts_by_source[i]);
+  }
   *out = g.release();
   return PA_OK;
 }
@@ -3676,6 +3730,8 @@ int pa_merge_distinct_pairs(pa_groupby* merged, const void* dev_pairs, const int
   if (!merged || !counts_by_source || n_sources < 1) return set_err(PA_ERR_INVALID, "null argument");
   PA_TRY(finish_pending(merged));
   if (!merged->merged || !merged->have_groups) return set_err(PA_ERR_STATE, "distinct pairs merge into a handle made by pa_merge_create");
+  if (merged->ks_str && !merged->ks_have)
+    return set_err(PA_ERR_STATE, "utf8 merged handle: attach the key strings with pa_merge_key_strings before merging distinct pairs");
   uint64_t total = 0;
   for (int i = 0; i < n_sources; ++i) {
     if (counts_by_source[i] < 0) return set_err(PA_ERR_INVALID, "negative pair count");
@@ -3685,6 +3741,201 @@ int pa_merge_distinct_pairs(pa_groupby* merged, const void* dev_pairs, const int
   if (total && !dev_pairs) return set_err(PA_ERR_INVALID, "null pair buffer");
   PA_TRY(ensure_device(merged));
   return merge_distinct(merged, dev_pairs, total, nullptr, nullptr);
+}
+
+// ---- utf8 keys across shards: the key bytes travel with the records (strkeys.cuh) ----
+// In-place exclusive scan of n 64-bit words (cub); `tmp`: its scratch
+static int scan_u64(cudaStream_t st, unsigned long long* data, uint64_t n, DevBuf* tmp) {
+  size_t bytes = 0;
+  CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, bytes, data, static_cast<int64_t>(n), st));
+  PA_TRY(tmp->alloc(std::max<size_t>(bytes, 1), st));
+  CUDA_TRY(cub::DeviceScan::ExclusiveSum(tmp->p, bytes, data, static_cast<int64_t>(n), st));
+  return PA_OK;
+}
+
+// Stream ordered: key bytes per owner of the G local groups (GroupResult, or the unordered bucket records when
+// `unordered_recs` is given) added into d_bytes[0 .. n_parts)
+static int keystr_count_async(pa_groupby* g, int32_t n_parts, const void* unordered_recs, uint32_t G, unsigned long long* d_bytes) {
+  if (!G) return PA_OK;
+  if (unordered_recs)
+    k_keystr_count_bk<<<(G + 255) / 256, 256, 0, g->stream>>>(g->keys[0].str, static_cast<const BkRec32*>(unordered_recs), G, static_cast<uint32_t>(n_parts), d_bytes);
+  else
+    k_keystr_count<<<(G + 255) / 256, 256, 0, g->stream>>>(g->keys[0].str, g->res, G, static_cast<uint32_t>(n_parts), d_bytes);
+  CUDA_TRY(cudaGetLastError());
+  return PA_OK;
+}
+
+// Lengths and key bytes of n exported records (`words` wide, in the order they were written): lengths[i], and the bytes
+// at the exclusive prefix of the lengths — owner segments are contiguous, so the bytes are grouped by owner too.
+// `off`, `tmp`: scratch.  Stream ordered.
+static int keystr_export(pa_groupby* g, const uint64_t* recs, int words, uint64_t n, uint32_t* lengths, uint8_t* bytes, DevBuf* off, DevBuf* tmp) {
+  cudaStream_t st = g->stream;
+  PA_TRY(off->alloc((n + 1) * 8, st));
+  k_keystr_lengths<<<static_cast<unsigned>((n + 1 + 255) / 256), 256, 0, st>>>(g->keys[0].str, recs, words, n, g->opt.row_base, lengths,
+                                                                                off->as<unsigned long long>());
+  CUDA_TRY(cudaGetLastError());
+  PA_TRY(scan_u64(st, off->as<unsigned long long>(), n + 1, tmp));
+  if (n) {
+    k_keystr_pack<<<static_cast<unsigned>((n * 32 + 255) / 256), 256, 0, st>>>(g->keys[0].str, recs, words, n, g->opt.row_base,
+                                                                               off->as<unsigned long long>(), bytes);
+    CUDA_TRY(cudaGetLastError());
+  }
+  return PA_OK;
+}
+
+// Owner side, after the record merge: the received records (`words` wide, nrec, as merged) with their lengths and key
+// bytes -> merged group and representative of every record, byte check against the representative.  Attaches the G
+// representative strings, compacted, to m — unless two different strings share a merged group: then *collided and
+// nothing is attached (the ranks retry with the next hash seed).  `bytes_expected`: what the sources say they sent.
+static int merge_key_strings(pa_groupby* m, const uint64_t* recs, int words, uint64_t nrec, const uint32_t* lengths, const uint8_t* bytes,
+                             uint64_t bytes_expected, bool* collided) {
+  cudaStream_t st = m->stream;
+  const uint32_t G = m->G;
+  *collided = false;
+  m->ks_have = false;
+  DevBuf off, tmp, rec_group, rep, flag, out_off;
+  PA_TRY(off.alloc((nrec + 1) * 8, st));
+  k_keystr_widen<<<static_cast<unsigned>((nrec + 1 + 255) / 256), 256, 0, st>>>(lengths, nrec, off.as<unsigned long long>());
+  CUDA_TRY(cudaGetLastError());
+  PA_TRY(scan_u64(st, off.as<unsigned long long>(), nrec + 1, &tmp));
+  PA_TRY(flag.alloc(4, st));
+  CUDA_TRY(cudaMemsetAsync(flag.p, 0, 4, st));
+  PA_TRY(rep.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 4, st));
+  CUDA_TRY(cudaMemsetAsync(rep.p, 0xFF, static_cast<size_t>(std::max<uint32_t>(G, 1)) * 4, st));
+  PA_TRY(out_off.alloc((static_cast<size_t>(G) + 1) * 8, st));
+  RowLookup lk;
+  if (nrec) {
+    PA_TRY(build_row_lookup(m, &lk));
+    PA_TRY(rec_group.alloc(nrec * 4, st));
+    k_keystr_rep<<<static_cast<unsigned>((nrec + 255) / 256), 256, 0, st>>>(recs, words, nrec, lk.a, m->m_first_row_g.as<uint64_t>(),
+                                                                           rec_group.as<uint32_t>(), rep.as<uint32_t>(), flag.as<uint32_t>());
+    CUDA_TRY(cudaGetLastError());
+    k_keystr_verify<<<static_cast<unsigned>((nrec * 32 + 255) / 256), 256, 0, st>>>(recs, words, nrec, rec_group.as<uint32_t>(), rep.as<uint32_t>(),
+                                                                                    off.as<unsigned long long>(), bytes, G, flag.as<uint32_t>());
+    CUDA_TRY(cudaGetLastError());
+  }
+  k_keystr_rep_lengths<<<(G + 1 + 255) / 256, 256, 0, st>>>(rep.as<uint32_t>(), m->res.key_kind, G, off.as<unsigned long long>(),
+                                                            out_off.as<unsigned long long>(), flag.as<uint32_t>());
+  CUDA_TRY(cudaGetLastError());
+  PA_TRY(scan_u64(st, out_off.as<unsigned long long>(), static_cast<uint64_t>(G) + 1, &tmp));
+  uint32_t h_flag = 0;
+  uint64_t h_total[2] = {0, 0};
+  CUDA_TRY(cudaMemcpyAsync(&h_flag, flag.p, 4, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaMemcpyAsync(&h_total[0], off.as<uint64_t>() + nrec, 8, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaMemcpyAsync(&h_total[1], out_off.as<uint64_t>() + G, 8, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaStreamSynchronize(st));
+  if (h_total[0] != bytes_expected)
+    return set_err(PA_ERR_INVALID, "the key-string lengths add up to %llu bytes, the sources sent %llu", (unsigned long long)h_total[0],
+                   (unsigned long long)bytes_expected);
+  if (h_flag & KS_NO_GROUP)
+    return set_err(PA_ERR_STATE, "key strings do not match the merged records (a record names no merged group, or a group has no representative)");
+  if (h_flag & KS_COLLISION) {
+    *collided = true;
+    return PA_OK;
+  }
+  PA_TRY(m->ks_bytes.alloc(std::max<uint64_t>(h_total[1], 1), st));
+  PA_TRY(m->ks_rows.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * 4, st));
+  if (G) {
+    k_keystr_rep_gather<<<static_cast<unsigned>((static_cast<uint64_t>(G) * 32 + 255) / 256), 256, 0, st>>>(
+        rep.as<uint32_t>(), G, off.as<unsigned long long>(), bytes, out_off.as<unsigned long long>(), m->ks_bytes.as<uint8_t>());
+    CUDA_TRY(cudaGetLastError());
+    k_iota_u32<<<(G + 255) / 256, 256, 0, st>>>(m->ks_rows.as<uint32_t>(), G);
+    CUDA_TRY(cudaGetLastError());
+  }
+  m->ks_off = std::move(out_off);
+  CUDA_TRY(cudaStreamSynchronize(st));   // the caller's record / byte buffers are read by now
+  m->ks_have = true;
+  return PA_OK;
+}
+
+int pa_groupby_key_hash_seed(pa_groupby* g, uint64_t* seed) {
+  if (!g || !seed) return set_err(PA_ERR_INVALID, "null argument");
+  if (!is_str_key(g)) return set_err(PA_ERR_INVALID, "key hash seeds belong to a pa_groupby_create handle with one utf8 / large_utf8 key");
+  *seed = g->keys[0].str_seed;
+  return PA_OK;
+}
+
+int pa_groupby_set_key_hash_seed(pa_groupby* g, uint64_t seed) {
+  if (!g) return set_err(PA_ERR_INVALID, "null argument");
+  if (!is_str_key(g)) return set_err(PA_ERR_INVALID, "key hash seeds belong to a pa_groupby_create handle with one utf8 / large_utf8 key");
+  PA_TRY(ensure_device(g));
+  PA_TRY(finish_pending(g));
+  return set_str_seed(g, seed);
+}
+
+int pa_groupby_partials_count_utf8(pa_groupby* g, int32_t n_parts, int64_t* records_host, int64_t* bytes_host) {
+  if (!g || !records_host || !bytes_host || n_parts < 1 || n_parts > 64) return set_err(PA_ERR_INVALID, "bad argument (1 <= n_parts <= 64)");
+  PA_TRY(finish_pending(g));
+  if (!g->have_groups || g->merged) return set_err(PA_ERR_STATE, "partials need a finished local aggregate");
+  if (!is_str_key(g)) return set_err(PA_ERR_INVALID, "pa_groupby_partials_count_utf8 takes one utf8 / large_utf8 key; use pa_groupby_partials_count");
+  PA_TRY(ensure_device(g));
+  cudaStream_t st = g->stream;
+  DevBuf counts;
+  PA_TRY(counts.alloc(sizeof(uint64_t) * 2 * n_parts, st));
+  CUDA_TRY(cudaMemsetAsync(counts.p, 0, sizeof(uint64_t) * 2 * n_parts, st));
+  PA_TRY(partials_count_async(g, n_parts, counts.as<unsigned long long>()));
+  PA_TRY(keystr_count_async(g, n_parts, nullptr, g->G, counts.as<unsigned long long>() + n_parts));
+  std::vector<uint64_t> h(static_cast<size_t>(2 * n_parts));
+  CUDA_TRY(cudaMemcpyAsync(h.data(), counts.p, sizeof(uint64_t) * 2 * n_parts, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaStreamSynchronize(st));
+  for (int i = 0; i < n_parts; ++i) {
+    records_host[i] = static_cast<int64_t>(h[i]);
+    bytes_host[i] = static_cast<int64_t>(h[n_parts + i]);
+  }
+  g->parts_n = n_parts;
+  g->parts_counts.assign(records_host, records_host + n_parts);
+  g->ks_counts.assign(bytes_host, bytes_host + n_parts);
+  return PA_OK;
+}
+
+int pa_groupby_partials_export_utf8(pa_groupby* g, int32_t n_parts, int32_t stage2, void* dev_records, int64_t capacity_records,
+                                    void* dev_lengths, void* dev_bytes, int64_t capacity_bytes) {
+  if (!g || !dev_records) return set_err(PA_ERR_INVALID, "null argument");
+  if (g->merged) return set_err(PA_ERR_STATE, "partials need a finished local aggregate");
+  if (!is_str_key(g)) return set_err(PA_ERR_INVALID, "pa_groupby_partials_export_utf8 takes one utf8 / large_utf8 key; use pa_groupby_partials_export");
+  if (g->parts_n != n_parts || g->ks_counts.size() != static_cast<size_t>(n_parts))
+    return set_err(PA_ERR_STATE, "call pa_groupby_partials_count_utf8(n_parts=%d) first", n_parts);
+  int64_t total = 0;
+  for (int64_t b : g->ks_counts) total += b;
+  if (capacity_bytes < total) return set_err(PA_ERR_INVALID, "key byte buffer too small (%lld bytes, %lld needed)", (long long)capacity_bytes, (long long)total);
+  if ((g->G && !dev_lengths) || (total && !dev_bytes)) return set_err(PA_ERR_INVALID, "null length / byte buffer");
+  const int words = stage2 ? REC_WORDS_STAGE2 : REC_WORDS;
+  PA_TRY(partials_export(g, n_parts, dev_records, capacity_records, words));
+  DevBuf off, tmp;
+  PA_TRY(keystr_export(g, static_cast<const uint64_t*>(dev_records), words, g->G, static_cast<uint32_t*>(dev_lengths), static_cast<uint8_t*>(dev_bytes),
+                       &off, &tmp));
+  CUDA_TRY(cudaStreamSynchronize(g->stream));
+  return PA_OK;
+}
+
+int pa_merge_key_strings(pa_groupby* merged, const void* dev_lengths, const void* dev_bytes, const int64_t* records_by_source,
+                         const int64_t* bytes_by_source, const uint64_t* seed_by_source, int32_t n_sources, int32_t* collided) {
+  if (!merged || !records_by_source || !bytes_by_source || !seed_by_source || n_sources < 1 || !collided) return set_err(PA_ERR_INVALID, "null argument");
+  *collided = 0;
+  PA_TRY(finish_pending(merged));
+  if (!merged->merged || !merged->ks_str || !merged->have_groups)
+    return set_err(PA_ERR_STATE, "key strings attach to a handle made by pa_merge_create with key format \"u\" / \"U\"");
+  uint64_t nrec = 0, nbytes = 0;
+  for (int i = 0; i < n_sources; ++i) {
+    if (records_by_source[i] < 0 || bytes_by_source[i] < 0) return set_err(PA_ERR_INVALID, "negative record / byte count");
+    nrec += static_cast<uint64_t>(records_by_source[i]);
+    nbytes += static_cast<uint64_t>(bytes_by_source[i]);
+    // differing hashes of one string merge into two groups, which no check after the merge can see
+    if (seed_by_source[i] != seed_by_source[0])
+      return set_err(PA_ERR_INVALID, "sources %d and 0 hashed their keys with different seeds (%llu vs %llu): agree on one seed "
+                                     "(pa_groupby_set_key_hash_seed), aggregate again and redo the exchange", i,
+                     (unsigned long long)seed_by_source[i], (unsigned long long)seed_by_source[0]);
+  }
+  if (nrec != merged->ks_nrec)
+    return set_err(PA_ERR_INVALID, "records_by_source adds up to %llu records, pa_merge_create merged %llu", (unsigned long long)nrec,
+                   (unsigned long long)merged->ks_nrec);
+  if ((nrec && !dev_lengths) || (nbytes && !dev_bytes)) return set_err(PA_ERR_INVALID, "null length / byte buffer");
+  PA_TRY(ensure_device(merged));
+  bool c = false;
+  PA_TRY(merge_key_strings(merged, static_cast<const uint64_t*>(merged->ks_recs), merged->ks_words, nrec, static_cast<const uint32_t*>(dev_lengths),
+                           static_cast<const uint8_t*>(dev_bytes), nbytes, &c));
+  *collided = c ? 1 : 0;
+  return PA_OK;
 }
 
 int pa_groupby_partials_export_padded(pa_groupby* g, int32_t n_parts, void* dev_blocks, int64_t block_records) {
@@ -3709,6 +3960,8 @@ int pa_merge_create_padded(const void* dev_blocks, int32_t n_sources, int64_t bl
   if (!dev_blocks || n_sources < 1 || n_sources > 64 || block_records < 1 || !value_format || !key_format || !out)
     return set_err(PA_ERR_INVALID, "bad argument (1 <= n_sources <= 64)");
   if (agg_mask & ~PA_AGG_ALL) return set_err(PA_ERR_INVALID, "bad aggregate mask");
+  if ((key_format[0] == 'u' || key_format[0] == 'U') && key_format[1] == 0)
+    return set_err(PA_ERR_NOT_IMPLEMENTED, "utf8 keys take the counted exchange (pa_merge_create + pa_merge_key_strings), not padded blocks");
   HandlePtr g;
   {
     int dev = opt && opt->device >= 0 ? opt->device : -1;
@@ -3815,11 +4068,28 @@ int pa_groupby_aggregate_chunked_keys(const struct ArrowDeviceArray* keys, const
   pa_options o;
   if (opt) o = *opt; else pa_options_init(&o);
   const int64_t base0 = o.row_base;
-  DevBuf records;                      // all chunks' records, chunk after chunk
-  records.plain = true;
+  // utf8 key: every chunk hashes with one seed and exports its key bytes next to its records; a chunk whose own check
+  // moves the seed, or a merge that finds two strings under one hash, redoes the chunks with the next seed (four at most)
+  const char* kf0 = key_schemas[0].format;
+  const bool str = n_keys == 1 && kf0 && (kf0[0] == 'u' || kf0[0] == 'U') && kf0[1] == 0;
+  for (uint64_t seed = 0;;) {
+  if (seed >= 4) return set_err(PA_ERR_STATE, "utf8 keys: four differently seeded 64-bit hashes all collided");
+  DevBuf records, lengths, bytes;      // all chunks' records (and key lengths / bytes), chunk after chunk
+  records.plain = true; lengths.plain = true; bytes.plain = true;
   std::vector<int64_t> counts(static_cast<size_t>(n_chunks), 0);
-  uint64_t total = 0;
-  for (int64_t c = 0; c < n_chunks; ++c) {
+  uint64_t total = 0, total_bytes = 0;
+  bool reseed = false;
+  // grows a buffer that outlives the per-chunk handles and their streams (plain allocation), keeping `used` bytes
+  auto grow = [](DevBuf* b, size_t need, size_t used) -> int {
+    if (need <= b->bytes) return PA_OK;
+    DevBuf bigger;
+    bigger.plain = true;
+    PA_TRY(bigger.alloc(std::max<size_t>(need * 2, 1u << 20), nullptr));
+    if (used) CUDA_TRY(cudaMemcpy(bigger.p, b->p, used, cudaMemcpyDeviceToDevice));
+    *b = std::move(bigger);
+    return PA_OK;
+  };
+  for (int64_t c = 0; c < n_chunks && !reseed; ++c) {
     const int64_t lo = c * chunk_rows, len = std::min(chunk_rows, n - lo);
     std::vector<ArrowDeviceArray> kc(keys, keys + n_keys);   // views: same buffers, shifted window
     ArrowDeviceArray vc = *values;
@@ -3842,23 +4112,35 @@ int pa_groupby_aggregate_chunked_keys(const struct ArrowDeviceArray* keys, const
         if (mine.width[j] != whole.width[j] || mine.bits[j] != whole.bits[j] || mine.nullable[j] != whole.nullable[j])
           return set_err(PA_ERR_STATE, "chunk %lld packs key column %d differently from the whole column", (long long)c, j);
     }
+    if (str) PA_TRY(set_str_seed(h, seed));
     PA_TRY(pa_groupby_aggregate(h, &vc, value_schema, agg_mask));
-    int64_t cnt = 0;
-    PA_TRY(pa_groupby_partials_count(h, 1, &cnt));
-    counts[static_cast<size_t>(c)] = cnt;
-    // grow the record buffer (plain allocation: it outlives the per-chunk handles and their streams)
-    const size_t need = (total + static_cast<uint64_t>(cnt)) * RW * 8;
-    if (need > records.bytes) {
-      DevBuf bigger;
-      bigger.plain = true;
-      PA_TRY(bigger.alloc(std::max<size_t>(need * 2, 1u << 20), nullptr));
-      if (total) CUDA_TRY(cudaMemcpy(bigger.p, records.p, total * RW * 8, cudaMemcpyDeviceToDevice));
-      records = std::move(bigger);
+    if (str && h->keys[0].str_seed != seed) {   // this chunk's own check moved the seed
+      seed = h->keys[0].str_seed;
+      reseed = true;
+      break;
     }
-    if (cnt) PA_TRY(partials_export(h, 1, static_cast<char*>(records.p) + total * RW * 8, cnt, RW));
+    int64_t cnt = 0, nbytes = 0;
+    if (str) PA_TRY(pa_groupby_partials_count_utf8(h, 1, &cnt, &nbytes));
+    else PA_TRY(pa_groupby_partials_count(h, 1, &cnt));
+    counts[static_cast<size_t>(c)] = cnt;
+    PA_TRY(grow(&records, (total + static_cast<uint64_t>(cnt)) * RW * 8, total * RW * 8));
+    if (str) {
+      PA_TRY(grow(&lengths, (total + static_cast<uint64_t>(cnt)) * 4, total * 4));
+      PA_TRY(grow(&bytes, total_bytes + static_cast<uint64_t>(nbytes), total_bytes));
+    }
+    if (cnt) {
+      uint64_t* recs = reinterpret_cast<uint64_t*>(static_cast<char*>(records.p) + total * RW * 8);
+      PA_TRY(partials_export(h, 1, recs, cnt, RW));
+      if (str) {
+        DevBuf off, tmp;
+        PA_TRY(keystr_export(h, recs, RW, static_cast<uint64_t>(cnt), lengths.as<uint32_t>() + total, bytes.as<uint8_t>() + total_bytes, &off, &tmp));
+      }
+    }
     PA_TRY(pa_groupby_sync(h));
     total += static_cast<uint64_t>(cnt);
+    total_bytes += static_cast<uint64_t>(nbytes);
   }
+  if (reseed) continue;
   o.row_base = base0;
   const std::string kfmt = composite ? "L" : key_schemas->format;
   pa_groupby* m = nullptr;
@@ -3869,9 +4151,18 @@ int pa_groupby_aggregate_chunked_keys(const struct ArrowDeviceArray* keys, const
     for (int j = 0; j < n_keys; ++j) kf.push_back(key_schemas[j].format);
     PA_TRY(set_merged_layout(m, whole, kf.data()));
   }
+  if (str) {
+    bool collided = false;
+    PA_TRY(merge_key_strings(m, records.as<uint64_t>(), RW, total, lengths.as<uint32_t>(), bytes.as<uint8_t>(), total_bytes, &collided));
+    if (collided) {
+      ++seed;
+      continue;
+    }
+  }
   CUDA_TRY(cudaDeviceSynchronize());   // `records` is released on return
   *merged_out = merged.release();
   return PA_OK;
+  }
 }
 
 // ---- multi-GPU through the C ABI: communicator + the whole sharded step (SURVEY.md §8b "multi-GPU variants taking a
@@ -3891,6 +4182,13 @@ struct pa_comm {
   int last_record_bytes = 0, last_unordered = 0;   // pa_comm_last_exchange
   int64_t last_table_slots = 0;
   int64_t last_pairs_sent = 0, last_pairs_received = 0, last_set_slots = 0;   // pa_comm_last_distinct
+  // utf8 key: lengths and key bytes sent / received, scratch of the byte offsets, the collision word of the all-reduce
+  DevBuf ksend_len, krecv_len, ksend_bytes, krecv_bytes, koff, ktmp, kflag;
+  uint64_t h_seed = 0;                    // (staging for the async copies)
+  uint32_t h_flag = 0;
+  int64_t last_bytes_sent = 0, last_bytes_received = 0;   // pa_comm_last_key_strings
+  uint64_t last_seed = 0;
+  int32_t last_attempts = 0;
 };
 
 #define NCCL_TRY(expr)                                                                                          \
@@ -3911,7 +4209,8 @@ static int comm_finish(pa_comm* c) {
   // The communicator outlives the handles (and their streams) it is used with: its scratch does not belong to any
   // stream's allocation order.
   for (DevBuf* b : {&c->send, &c->recv, &c->d_counts, &c->d_all, &c->d_cursor, &c->psend, &c->precv, &c->pset, &c->layouts, &c->merge.tkeys, &c->merge.idx,
-                    &c->merge.m_first, &c->merge.m_slot, &c->merge.s_first, &c->merge.s_slot, &c->merge.cub_tmp})
+                    &c->merge.m_first, &c->merge.m_slot, &c->merge.s_first, &c->merge.s_slot, &c->merge.cub_tmp, &c->ksend_len, &c->krecv_len,
+                    &c->ksend_bytes, &c->krecv_bytes, &c->koff, &c->ktmp, &c->kflag})
     b->plain = true;
   for (auto& e : c->ev) CUDA_TRY(cudaEventCreate(&e));
   return PA_OK;
@@ -3973,6 +4272,15 @@ int pa_comm_last_key_layout(pa_comm* c, double* agree_ms, double* repack_ms) {
   return PA_OK;
 }
 
+int pa_comm_last_key_strings(pa_comm* c, int64_t* bytes_sent, int64_t* bytes_received, uint64_t* seed, int32_t* attempts) {
+  if (!c) return set_err(PA_ERR_INVALID, "null argument");
+  if (bytes_sent) *bytes_sent = c->last_bytes_sent;
+  if (bytes_received) *bytes_received = c->last_bytes_received;
+  if (seed) *seed = c->last_seed;
+  if (attempts) *attempts = c->last_attempts;
+  return PA_OK;
+}
+
 int pa_comm_last_phases(pa_comm* c, double phase_ms[5]) {
   if (!c || !phase_ms) return set_err(PA_ERR_INVALID, "null argument");
   for (int i = 0; i < 5; ++i) phase_ms[i] = c->phase_ms[i];
@@ -4005,7 +4313,6 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
     return set_err(PA_ERR_NOT_IMPLEMENTED, "sharded aggregates: sum / mean / count / min / max / first / last / product / variance / stddev / "
                                            "all / any / count_distinct");
   if (g->device != c->device) return set_err(PA_ERR_INVALID, "handle lives on device %d, communicator on %d", g->device, c->device);
-  PA_TRY(check_shardable(g));
   PA_TRY(ensure_device(g));
   cudaStream_t st = g->stream;
   const int W = c->world;
@@ -4044,6 +4351,14 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
       c->repack_ms = t;
     }
   }
+  // utf8 key: the records carry the hash of the key bytes, and the bytes travel with them (strkeys.cuh).  Every rank
+  // must hash with the same seed, and no owner may see two strings under one hash: the count gather carries every
+  // rank's seed, and after the owner's byte check one all-reduce tells every rank whether some owner saw a collision.
+  // Either way all ranks redo the step together with the agreed (max) or the next seed, four seeds at most; every such
+  // branch is taken on gathered values only.
+  const bool str = is_str_key(g);
+  c->last_bytes_sent = 0; c->last_bytes_received = 0; c->last_attempts = 0;
+  for (int attempt = 1;; ++attempt) {
   CUDA_TRY(cudaEventRecord(c->ev[0], st));
   // 1. local pass.  sum / mean of floats / count need one 32-byte sector per group (compact records, merge.cuh),
   // everything else the full record; with compact records the bucketed path may hand over its unordered group records
@@ -4057,7 +4372,8 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   const bool distinct = (agg_mask & PA_AGG_COUNT_DISTINCT) != 0;
   const bool full_only = stage2 || distinct || (agg_mask & (PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY));
   const bool compact = !full_only && !is_wide(agg_mask, vc_) && !(agg_mask & (AGG_FIRST | AGG_LAST));
-  g->want_unordered = compact && !g->resample;
+  // (a utf8 key's first pass checks its grouping byte for byte, which reads the ordered groups)
+  g->want_unordered = compact && !g->resample && (!str || g->str_verified);
   const int local_rc = aggregate_entry(g, values, value_schema, agg_mask, false);
   g->want_unordered = false;
   if (local_rc != PA_OK) return local_rc;
@@ -4070,7 +4386,9 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   // (every rank also tells the others where its row shard ends: the merge orders by GLOBAL first row and only has
   // to sort the bits below the largest one)
   // (count_distinct: the W pair counts per owner follow, at [W + 1, 2 W + 1), in the same gather)
-  const int W1 = W + 1 + (distinct ? W : 0);
+  // (utf8 key: then the rank's hash seed and its W key byte counts per owner, at KS and [KS + 1, KS + 1 + W))
+  const int KS = W + 1 + (distinct ? W : 0);
+  const int W1 = KS + (str ? 1 + W : 0);
   PA_TRY(c->d_counts.alloc(sizeof(uint64_t) * W1, st));
   PA_TRY(c->d_all.alloc(sizeof(uint64_t) * W1 * W, st));
   CUDA_TRY(cudaMemsetAsync(c->d_counts.p, 0, sizeof(uint64_t) * W1, st));
@@ -4085,12 +4403,29 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
     PA_TRY(partials_count_async(g, W, c->d_counts.as<unsigned long long>()));
   }
   if (distinct) PA_TRY(pairs_count_async(g, W, c->d_counts.as<unsigned long long>() + W + 1));
+  if (str) {
+    c->h_seed = g->keys[0].str_seed;
+    CUDA_TRY(cudaMemcpyAsync(c->d_counts.as<uint64_t>() + KS, &c->h_seed, sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+    PA_TRY(keystr_count_async(g, W, unordered ? g->unordered_recs : nullptr, G_local, c->d_counts.as<unsigned long long>() + KS + 1));
+  }
   NCCL_TRY(ncclAllGather(c->d_counts.p, c->d_all.p, W1, ncclUint64, c->comm, st));
   std::vector<uint64_t> all(static_cast<size_t>(W1) * W);
   CUDA_TRY(cudaMemcpyAsync(all.data(), c->d_all.p, sizeof(uint64_t) * W1 * W, cudaMemcpyDeviceToHost, st));
   CUDA_TRY(cudaStreamSynchronize(st));
-  std::vector<int64_t> send_cnt(W), recv_cnt(W), psend_cnt(W, 0), precv_cnt(W, 0);
-  uint64_t send_total = 0, recv_total = 0, row_bound = 1, psend_total = 0, precv_total = 0;
+  if (str) {   // a rank whose own check moved its seed: everybody takes the largest seed and redoes the step
+    uint64_t lo = ~0ull, hi = 0;
+    for (int p = 0; p < W; ++p) {
+      lo = std::min(lo, all[static_cast<size_t>(p) * W1 + KS]);
+      hi = std::max(hi, all[static_cast<size_t>(p) * W1 + KS]);
+    }
+    if (hi >= 4) return set_err(PA_ERR_STATE, "utf8 keys: four differently seeded 64-bit hashes all collided");
+    if (lo != hi) {
+      PA_TRY(set_str_seed(g, hi));
+      continue;
+    }
+  }
+  std::vector<int64_t> send_cnt(W), recv_cnt(W), psend_cnt(W, 0), precv_cnt(W, 0), ksend_cnt(W, 0), krecv_cnt(W, 0);
+  uint64_t send_total = 0, recv_total = 0, row_bound = 1, psend_total = 0, precv_total = 0, ksend_total = 0, krecv_total = 0;
   for (int p = 0; p < W; ++p) {
     send_cnt[p] = static_cast<int64_t>(all[static_cast<size_t>(c->rank) * W1 + p]);
     recv_cnt[p] = static_cast<int64_t>(all[static_cast<size_t>(p) * W1 + c->rank]);
@@ -4102,6 +4437,12 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
       precv_cnt[p] = static_cast<int64_t>(all[static_cast<size_t>(p) * W1 + W + 1 + c->rank]);
       psend_total += psend_cnt[p];
       precv_total += precv_cnt[p];
+    }
+    if (str) {
+      ksend_cnt[p] = static_cast<int64_t>(all[static_cast<size_t>(c->rank) * W1 + KS + 1 + p]);
+      krecv_cnt[p] = static_cast<int64_t>(all[static_cast<size_t>(p) * W1 + KS + 1 + c->rank]);
+      ksend_total += ksend_cnt[p];
+      krecv_total += krecv_cnt[p];
     }
   }
   // (checked for every owner: every rank sees every count, so all ranks fail together before any record is sent)
@@ -4134,10 +4475,30 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
     PA_TRY(c->precv.alloc(std::max<uint64_t>(precv_total, 1) * PW * 8, st));
     PA_TRY(pairs_export(g, W, psend_cnt.data(), c->psend.p, &c->d_cursor));
   }
+  if (str) {   // lengths and key bytes of the records just written, in the same owner segments
+    PA_TRY(c->ksend_len.alloc(std::max<uint64_t>(send_total, 1) * 4, st));
+    PA_TRY(c->krecv_len.alloc(std::max<uint64_t>(recv_total, 1) * 4, st));
+    PA_TRY(c->ksend_bytes.alloc(std::max<uint64_t>(ksend_total, 1), st));
+    PA_TRY(c->krecv_bytes.alloc(std::max<uint64_t>(krecv_total, 1), st));
+    PA_TRY(keystr_export(g, c->send.as<uint64_t>(), words, send_total, c->ksend_len.as<uint32_t>(), c->ksend_bytes.as<uint8_t>(), &c->koff, &c->ktmp));
+  }
   CUDA_TRY(cudaEventRecord(c->ev[2], st));
-  // 4. all-to-all of the records; the distinct pairs, grouped by owner, in a second exchange
+  // 4. all-to-all of the records; the distinct pairs, grouped by owner, in a second exchange; a utf8 key's lengths and
+  // bytes in one more
   PA_TRY(exchange_grouped(c, st, c->send.as<uint64_t>(), send_cnt.data(), c->recv.as<uint64_t>(), recv_cnt.data(), RW));
   if (distinct) PA_TRY(exchange_grouped(c, st, c->psend.as<uint64_t>(), psend_cnt.data(), c->precv.as<uint64_t>(), precv_cnt.data(), PW));
+  if (str) {
+    NCCL_TRY(ncclGroupStart());
+    uint64_t so = 0, ro = 0, sb = 0, rb = 0;
+    for (int p = 0; p < W; ++p) {
+      if (send_cnt[p]) NCCL_TRY(ncclSend(c->ksend_len.as<uint32_t>() + so, static_cast<size_t>(send_cnt[p]), ncclUint32, p, c->comm, st));
+      if (recv_cnt[p]) NCCL_TRY(ncclRecv(c->krecv_len.as<uint32_t>() + ro, static_cast<size_t>(recv_cnt[p]), ncclUint32, p, c->comm, st));
+      if (ksend_cnt[p]) NCCL_TRY(ncclSend(c->ksend_bytes.as<uint8_t>() + sb, static_cast<size_t>(ksend_cnt[p]), ncclUint8, p, c->comm, st));
+      if (krecv_cnt[p]) NCCL_TRY(ncclRecv(c->krecv_bytes.as<uint8_t>() + rb, static_cast<size_t>(krecv_cnt[p]), ncclUint8, p, c->comm, st));
+      so += send_cnt[p]; ro += recv_cnt[p]; sb += ksend_cnt[p]; rb += krecv_cnt[p];
+    }
+    NCCL_TRY(ncclGroupEnd());
+  }
   CUDA_TRY(cudaEventRecord(c->ev[3], st));
   // 5. owner-side merge
   const std::string kfmt = g->resample ? g->index_format : composite ? "L" : g->keys[0].format;
@@ -4153,6 +4514,26 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
     std::vector<const char*> kf;
     for (const Column& k : g->keys) kf.push_back(k.format.c_str());
     PA_TRY(set_merged_layout(m.get(), agreed, kf.data()));
+  }
+  if (str) {   // the owner's byte check, then every rank learns whether any owner saw two strings under one hash
+    bool collided = false;
+    PA_TRY(merge_key_strings(m.get(), c->recv.as<uint64_t>(), words, recv_total, c->krecv_len.as<uint32_t>(), c->krecv_bytes.as<uint8_t>(),
+                             krecv_total, &collided));
+    c->h_flag = collided ? 1u : 0u;
+    PA_TRY(c->kflag.alloc(4, st));
+    CUDA_TRY(cudaMemcpyAsync(c->kflag.p, &c->h_flag, 4, cudaMemcpyHostToDevice, st));
+    NCCL_TRY(ncclAllReduce(c->kflag.p, c->kflag.p, 1, ncclUint32, ncclMax, c->comm, st));
+    CUDA_TRY(cudaMemcpyAsync(&c->h_flag, c->kflag.p, 4, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    c->last_bytes_sent = static_cast<int64_t>(ksend_total);
+    c->last_bytes_received = static_cast<int64_t>(krecv_total);
+    c->last_seed = g->keys[0].str_seed;
+    c->last_attempts = attempt;
+    if (c->h_flag) {
+      if (g->keys[0].str_seed + 1 >= 4) return set_err(PA_ERR_STATE, "utf8 keys: four differently seeded 64-bit hashes all collided");
+      PA_TRY(set_str_seed(g, g->keys[0].str_seed + 1));
+      continue;
+    }
   }
   uint64_t set_slots = 0;
   if (distinct) PA_TRY(merge_distinct(m.get(), c->precv.p, precv_total, &c->pset, &set_slots));
@@ -4170,6 +4551,7 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   c->last_set_slots = static_cast<int64_t>(set_slots);
   *merged_out = m.release();
   return PA_OK;
+  }
 }
 
 // ---- synthetic generator ----

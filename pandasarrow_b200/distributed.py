@@ -21,6 +21,14 @@ A utf8 column in a sharded composite key must therefore be dictionary-encoded ON
 is sliced into shards: per-shard `dictionary_encode()` gives every shard its own codes, and the agreement fails with a
 dictionary-fingerprint error instead of merging different strings into one group.
 
+A single utf8 / large_utf8 key (group_by("name")) is grouped by a seeded 64-bit hash of its bytes, and its records carry
+that hash.  Every record therefore travels with its group's key bytes (partials_export_utf8, exchange_key_strings),
+and the owner compares the bytes of every record of a merged group with its representative's (merge_key_strings).
+All shards must hash with one seed: a shard whose own byte check found a collision has moved to the next seed, so
+before the exchange the shards agree on the largest (agree_key_hash_seed) and re-aggregate when it is not theirs.  A
+collision that only the owner sees (two strings of different shards, one hash) makes every rank retry with the next
+seed; four seeds at most, as on one GPU.
+
 torch.distributed is plumbing only (rendezvous + the collective); the exchange helpers work on any
 backend, which is what the world_size-2 gloo tests exercise on CPU.
 """
@@ -80,6 +88,55 @@ def exchange_records(send, send_counts: Sequence[int], group=None, words: int = 
     dist.all_to_all_single(recv.view(-1), send.reshape(-1), output_split_sizes=[c * w for c in recv_counts],
                            input_split_sizes=[int(c) * w for c in send_counts], group=group)
     return recv, recv_counts
+
+
+def exchange_key_strings(lengths, data, send_counts: Sequence[int], send_bytes: Sequence[int], group=None):
+    """All-to-all of a utf8 key's strings next to exchange_records: `lengths` (int32, one per record, grouped by
+    destination like the records, send_counts of them per rank) and `data` (uint8, send_bytes[p] bytes for rank p).
+    Returns (recv lengths, recv bytes, recv record counts, recv byte counts), grouped by source rank."""
+    import torch
+    import torch.distributed as dist
+    world = dist.get_world_size(group)
+    assert len(send_counts) == world and len(send_bytes) == world
+    dev = lengths.device
+    sc = torch.tensor([[int(c), int(b)] for c, b in zip(send_counts, send_bytes)], dtype=torch.int64, device=dev)
+    rc = torch.empty_like(sc)
+    dist.all_to_all_single(rc.view(-1), sc.view(-1), group=group)
+    recv_counts = [int(x) for x in rc[:, 0].tolist()]
+    recv_bytes = [int(x) for x in rc[:, 1].tolist()]
+    rlen = torch.empty(sum(recv_counts), dtype=lengths.dtype, device=dev)
+    dist.all_to_all_single(rlen, lengths.reshape(-1), output_split_sizes=recv_counts, input_split_sizes=[int(c) for c in send_counts],
+                           group=group)
+    rdata = torch.empty(sum(recv_bytes), dtype=data.dtype, device=dev)
+    dist.all_to_all_single(rdata, data.reshape(-1), output_split_sizes=recv_bytes, input_split_sizes=[int(b) for b in send_bytes],
+                           group=group)
+    return rlen, rdata, recv_counts, recv_bytes
+
+
+def agree_key_hash_seed(gb, group=None) -> Tuple[int, bool]:
+    """One hash seed for a utf8 key on every shard: all_reduce MAX of the seeds (any torch.distributed backend), set on
+    `gb` (which drops its groups when the seed changes).  Returns (agreed seed, whether every shard already hashed with
+    it); when not, every shard aggregates again.  PaError on every rank when the agreed seed is past the fourth."""
+    import torch
+    import torch.distributed as dist
+    from .groupby import PaError
+    mine = gb.key_hash_seed()
+    t = torch.tensor([mine, -mine], dtype=torch.int64)       # (max, -min) in one reduction
+    if dist.get_backend(group) == "nccl":
+        t = t.cuda()
+    dist.all_reduce(t, op=dist.ReduceOp.MAX, group=group)
+    hi, lo = int(t[0]), -int(t[1])
+    if hi >= MAX_HASH_SEEDS:
+        raise PaError(4, "utf8 keys: four differently seeded 64-bit hashes all collided")
+    gb.set_key_hash_seed(hi)
+    return hi, lo == hi
+
+
+MAX_HASH_SEEDS = 4   # as on one GPU (the library's utf8 key check)
+
+
+def _utf8(gb) -> bool:
+    return len(getattr(gb, "key_names", ())) == 1 and getattr(gb, "key_formats", [None])[0] in ("u", "U")
 
 
 def agree_key_layout(gb, group=None):
@@ -172,6 +229,15 @@ class Comm:
             m._adopt_keys(gb.key_names, gb._dicts)
         return m
 
+    def key_strings_info(self) -> Dict[str, int]:
+        """utf8 key exchange of the last step (pa_comm_last_key_strings): key bytes sent and received, the agreed hash
+        seed and the attempts the step took; zeros for a step without a utf8 key."""
+        import ctypes as C
+        from .groupby import _check
+        sent, recv, seed, attempts = C.c_int64(), C.c_int64(), C.c_uint64(), C.c_int32()
+        _check(self._L.pa_comm_last_key_strings(self._h, C.byref(sent), C.byref(recv), C.byref(seed), C.byref(attempts)))
+        return {"bytes_sent": sent.value, "bytes_received": recv.value, "seed": seed.value, "attempts": attempts.value}
+
     def key_layout_info(self) -> Dict[str, float]:
         """Composite-key agreement of the last step (pa_comm_last_key_layout): device ms of the layout gather and of the
         repack (0 when none happened)."""
@@ -253,7 +319,11 @@ def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_fo
 
     tail_stream (a torch.cuda.Stream, padded path only): the exchange and the merge run on it, behind an event recorded
     after the export — the handle's own stream is free for the next step's local pass while this step's records travel
-    and merge (the serial tail is launch / NCCL latency on a handful of CTAs)."""
+    and merge (the serial tail is launch / NCCL latency on a handful of CTAs).
+
+    A single utf8 / large_utf8 key takes the counted exchange: the shards agree on a hash seed, the records travel with
+    their key bytes, the owner checks and attaches the strings, and an all-reduce of the collision flag decides together
+    whether every rank retries with the next seed.  `key_format` may be None (taken from `gb`)."""
     import torch
     import torch.distributed as dist
     from .groupby import MergedGroupBy, PaError
@@ -264,6 +334,8 @@ def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_fo
     if padded is None:
         padded = stream is not None and stream == torch.cuda.current_stream(dev).cuda_stream
     padded = padded and not stage2 and not any(a in ("all", "any", "count_distinct") for a in aggs)
+    if _utf8(gb):
+        return _sharded_utf8(gb, values, aggs, value_format, key_format or gb.key_formats[0], group, stream, dev, world)
     composite = _composite(gb)
     if composite:
         layout = agree_key_layout(gb, group)
@@ -321,6 +393,49 @@ def sharded_aggregate(gb, values, aggs: Sequence[str], value_format: str, key_fo
         _, precv, precv_counts = counted_exchange(gb.distinct_pairs_count, gb.distinct_pairs_export, PA_DISTINCT_PAIR_WORDS)
         merged.merge_distinct_pairs(precv.data_ptr(), precv_counts)
     return merged
+
+
+def _sharded_utf8(gb, values, aggs, value_format, key_format, group, stream, dev, world):
+    import torch
+    import torch.distributed as dist
+    from .groupby import MergedGroupBy, PaError
+    stage2 = any(PA_AGG[a] & PA_AGG_STAGE2 for a in aggs)
+    words = PA_PARTIAL_WORDS_STAGE2 if stage2 else PA_PARTIAL_WORDS
+    # every seed is reached at most twice: by a shard's own check, and by a collision an owner saw
+    for _ in range(2 * MAX_HASH_SEEDS):
+        gb.aggregate(values, aggs, fetch=False)
+        seed, unanimous = agree_key_hash_seed(gb, group)
+        if not unanimous:
+            continue
+        counts, nbytes = gb.partials_count_utf8(world)
+        send = torch.empty((max(sum(counts), 1), words), dtype=torch.int64, device=dev)
+        lens = torch.empty(max(sum(counts), 1), dtype=torch.int32, device=dev)
+        data = torch.empty(max(sum(nbytes), 1), dtype=torch.uint8, device=dev)
+        gb.partials_export_utf8(world, send.data_ptr(), send.shape[0], lens.data_ptr(), data.data_ptr(), data.numel(), stage2=stage2)
+        recv, recv_counts = exchange_records(send[:sum(counts)], counts, group, words=words)
+        rlens, rdata, _, recv_bytes = exchange_key_strings(lens[:sum(counts)], data[:sum(nbytes)], counts, nbytes, group)
+        torch.cuda.synchronize()
+        merged = MergedGroupBy(recv.data_ptr(), recv_counts, [a for a in aggs if a != "count_distinct"], value_format, key_format,
+                               device=dev.index, stream=stream)
+        collided = merged.merge_key_strings(rlens.data_ptr(), rdata.data_ptr(), recv_counts, recv_bytes, [seed] * world)
+        flag = torch.tensor([int(collided)], dtype=torch.int32, device=dev)
+        dist.all_reduce(flag, op=dist.ReduceOp.MAX, group=group)
+        if int(flag.item()):
+            merged.close()
+            if seed + 1 >= MAX_HASH_SEEDS:
+                raise PaError(4, "utf8 keys: four differently seeded 64-bit hashes all collided")
+            gb.set_key_hash_seed(seed + 1)
+            continue
+        merged._keep = (send, recv)
+        if "count_distinct" in aggs:
+            counts = gb.distinct_pairs_count(world)
+            psend = torch.empty((max(sum(counts), 1), PA_DISTINCT_PAIR_WORDS), dtype=torch.int64, device=dev)
+            gb.distinct_pairs_export(world, psend.data_ptr(), psend.shape[0])
+            precv, precv_counts = exchange_records(psend[:sum(counts)], counts, group, words=PA_DISTINCT_PAIR_WORDS)
+            torch.cuda.synchronize()
+            merged.merge_distinct_pairs(precv.data_ptr(), precv_counts)
+        return merged
+    raise PaError(4, "utf8 keys: four differently seeded 64-bit hashes all collided")
 
 
 def resample_anchor(first_ts_local: Optional[int], ticks_per_day: int = 86_400 * 10**9, group=None) -> int:

@@ -12,7 +12,7 @@ DeviceColumn views of CUDA memory (zero copy).
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, List, Optional, Sequence, Union
+from typing import Dict, List, Optional, Sequence, Tuple, Union
 
 import pyarrow as pa
 
@@ -352,6 +352,31 @@ class GroupBy:
         fn = self._L.pa_groupby_partials_export_stage2 if stage2 else self._L.pa_groupby_partials_export
         _check(fn(self._h, n_parts, records_ptr, capacity_records))
 
+    # ---- a single utf8 / large_utf8 key across shards: records travel with their key bytes ----
+    def key_hash_seed(self) -> int:
+        """pa_groupby_key_hash_seed: the seed this utf8 key is hashed with (raised by the handle's own byte check)."""
+        out = C.c_uint64()
+        _check(self._L.pa_groupby_key_hash_seed(self._h, C.byref(out)))
+        return out.value
+
+    def set_key_hash_seed(self, seed: int):
+        """pa_groupby_set_key_hash_seed: re-hash the key with `seed` (one that all shards agreed on, see
+        distributed.agree_key_hash_seed); groups and results of earlier aggregates are dropped."""
+        _check(self._L.pa_groupby_set_key_hash_seed(self._h, int(seed)))
+
+    def partials_count_utf8(self, n_parts: int) -> Tuple[List[int], List[int]]:
+        """Records and key bytes owned by each of n_parts ranks (after an aggregate)."""
+        recs, nbytes = (C.c_int64 * n_parts)(), (C.c_int64 * n_parts)()
+        _check(self._L.pa_groupby_partials_count_utf8(self._h, n_parts, recs, nbytes))
+        return list(recs), list(nbytes)
+
+    def partials_export_utf8(self, n_parts: int, records_ptr: int, capacity_records: int, lengths_ptr: int, bytes_ptr: int,
+                             capacity_bytes: int, stage2: bool = False):
+        """Records (as partials_export), one uint32 key length per record and the key bytes, grouped by owner in the same
+        order, into device memory (after partials_count_utf8)."""
+        _check(self._L.pa_groupby_partials_export_utf8(self._h, n_parts, int(bool(stage2)), records_ptr, capacity_records,
+                                                       lengths_ptr, bytes_ptr, capacity_bytes))
+
     def partials_export_padded(self, n_parts: int, blocks_ptr: int, block_records: int):
         _check(self._L.pa_groupby_partials_export_padded(self._h, n_parts, blocks_ptr, block_records))
 
@@ -455,6 +480,19 @@ class MergedGroupBy(GroupBy):
     def _adopt_keys(self, key_names, dictionaries):
         self.key_names, self._dicts = list(key_names), list(dictionaries)
 
+    def merge_key_strings(self, lengths_ptr: int, bytes_ptr: int, records_by_source: Sequence[int], bytes_by_source: Sequence[int],
+                          seed_by_source: Sequence[int]) -> bool:
+        """pa_merge_key_strings (key format "u" / "U"): attaches the merged groups' key strings from the received lengths and
+        bytes, grouped by source.  Returns True when two different strings shared a hash: then nothing is attached and
+        the ranks retry with the next seed.  The record buffer given to the constructor must still be alive."""
+        n = len(records_by_source)
+        recs = (C.c_int64 * n)(*[int(c) for c in records_by_source])
+        nbytes = (C.c_int64 * n)(*[int(c) for c in bytes_by_source])
+        seeds = (C.c_uint64 * n)(*[int(c) for c in seed_by_source])
+        collided = C.c_int32()
+        _check(self._L.pa_merge_key_strings(self._h, lengths_ptr, bytes_ptr, recs, nbytes, seeds, n, C.byref(collided)))
+        return bool(collided.value)
+
     def merge_distinct_pairs(self, pairs_ptr: int, counts_by_source: Sequence[int]):
         """Adds count_distinct (fetch("count_distinct")) from the received distinct-pair records, grouped by source."""
         counts = (C.c_int64 * len(counts_by_source))(*[int(c) for c in counts_by_source])
@@ -477,7 +515,8 @@ def aggregate_chunked(keys, values: pa.Array, aggs: Sequence[str], chunk_rows: i
     """Host columns larger than the device (or than 2^32-2 rows): pa_groupby_aggregate_chunked — the columns are
     aggregated `chunk_rows` rows at a time and the chunks' partial records merged like ranks'.  `keys`: one key array,
     or a list of them (a composite key: utf8 members are dictionary-encoded once over the whole column; unique(j)
-    returns a DictionaryArray for dictionary columns)."""
+    returns a DictionaryArray for dictionary columns).  A single utf8 / large_utf8 key stays strings: its key bytes
+    travel with the chunks' records and unique() returns the input's string type."""
     mask = 0
     for a in aggs:
         mask |= PA_AGG[a]
