@@ -151,7 +151,19 @@ int pa_device_count(int* out);
  * keys[i] with key_schemas[i] describe the i-th key column (all the same length).  Supported key
  * formats: l L i I (int64/uint64/int32/uint32), ts* / tt* / td* (64-bit temporal), and
  * dictionary-encoded columns (the int32 indices are the key; the dictionary is not read).
- * Null keys form their own group.  Composite keys must pack into 64 bits.
+ * Null keys form their own group.  A single key may also be utf8 / large_utf8 ("u" / "U": offsets + bytes, host or
+ * device buffers, slices honoured).
+ * A composite key (2 .. PA_MAX_KEY_COLS columns) that packs into 64 bits and has no utf8 column groups on its packed
+ * word (see "composite keys across shards").  Any other composite key — wider than 64 bits, or with a utf8 / large_utf8
+ * column — is a hashed key: a seeded 64-bit hash over all its columns in order (per column the null flag and, for a
+ * valid slot, its value bits, a dictionary column's index, or a utf8 slot's length and bytes; never a null slot's
+ * value) stands in for the key, 8 bytes per row computed here.  The first call that builds groups checks every row
+ * against its group's first row (null flags, then the values of columns valid in both) and re-hashes with the next
+ * seed on a mismatch, four seeds at most (then PA_ERR_STATE); until that check has passed, pa_groupby_aggregate_async
+ * runs synchronously.  Group order and every result are those of the key columns themselves.  A hashed composite key
+ * groups on one GPU: pa_groupby_key_layout / _set_key_layout, the partial-record and distinct-pair exports and
+ * pa_groupby_sharded_aggregate return PA_ERR_NOT_IMPLEMENTED for it, and pa_groupby_aggregate_chunked_keys refuses
+ * composite keys that do not pack, as it always has.
  * Work is lazy: the table is built by the first aggregate (fused with it) or by
  * pa_groupby_num_groups / pa_groupby_unique. */
 int pa_groupby_create(const struct ArrowDeviceArray* keys, const struct ArrowSchema* key_schemas,
@@ -374,8 +386,10 @@ int pa_merge_create_padded(const void* dev_blocks, int32_t n_sources, int64_t bl
  * record carrying the group's global first row: the first string in row order).  The plain pa_groupby_partials_count /
  * _export / _export_stage2 / _export_padded and pa_merge_create_padded refuse utf8 keys.
  *
- * The hash seed of a handle with one utf8 / large_utf8 key (0 at creation, raised by the handle's own check on a
- * collision); PA_ERR_INVALID for any other handle. */
+ * The hash seed of a handle with a hashed key — one utf8 / large_utf8 key, or a composite key that does not pack into
+ * 64 bits (pa_groupby_create) — 0 at creation, raised by the handle's own check on a collision; PA_ERR_INVALID for any
+ * other handle.  Test hook: with the environment variable PA_TEST_STR_HASH_BITS=b, hashes made under seed 0 keep only
+ * their low b bits (utf8 keys and hashed composite keys alike), so that different keys share a hash on demand. */
 int pa_groupby_key_hash_seed(pa_groupby* g, uint64_t* seed);
 /* Re-hashes the key column with `seed` (the largest seed of all shards, see pa_merge_key_strings).  Completes a pending
  * aggregate first; groups, outputs, groupings, distinct pairs and stage-2 terms are dropped like pa_groupby_set_key_layout
@@ -410,7 +424,11 @@ int pa_merge_key_strings(pa_groupby* merged, const void* dev_lengths, const void
  * pa_groupby_create has a validity bitmap and a nonzero null_count, and a dictionary column takes bits_for(dictionary
  * length) bits.  Shards of one frame can therefore pack the same group into different words.  Before their records
  * meet, all shards agree on one layout (pa_key_layout_agree over every shard's pa_groupby_key_layout) and repack to it
- * (pa_groupby_set_key_layout); pa_groupby_sharded_aggregate does both by itself. */
+ * (pa_groupby_set_key_layout); pa_groupby_sharded_aggregate does both by itself.  A composite key that does not pack
+ * (a hashed composite key, pa_groupby_create) has no layout: these calls, the partial-record and distinct-pair exports
+ * and the sharded step return PA_ERR_NOT_IMPLEMENTED for it.  Whether a shard's key packs depends on its own nulls and
+ * dictionaries, so in the sharded step a hashed rank still takes part in the layout gather (with an empty layout) and
+ * every rank fails together. */
 #define PA_MAX_KEY_COLS 4
 typedef struct pa_key_layout {
   int32_t n_keys;                               /* 2 .. PA_MAX_KEY_COLS */
@@ -455,7 +473,8 @@ int pa_groupby_aggregate_chunked(const struct ArrowDeviceArray* keys, const stru
                                  uint32_t agg_mask, int64_t chunk_rows, const pa_options* opt, pa_groupby** merged_out);
 /* The same with n_keys key columns (a composite key as pa_groupby_create takes it).  Chunks are views of the same
  * columns, so every chunk packs with the layout of the whole columns; the merged handle carries that layout and
- * answers pa_groupby_unique for every key column. */
+ * answers pa_groupby_unique for every key column.  A composite key must pack into 64 bits and hold no utf8 column
+ * (dictionary-encode it): decided from the whole columns before any chunk, PA_ERR_NOT_IMPLEMENTED otherwise. */
 int pa_groupby_aggregate_chunked_keys(const struct ArrowDeviceArray* keys, const struct ArrowSchema* key_schemas, int32_t n_keys,
                                       const struct ArrowDeviceArray* values, const struct ArrowSchema* value_schema,
                                       uint32_t agg_mask, int64_t chunk_rows, const pa_options* opt, pa_groupby** merged_out);

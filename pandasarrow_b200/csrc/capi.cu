@@ -36,6 +36,7 @@
 #include "csort.cuh"
 #include "sort.cuh"
 #include "strkeys.cuh"
+#include "rowkeys.cuh"
 
 using namespace pa;
 
@@ -131,11 +132,10 @@ struct Column {
   uint64_t dict_fp = 0;
   DevBuf own_data, own_valid;       // set when the input lived on the host (or was unpacked)
   DevBuf own_bits;                  // boolean host input: the packed bits on the device
-  // utf8 / large_utf8 KEY columns (strkeys.cuh): `data` is the per-row 64-bit hash, the strings stay reachable here
+  // utf8 / large_utf8 KEY columns (strkeys.cuh): the key word is a hash (pa_groupby::hashed), the strings stay reachable here
   bool is_str = false;
   StrCol str{};
   DevBuf own_offsets, own_bytes;
-  uint64_t str_seed = 0;
 };
 
 int parse_format(const char* f, int* width, int* vc) {
@@ -345,29 +345,8 @@ int load_column(const ArrowDeviceArray* da, const ArrowSchema* sc, cudaStream_t 
   return PA_OK;
 }
 
-// Collision hook for tests (PA_TEST_STR_HASH_BITS=b): hashes made under seed 0 keep only their low b bits, so that
-// different strings share a hash on demand.  Unset: every bit is kept.
-uint64_t test_hash_keep(uint64_t seed) {
-  static const char* bits = getenv("PA_TEST_STR_HASH_BITS");
-  if (!bits || seed != 0) return ~0ull;
-  const int b = atoi(bits);
-  return b <= 0 ? 0ull : b >= 64 ? ~0ull : (1ull << b) - 1;
-}
-
-// utf8 / large_utf8 key column: offsets + bytes onto the device (or borrowed), then one 64-bit hash per row.
-int hash_string_key(Column* out, cudaStream_t st, int num_sms) {
-  PA_TRY(out->own_data.alloc(static_cast<size_t>(std::max<int64_t>(out->n, 1)) * 8, st));
-  if (out->n > 0) {
-    const int grid = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((out->n + 255) / 256, static_cast<int64_t>(num_sms) * 16)));
-    k_str_hash<<<grid, 256, 0, st>>>(out->str, out->valid, out->bit_off, out->n, 0x5851F42D4C957F2Dull + out->str_seed * 0x9E3779B97F4A7C15ull,
-                                     test_hash_keep(out->str_seed), out->own_data.as<uint64_t>());
-    CUDA_TRY(cudaGetLastError());
-  }
-  out->data = out->own_data.p;
-  return PA_OK;
-}
-
-int load_string_key(const ArrowDeviceArray* da, const ArrowSchema* sc, cudaStream_t st, int device, int num_sms, Column* out) {
+// utf8 / large_utf8 key column: offsets + bytes onto the device (or borrowed); setup_keys hashes the key.
+int load_string_key(const ArrowDeviceArray* da, const ArrowSchema* sc, cudaStream_t st, int device, Column* out) {
   const ArrowArray& a = da->array;
   if (a.n_buffers < 3) return set_err(PA_ERR_INVALID, "utf8 array needs 3 buffers (validity, offsets, data), got %lld", (long long)a.n_buffers);
   const bool wide = sc->format[0] == 'U';
@@ -413,7 +392,7 @@ int load_string_key(const ArrowDeviceArray* da, const ArrowSchema* sc, cudaStrea
     return set_err(PA_ERR_INVALID, "unsupported device_type %d", (int)da->device_type);
   }
   out->str.wide = wide ? 1 : 0;
-  return hash_string_key(out, st, num_sms);
+  return PA_OK;
 }
 
 struct KeyField {
@@ -441,7 +420,12 @@ struct pa_groupby {
   std::vector<Column> keys;
   std::vector<KeyField> fields;
   bool packed = false;
-  bool str_verified = false;        // utf8 key: the hash grouping has been checked byte for byte (strkeys.cuh)
+  // hashed key — one utf8 column, or a composite key that does not pack into 64 bits: the key word is a seeded 64-bit
+  // hash (strkeys.cuh, rowkeys.cuh) in packed_keys; key_verified once a pass has checked every row against its group's
+  // first row, key_seed counts the re-hashes after a collision
+  bool hashed = false;
+  bool key_verified = false;
+  uint64_t key_seed = 0;
   DevBuf packed_keys;
   const void* key_data = nullptr;   // what the scan kernels read
   const uint8_t* key_valid = nullptr;
@@ -1286,7 +1270,23 @@ int build_row_lookup(pa_groupby* g, RowLookup* lk) {
   return PA_OK;
 }
 
-int verify_string_keys(pa_groupby* g, bool* collided) {
+// The key columns of a hashed key, as k_row_hash / k_row_verify read them
+RowKeys row_keys(const pa_groupby* g) {
+  RowKeys k{};
+  k.n_cols = static_cast<int>(g->keys.size());
+  k.n = g->n;
+  for (int j = 0; j < k.n_cols; ++j) {
+    const Column& c = g->keys[j];
+    k.valid[j] = c.valid;
+    k.off[j] = c.bit_off;
+    if (c.is_str) k.str[j] = c.str;
+    else { k.col[j] = c.data; k.width[j] = c.width; }
+  }
+  return k;
+}
+
+// Every row of a hashed key against its group's first row (k_row_verify); *collided: two different keys share a hash
+int verify_hashed_keys(pa_groupby* g, bool* collided) {
   cudaStream_t st = g->stream;
   *collided = false;
   if (g->n == 0 || g->G == 0) return PA_OK;
@@ -1296,12 +1296,12 @@ int verify_string_keys(pa_groupby* g, bool* collided) {
   PA_TRY(flag.alloc(4, st));
   CUDA_TRY(cudaMemsetAsync(flag.p, 0, 4, st));
   const int grid = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((g->n + 255) / 256, static_cast<int64_t>(g->num_sms) * 16)));
-  k_str_verify<<<grid, 256, 0, st>>>(g->keys[0].str, lk.a, g->res.first_row, flag.as<uint32_t>());
+  k_row_verify<<<grid, 256, 0, st>>>(row_keys(g), lk.a, g->res.first_row, flag.as<uint32_t>());
   CUDA_TRY(cudaGetLastError());
   uint32_t h = 0;
   CUDA_TRY(cudaMemcpyAsync(&h, flag.p, 4, cudaMemcpyDeviceToHost, st));
   CUDA_TRY(cudaStreamSynchronize(st));
-  if (h == 2u) return set_err(PA_ERR_STATE, "utf8 keys: a row's hash is missing from the group table");
+  if (h == 2u) return set_err(PA_ERR_STATE, "%s: a row's hash is missing from the group table", g->keys.size() == 1 ? "utf8 keys" : "hashed composite key");
   *collided = h != 0;
   return PA_OK;
 }
@@ -1618,8 +1618,17 @@ int key_bits(int width, bool is_dict, int64_t dict_len) {
   return (is_dict && dict_len > 0) ? bits_for(static_cast<uint64_t>(dict_len)) : width * 8;
 }
 
+// Bits a composite key packs into under layout l: value bits plus a null bit per nullable column
+int layout_bits(const pa_key_layout& l) {
+  int bits = 0;
+  for (int j = 0; j < l.n_keys; ++j) bits += l.bits[j] + l.nullable[j];
+  return bits;
+}
+
 // The one place the packing order is decided: column j at the bits after columns 0 .. j-1, value bits then null bit.
 int layout_fields(const pa_key_layout& l, std::vector<KeyField>* fields) {
+  const int total = layout_bits(l);
+  if (total > 64) return set_err(PA_ERR_NOT_IMPLEMENTED, "composite key needs %d bits; only keys that pack into 64 bits are supported", total);
   fields->assign(l.n_keys, KeyField{});
   int shift = 0;
   for (int j = 0; j < l.n_keys; ++j) {
@@ -1628,7 +1637,6 @@ int layout_fields(const pa_key_layout& l, std::vector<KeyField>* fields) {
     f.shift = shift;
     shift += f.bits + f.nullable;
   }
-  if (shift > 64) return set_err(PA_ERR_NOT_IMPLEMENTED, "composite key needs %d bits; only keys that pack into 64 bits are supported", shift);
   return PA_OK;
 }
 
@@ -1773,11 +1781,45 @@ int pack_keys(pa_groupby* g) {
   return PA_OK;
 }
 
+// Collision hook for tests (PA_TEST_STR_HASH_BITS=b): hashes made under seed 0 keep only their low b bits, so that
+// different keys share a hash on demand — utf8 keys and hashed composite keys alike.  Unset: every bit is kept.
+uint64_t test_hash_keep(uint64_t seed) {
+  static const char* bits = getenv("PA_TEST_STR_HASH_BITS");
+  if (!bits || seed != 0) return ~0ull;
+  const int b = atoi(bits);
+  return b <= 0 ? 0ull : b >= 64 ? ~0ull : (1ull << b) - 1;
+}
+
+// A hashed key's words under g->key_seed: k_str_hash for one utf8 column (the words shards exchange), k_row_hash for a
+// composite key
+int hash_keys(pa_groupby* g) {
+  cudaStream_t st = g->stream;
+  const uint64_t seed = 0x5851F42D4C957F2Dull + g->key_seed * 0x9E3779B97F4A7C15ull, keep = test_hash_keep(g->key_seed);
+  PA_TRY(g->packed_keys.alloc(static_cast<size_t>(std::max<int64_t>(g->n, 1)) * 8, st));
+  uint64_t* out = g->packed_keys.as<uint64_t>();
+  if (g->n > 0) {
+    const int grid = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((g->n + 255) / 256, static_cast<int64_t>(g->num_sms) * 16)));
+    const Column& k = g->keys[0];
+    if (g->keys.size() == 1) k_str_hash<<<grid, 256, 0, st>>>(k.str, k.valid, k.bit_off, g->n, seed, keep, out);
+    else k_row_hash<<<grid, 256, 0, st>>>(row_keys(g), seed, keep, out);
+    CUDA_TRY(cudaGetLastError());
+  }
+  g->key_data = out;
+  return PA_OK;
+}
+
+// Packed when the key is one fixed-width column (verbatim) or a composite key whose layout fits 64 bits (k_pack_keys);
+// otherwise — a utf8 column, or more than 64 bits — hashed.
 int setup_keys(pa_groupby* g) {
   const int nk = static_cast<int>(g->keys.size());
+  if (nk > kMaxKeyCols) return set_err(PA_ERR_INVALID, "at most %d key columns", kMaxKeyCols);
+  bool has_str = false;
+  for (const Column& k : g->keys) {
+    if (!k.is_str && k.width != 4 && k.width != 8) return set_err(PA_ERR_INVALID, "key columns must be 32- or 64-bit (format '%s')", k.format.c_str());
+    has_str = has_str || k.is_str;
+  }
   if (nk == 1) {
     const Column& k = g->keys[0];
-    if (k.width != 4 && k.width != 8) return set_err(PA_ERR_INVALID, "key columns must be 32- or 64-bit (format '%s')", k.format.c_str());
     g->fields.assign(1, KeyField{});
     g->packed = false;
     g->key_data = k.data;
@@ -1785,15 +1827,22 @@ int setup_keys(pa_groupby* g) {
     g->key_bit_off = k.bit_off;
     g->key_width = k.width;
     g->fields[0].width = k.width;
-    return PA_OK;
+    g->hashed = k.is_str;
+    return k.is_str ? hash_keys(g) : PA_OK;
   }
-  if (nk > kMaxKeyCols) return set_err(PA_ERR_INVALID, "at most %d key columns", kMaxKeyCols);
-  for (const Column& k : g->keys)
-    if (k.width != 4 && k.width != 8) return set_err(PA_ERR_INVALID, "key columns must be 32- or 64-bit (format '%s')", k.format.c_str());
   pa_key_layout own;
   column_layout(g, &own);
-  PA_TRY(layout_fields(own, &g->fields));
-  return pack_keys(g);
+  if (!has_str && layout_bits(own) <= 64) {
+    PA_TRY(layout_fields(own, &g->fields));
+    return pack_keys(g);
+  }
+  g->fields.clear();
+  g->packed = false;
+  g->hashed = true;
+  g->key_valid = nullptr;   // every row belongs to a regular group: nulls are part of the hashed row
+  g->key_bit_off = 0;
+  g->key_width = 8;
+  return hash_keys(g);
 }
 
 // A merged handle's composite key: the records carry the packed word, pa_groupby_unique unpacks column j of it
@@ -1815,30 +1864,40 @@ int set_merged_layout(pa_groupby* g, const pa_key_layout& l, const char* const* 
   return PA_OK;
 }
 
-int verify_string_keys(pa_groupby* g, bool* collided);
+// Drops everything computed from the handle's key words (after a repack or a rehash)
+void drop_results(pa_groupby* g) {
+  g->have_groups = false; g->bk_have_hist = false; g->G = 0; g->outs.clear();
+  g->have_groupings = false;
+  g->parts_n = 0;
+  g->s2_ext = 0; g->s2_m2.reset(); g->s2_prod.reset();
+  g->cd_have = false; g->cd_n = 0; g->cd_id.reset(); g->cd_bits.reset(); g->dp_parts_n = 0;
+}
+
+// Hashed key: rehash with hash seed `seed`; the next aggregate groups and checks anew
+int set_key_seed(pa_groupby* g, uint64_t seed) {
+  if (g->key_seed == seed) return PA_OK;
+  g->key_seed = seed;
+  PA_TRY(hash_keys(g));
+  g->key_verified = false;
+  drop_results(g);
+  return PA_OK;
+}
 
 int aggregate_impl_raw(pa_groupby* g, const Column* val, uint32_t mask, bool deferred, int start_at);
 
-// utf8 keys are grouped by a seeded 64-bit hash of their bytes; the first pass on a handle checks the grouping byte
-// for byte against each group's representative and, should two different strings ever share a hash, re-hashes the
-// column with another seed and repeats (strkeys.cuh).
+// Hashed keys (one utf8 column, or a composite key that does not pack into 64 bits) are grouped by a seeded 64-bit
+// hash; the first pass on a handle checks every row against its group's representative and, should two different
+// keys ever share a hash, re-hashes with another seed and repeats (strkeys.cuh, rowkeys.cuh).
 int aggregate_impl(pa_groupby* g, const Column* val, uint32_t mask, bool deferred = false, int start_at = 0) {
-  const bool str = !g->resample && !g->merged && g->keys.size() == 1 && g->keys[0].is_str;
-  if (!str || g->str_verified) return aggregate_impl_raw(g, val, mask, deferred, start_at);
+  if (!g->hashed || g->key_verified) return aggregate_impl_raw(g, val, mask, deferred, start_at);
   for (int attempt = 0; attempt < 4; ++attempt) {
     PA_TRY(aggregate_impl_raw(g, val, mask, false, attempt == 0 ? start_at : 0));
     bool collided = false;
-    PA_TRY(verify_string_keys(g, &collided));
-    if (!collided) { g->str_verified = true; return PA_OK; }
-    g->keys[0].str_seed += 1;
-    PA_TRY(hash_string_key(&g->keys[0], g->stream, g->num_sms));
-    g->key_data = g->keys[0].data;
-    g->have_groups = false;
-    g->bk_have_hist = false;
-    g->G = 0;
-    g->outs.clear();
+    PA_TRY(verify_hashed_keys(g, &collided));
+    if (!collided) { g->key_verified = true; return PA_OK; }
+    PA_TRY(set_key_seed(g, g->key_seed + 1));
   }
-  return set_err(PA_ERR_STATE, "utf8 keys: four differently seeded 64-bit hashes all collided");
+  return set_err(PA_ERR_STATE, "%s: four differently seeded 64-bit hashes all collided", g->keys.size() == 1 ? "utf8 keys" : "hashed composite key");
 }
 
 int aggregate_impl_raw(pa_groupby* g, const Column* val, uint32_t mask, bool deferred, int start_at) {
@@ -2355,8 +2414,7 @@ int pa_groupby_create(const struct ArrowDeviceArray* keys, const struct ArrowSch
   for (int i = 0; i < n_keys; ++i) {
     const char* kf = key_schemas[i].format;
     if (kf && (kf[0] == 'u' || kf[0] == 'U') && kf[1] == 0) {
-      if (n_keys != 1) return set_err(PA_ERR_NOT_IMPLEMENTED, "utf8 keys inside a composite key: dictionary-encode that column");
-      PA_TRY(load_string_key(&keys[i], &key_schemas[i], g->stream, g->device, g->num_sms, &g->keys[i]));
+      PA_TRY(load_string_key(&keys[i], &key_schemas[i], g->stream, g->device, &g->keys[i]));
     } else {
       PA_TRY(load_column(&keys[i], &key_schemas[i], g->stream, g->device, &g->keys[i]));
     }
@@ -2383,22 +2441,44 @@ int pa_groupby_num_groups(pa_groupby* g, int64_t* out) {
   return PA_OK;
 }
 
-static int unique_strings(pa_groupby* g, const StrCol& col, const uint32_t* rows, bool large, struct ArrowArray* out,
+static int unique_strings(pa_groupby* g, const StrCol& col, const uint32_t* rows, const uint8_t* kind, bool large, struct ArrowArray* out,
                           struct ArrowSchema* out_schema);
+
+// unique(j) of a hashed key: column j at every group's first row, with its validity
+static int unique_hashed(pa_groupby* g, int32_t key_i, struct ArrowArray* out, struct ArrowSchema* out_schema) {
+  cudaStream_t st = g->stream;
+  const Column& k = g->keys[key_i];
+  const uint32_t G = g->G;
+  DevBuf kind, vals, valid;
+  PA_TRY(kind.alloc(std::max<uint32_t>(G, 1), st));
+  if (!k.is_str) PA_TRY(vals.alloc(static_cast<size_t>(std::max<uint32_t>(G, 1)) * k.width, st));
+  if (G) {
+    k_gather_rep<<<(G + 255) / 256, 256, 0, st>>>(k.is_str ? nullptr : k.data, k.width, k.valid, k.bit_off, g->res.first_row, G, vals.p, kind.as<uint8_t>());
+    CUDA_TRY(cudaGetLastError());
+  }
+  if (k.is_str) return unique_strings(g, k.str, g->res.first_row, kind.as<uint8_t>(), k.str.wide != 0, out, out_schema);
+  PA_TRY(valid.alloc(((static_cast<size_t>(G) + 31) / 32 + 1) * 4, st));
+  if (G) {
+    k_kind_validity<<<(G + 31) / 32 * 32 / 256 + 1, 256, 0, st>>>(kind.as<uint8_t>(), G, valid.as<uint32_t>());
+    CUDA_TRY(cudaGetLastError());
+  }
+  return export_host(st, k.format, k.width, G, vals.p, valid.as<uint32_t>(), out, out_schema);
+}
 
 int pa_groupby_unique(pa_groupby* g, int32_t key_i, struct ArrowArray* out, struct ArrowSchema* out_schema) {
   if (!g || !out || !out_schema) return set_err(PA_ERR_INVALID, "null argument");
   PA_TRY(ensure_groups(g));
   PA_TRY(ensure_device(g));
-  if (!g->resample && !g->merged && g->keys.size() == 1 && g->keys[0].is_str) {
-    if (key_i != 0) return set_err(PA_ERR_INVALID, "key index %d out of range", key_i);
-    return unique_strings(g, g->keys[0].str, g->res.first_row, g->keys[0].str.wide != 0, out, out_schema);
+  if (g->hashed) {
+    if (key_i < 0 || key_i >= static_cast<int>(g->keys.size())) return set_err(PA_ERR_INVALID, "key index %d out of range", key_i);
+    if (g->keys.size() == 1) return unique_strings(g, g->keys[0].str, g->res.first_row, g->res.key_kind, g->keys[0].str.wide != 0, out, out_schema);
+    return unique_hashed(g, key_i, out, out_schema);
   }
   if (g->merged && g->ks_str) {
     if (key_i != 0) return set_err(PA_ERR_INVALID, "key index %d out of range", key_i);
     if (!g->ks_have) return set_err(PA_ERR_STATE, "utf8 merged handle without its key strings: call pa_merge_key_strings first");
     const StrCol col{g->ks_off.p, g->ks_bytes.as<uint8_t>(), 1};
-    return unique_strings(g, col, g->ks_rows.as<uint32_t>(), g->keys[0].format == "U", out, out_schema);
+    return unique_strings(g, col, g->ks_rows.as<uint32_t>(), g->res.key_kind, g->keys[0].format == "U", out, out_schema);
   }
   if (g->resample) {
     if (key_i != 0) return set_err(PA_ERR_INVALID, "key index %d out of range", key_i);
@@ -2669,14 +2749,15 @@ int ensure_groupings(pa_groupby* g) {
 
 // unique() of a utf8 / large_utf8 key: the bytes of col's row rows[g] for every group g, in group order — a local
 // handle's first rows in its key column, or a merged handle's compacted representatives — as utf8 (large: large_utf8)
-// with int32 offsets (a result of more than 2 GiB of distinct strings is refused).
-static int unique_strings(pa_groupby* g, const StrCol& col, const uint32_t* rows, bool large, struct ArrowArray* out,
+// with int32 offsets (a result of more than 2 GiB of distinct strings is refused).  kind[g] == KK_NULL: group g's
+// string is null (the key kinds, or a hashed composite key's column at the first rows).
+static int unique_strings(pa_groupby* g, const StrCol& col, const uint32_t* rows, const uint8_t* kind, bool large, struct ArrowArray* out,
                           struct ArrowSchema* out_schema) {
   cudaStream_t st = g->stream;
   const uint32_t G = g->G;
   DevBuf offs, tile_sums, bytes, valid;
   PA_TRY(offs.alloc(static_cast<size_t>(G + 1) * 4, st));
-  k_str_lengths<<<(G + 1 + 255) / 256, 256, 0, st>>>(col, rows, g->res.key_kind, G, offs.as<uint32_t>());
+  k_str_lengths<<<(G + 1 + 255) / 256, 256, 0, st>>>(col, rows, kind, G, offs.as<uint32_t>());
   CUDA_TRY(cudaGetLastError());
   uint64_t total64 = 0;
   {
@@ -2693,9 +2774,9 @@ static int unique_strings(pa_groupby* g, const StrCol& col, const uint32_t* rows
   PA_TRY(bytes.alloc(std::max<uint64_t>(total64, 1), st));
   PA_TRY(valid.alloc(((static_cast<size_t>(G) + 31) / 32 + 1) * 4, st));
   if (G) {
-    k_str_gather<<<(static_cast<uint64_t>(G) * 32 + 255) / 256, 256, 0, st>>>(col, rows, g->res.key_kind, G, offs.as<uint32_t>(), bytes.as<uint8_t>());
+    k_str_gather<<<(static_cast<uint64_t>(G) * 32 + 255) / 256, 256, 0, st>>>(col, rows, kind, G, offs.as<uint32_t>(), bytes.as<uint8_t>());
     CUDA_TRY(cudaGetLastError());
-    k_kind_validity<<<(G + 31) / 32 * 32 / 256 + 1, 256, 0, st>>>(g->res.key_kind, G, valid.as<uint32_t>());
+    k_kind_validity<<<(G + 31) / 32 * 32 / 256 + 1, 256, 0, st>>>(kind, G, valid.as<uint32_t>());
     CUDA_TRY(cudaGetLastError());
   }
   auto* priv = new ExportPriv();
@@ -3373,38 +3454,29 @@ int pa_sort_indices(pa_groupby* g, struct ArrowArray* out, struct ArrowSchema* o
 }
 
 // ---- multi-GPU partial export / merge ----
+// A hashed composite key's word is a hash that an owner could only check against the key's columns, which do not
+// travel: such a key groups on one GPU.
+static int check_not_hashed_composite(const pa_groupby* g) {
+  if (g->hashed && g->keys.size() > 1)
+    return set_err(PA_ERR_NOT_IMPLEMENTED, "a hashed composite key (one wider than 64 bits, or with a utf8 column) groups on one GPU: "
+                                           "it has no key layout, partial records or distinct pairs to exchange across shards or chunks");
+  return PA_OK;
+}
+
 // keys the plain record exchange routes: one fixed-width column, a packed composite key or a resample index.  A utf8
 // key's record carries a hash the owner cannot check without the key bytes: the _utf8 entry points export both.
 static int check_shardable(const pa_groupby* g) {
+  PA_TRY(check_not_hashed_composite(g));
   if (!g->resample && g->keys[0].is_str)
     return set_err(PA_ERR_NOT_IMPLEMENTED, "partial records of utf8 keys need their key bytes: use pa_groupby_partials_count_utf8 / "
                                            "pa_groupby_partials_export_utf8 (the padded exchange does not take utf8 keys)");
   return PA_OK;
 }
 
-static bool is_str_key(const pa_groupby* g) { return !g->resample && !g->merged && g->keys.size() == 1 && g->keys[0].is_str; }
-
-// Drops everything computed from the handle's key words (after a repack or a rehash)
-static void drop_results(pa_groupby* g) {
-  g->have_groups = false; g->bk_have_hist = false; g->G = 0; g->outs.clear();
-  g->have_groupings = false;
-  g->parts_n = 0;
-  g->s2_ext = 0; g->s2_m2.reset(); g->s2_prod.reset();
-  g->cd_have = false; g->cd_n = 0; g->cd_id.reset(); g->cd_bits.reset(); g->dp_parts_n = 0;
-}
-
-// utf8 key: rehash the column with hash seed `seed` (strkeys.cuh); the next aggregate groups and checks anew
-static int set_str_seed(pa_groupby* g, uint64_t seed) {
-  if (g->keys[0].str_seed == seed) return PA_OK;
-  g->keys[0].str_seed = seed;
-  PA_TRY(hash_string_key(&g->keys[0], g->stream, g->num_sms));
-  g->key_data = g->keys[0].data;
-  g->str_verified = false;
-  drop_results(g);
-  return PA_OK;
-}
+static bool is_str_key(const pa_groupby* g) { return g->hashed && g->keys.size() == 1; }
 
 static int check_composite_local(const pa_groupby* g) {
+  PA_TRY(check_not_hashed_composite(g));
   if (g->resample || g->merged || !g->packed) return set_err(PA_ERR_INVALID, "key layouts describe the composite key (2+ columns) of a pa_groupby_create handle");
   return PA_OK;
 }
@@ -3574,11 +3646,13 @@ static int partials_export(pa_groupby* g, int32_t n_parts, void* dev_records, in
 }
 
 int pa_groupby_partials_export(pa_groupby* g, int32_t n_parts, void* dev_records, int64_t capacity_records) {
+  if (g) PA_TRY(check_not_hashed_composite(g));
   return partials_export(g, n_parts, dev_records, capacity_records, REC_WORDS);
 }
 
 int pa_groupby_partials_export_stage2(pa_groupby* g, int32_t n_parts, void* dev_records, int64_t capacity_records) {
   if (g && g->merged) return set_err(PA_ERR_STATE, "partials need a finished local aggregate");
+  if (g) PA_TRY(check_not_hashed_composite(g));
   return partials_export(g, n_parts, dev_records, capacity_records, REC_WORDS_STAGE2);
 }
 
@@ -3589,6 +3663,7 @@ static int pairs_check(pa_groupby* g, int32_t n_parts) {
   if (n_parts < 1 || n_parts > 64) return set_err(PA_ERR_INVALID, "bad argument (1 <= n_parts <= 64)");
   PA_TRY(finish_pending(g));
   if (g->merged) return set_err(PA_ERR_STATE, "distinct pairs come from a local aggregate, not from a merged handle");
+  PA_TRY(check_not_hashed_composite(g));
   if (!g->cd_have) return set_err(PA_ERR_STATE, "the last aggregate computed no count_distinct: no distinct pairs to export");
   return ensure_device(g);
 }
@@ -3850,8 +3925,10 @@ static int merge_key_strings(pa_groupby* m, const uint64_t* recs, int words, uin
 
 int pa_groupby_key_hash_seed(pa_groupby* g, uint64_t* seed) {
   if (!g || !seed) return set_err(PA_ERR_INVALID, "null argument");
-  if (!is_str_key(g)) return set_err(PA_ERR_INVALID, "key hash seeds belong to a pa_groupby_create handle with one utf8 / large_utf8 key");
-  *seed = g->keys[0].str_seed;
+  if (!g->hashed)
+    return set_err(PA_ERR_INVALID, "key hash seeds belong to a pa_groupby_create handle with a hashed key (one utf8 / large_utf8 key, "
+                                   "or a composite key that does not pack into 64 bits)");
+  *seed = g->key_seed;
   return PA_OK;
 }
 
@@ -3860,13 +3937,14 @@ int pa_groupby_set_key_hash_seed(pa_groupby* g, uint64_t seed) {
   if (!is_str_key(g)) return set_err(PA_ERR_INVALID, "key hash seeds belong to a pa_groupby_create handle with one utf8 / large_utf8 key");
   PA_TRY(ensure_device(g));
   PA_TRY(finish_pending(g));
-  return set_str_seed(g, seed);
+  return set_key_seed(g, seed);
 }
 
 int pa_groupby_partials_count_utf8(pa_groupby* g, int32_t n_parts, int64_t* records_host, int64_t* bytes_host) {
   if (!g || !records_host || !bytes_host || n_parts < 1 || n_parts > 64) return set_err(PA_ERR_INVALID, "bad argument (1 <= n_parts <= 64)");
   PA_TRY(finish_pending(g));
   if (!g->have_groups || g->merged) return set_err(PA_ERR_STATE, "partials need a finished local aggregate");
+  PA_TRY(check_not_hashed_composite(g));
   if (!is_str_key(g)) return set_err(PA_ERR_INVALID, "pa_groupby_partials_count_utf8 takes one utf8 / large_utf8 key; use pa_groupby_partials_count");
   PA_TRY(ensure_device(g));
   cudaStream_t st = g->stream;
@@ -3892,6 +3970,7 @@ int pa_groupby_partials_export_utf8(pa_groupby* g, int32_t n_parts, int32_t stag
                                     void* dev_lengths, void* dev_bytes, int64_t capacity_bytes) {
   if (!g || !dev_records) return set_err(PA_ERR_INVALID, "null argument");
   if (g->merged) return set_err(PA_ERR_STATE, "partials need a finished local aggregate");
+  PA_TRY(check_not_hashed_composite(g));
   if (!is_str_key(g)) return set_err(PA_ERR_INVALID, "pa_groupby_partials_export_utf8 takes one utf8 / large_utf8 key; use pa_groupby_partials_export");
   if (g->parts_n != n_parts || g->ks_counts.size() != static_cast<size_t>(n_parts))
     return set_err(PA_ERR_STATE, "call pa_groupby_partials_count_utf8(n_parts=%d) first", n_parts);
@@ -4068,6 +4147,19 @@ int pa_groupby_aggregate_chunked_keys(const struct ArrowDeviceArray* keys, const
   pa_options o;
   if (opt) o = *opt; else pa_options_init(&o);
   const int64_t base0 = o.row_base;
+  // Chunks merge by their packed key words, so a composite key must pack into 64 bits — decided here, from the whole
+  // columns, because pa_groupby_create would hash a chunk that does not pack
+  if (composite) {
+    for (int j = 0; j < n_keys; ++j) {
+      const char* f = key_schemas[j].format;
+      if (f && (f[0] == 'u' || f[0] == 'U') && f[1] == 0)
+        return set_err(PA_ERR_NOT_IMPLEMENTED, "utf8 keys inside a composite key: dictionary-encode that column");
+    }
+    if (n_keys <= PA_MAX_KEY_COLS) {
+      std::vector<KeyField> fields;
+      PA_TRY(layout_fields(whole, &fields));
+    }
+  }
   // utf8 key: every chunk hashes with one seed and exports its key bytes next to its records; a chunk whose own check
   // moves the seed, or a merge that finds two strings under one hash, redoes the chunks with the next seed (four at most)
   const char* kf0 = key_schemas[0].format;
@@ -4112,10 +4204,10 @@ int pa_groupby_aggregate_chunked_keys(const struct ArrowDeviceArray* keys, const
         if (mine.width[j] != whole.width[j] || mine.bits[j] != whole.bits[j] || mine.nullable[j] != whole.nullable[j])
           return set_err(PA_ERR_STATE, "chunk %lld packs key column %d differently from the whole column", (long long)c, j);
     }
-    if (str) PA_TRY(set_str_seed(h, seed));
+    if (str) PA_TRY(set_key_seed(h, seed));
     PA_TRY(pa_groupby_aggregate(h, &vc, value_schema, agg_mask));
-    if (str && h->keys[0].str_seed != seed) {   // this chunk's own check moved the seed
-      seed = h->keys[0].str_seed;
+    if (str && h->key_seed != seed) {   // this chunk's own check moved the seed
+      seed = h->key_seed;
       reseed = true;
       break;
     }
@@ -4318,8 +4410,10 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   const int W = c->world;
   // 0. composite key: every rank's key layout to everybody, one agreed layout, repack when it differs from this
   // handle's.  On every step (never cached): a rank that skipped the gather while another ran it would hang the step.
-  // A rank that cannot describe its layout still takes part (with n_keys = 0), so that every rank fails together.
-  const bool composite = g->packed && !g->resample;
+  // A rank that cannot describe its layout still takes part (with n_keys = 0), so that every rank fails together.  That
+  // includes a rank whose composite key is hashed (whether a key packs depends on the shard's own nulls and
+  // dictionaries), so the branch is taken on the number of key columns.
+  const bool composite = !g->resample && g->keys.size() > 1;
   pa_key_layout agreed{};
   c->agree_ms = 0; c->repack_ms = 0;
   if (composite) {
@@ -4373,7 +4467,7 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   const bool full_only = stage2 || distinct || (agg_mask & (PA_AGG_BOOL_ALL | PA_AGG_BOOL_ANY));
   const bool compact = !full_only && !is_wide(agg_mask, vc_) && !(agg_mask & (AGG_FIRST | AGG_LAST));
   // (a utf8 key's first pass checks its grouping byte for byte, which reads the ordered groups)
-  g->want_unordered = compact && !g->resample && (!str || g->str_verified);
+  g->want_unordered = compact && !g->resample && (!str || g->key_verified);
   const int local_rc = aggregate_entry(g, values, value_schema, agg_mask, false);
   g->want_unordered = false;
   if (local_rc != PA_OK) return local_rc;
@@ -4404,7 +4498,7 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
   }
   if (distinct) PA_TRY(pairs_count_async(g, W, c->d_counts.as<unsigned long long>() + W + 1));
   if (str) {
-    c->h_seed = g->keys[0].str_seed;
+    c->h_seed = g->key_seed;
     CUDA_TRY(cudaMemcpyAsync(c->d_counts.as<uint64_t>() + KS, &c->h_seed, sizeof(uint64_t), cudaMemcpyHostToDevice, st));
     PA_TRY(keystr_count_async(g, W, unordered ? g->unordered_recs : nullptr, G_local, c->d_counts.as<unsigned long long>() + KS + 1));
   }
@@ -4420,7 +4514,7 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
     }
     if (hi >= 4) return set_err(PA_ERR_STATE, "utf8 keys: four differently seeded 64-bit hashes all collided");
     if (lo != hi) {
-      PA_TRY(set_str_seed(g, hi));
+      PA_TRY(set_key_seed(g, hi));
       continue;
     }
   }
@@ -4527,11 +4621,11 @@ int pa_groupby_sharded_aggregate(pa_groupby* g, pa_comm* c, const struct ArrowDe
     CUDA_TRY(cudaStreamSynchronize(st));
     c->last_bytes_sent = static_cast<int64_t>(ksend_total);
     c->last_bytes_received = static_cast<int64_t>(krecv_total);
-    c->last_seed = g->keys[0].str_seed;
+    c->last_seed = g->key_seed;
     c->last_attempts = attempt;
     if (c->h_flag) {
-      if (g->keys[0].str_seed + 1 >= 4) return set_err(PA_ERR_STATE, "utf8 keys: four differently seeded 64-bit hashes all collided");
-      PA_TRY(set_str_seed(g, g->keys[0].str_seed + 1));
+      if (g->key_seed + 1 >= 4) return set_err(PA_ERR_STATE, "utf8 keys: four differently seeded 64-bit hashes all collided");
+      PA_TRY(set_key_seed(g, g->key_seed + 1));
       continue;
     }
   }

@@ -3,9 +3,9 @@
 // reference's golden tests key on strings (tests/cudf_examples/dataframe_resample_test.cpp:8-69); round 1
 // dictionary-encoded such keys on the HOST.  Here:
 //   k_str_hash    every row's string -> a seeded 64-bit hash; the ordinary stages 1-3 then run on that 8-byte column
-//   k_str_verify  exactness: every row's bytes are compared with the bytes of its group's first row (the group's
-//                 representative); two different strings with one hash set a flag and the host re-hashes the
-//                 column with another seed (probability ~ n_groups^2 / 2^65 per attempt)
+//   exactness: every row's bytes are compared with the bytes of its group's first row (the group's representative,
+//              k_row_verify in rowkeys.cuh); two different strings with one hash set a flag and the host re-hashes the
+//              column with another seed (probability ~ n_groups^2 / 2^65 per attempt)
 //   k_str_lengths / k_str_gather   unique(): lengths of the representatives -> offsets (scan) -> bytes
 #pragma once
 #include "bucketed.cuh"
@@ -50,25 +50,6 @@ __global__ void __launch_bounds__(256) k_str_hash(StrCol c, const uint8_t* valid
     if (valid && !bit_at(valid, bit_off + i)) { out[i] = 0; continue; }
     const int64_t a = str_off(c, i), b = str_off(c, i + 1);
     out[i] = str_hash64(c.bytes + a, b - a, seed) & keep;
-  }
-}
-
-// Every row against the representative (first row) of the group its HASH belongs to; `a` is the read-only
-// hash -> group lookup of rowids.cuh built over the hash column.
-__global__ void __launch_bounds__(256) k_str_verify(StrCol c, RowIdArgs a, const uint32_t* first_row, uint32_t* collision) {
-  int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-  const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
-  for (; i < a.n; i += stride) {
-    if (a.kvalid && !bit_at(a.kvalid, a.koff + i)) continue;
-    const uint32_t g = rowid_lookup(a, i);
-    if (g >= a.G) { atomicExch(collision, 2u); continue; }
-    const int64_t r = first_row[g];
-    if (r == i) continue;
-    const int64_t x = str_off(c, i), lx = str_off(c, i + 1) - x;
-    const int64_t y = str_off(c, r), ly = str_off(c, r + 1) - y;
-    bool same = lx == ly;
-    for (int64_t j = 0; same && j < lx; ++j) same = c.bytes[x + j] == c.bytes[y + j];
-    if (!same) atomicExch(collision, 1u);
   }
 }
 

@@ -166,19 +166,26 @@ Column = Union[pa.Array, DeviceColumn]
 
 
 class GroupBy:
-    """pd::GroupBy: hash group-by on one (or several 64-bit-packable) key column(s).
+    """pd::GroupBy: hash group-by on one or several (up to 4) key columns.
 
     `frame` maps column names to columns (pyarrow RecordBatch/Table, or a dict of pa.Array /
     DeviceColumn); `key` names the key column(s) — or pass key arrays directly with `key_arrays`
-    (DataFrame::group_by(ArrayPtr), dataframe.cpp:1231-1235)."""
+    (DataFrame::group_by(ArrayPtr), dataframe.cpp:1231-1235).
+
+    A composite key that packs into 64 bits groups on its packed word; a wider one (two int64 ids, say) groups on a
+    seeded 64-bit row hash that the first pass checks row by row.  encode_utf8=True dictionary-encodes utf8 members of
+    a composite key on the host (their codes pack); encode_utf8=False hands them to the library as strings (a hashed
+    key, unique(j) returns the strings).  Only packed composite keys cross GPUs or host chunks."""
 
     def __init__(self, key, frame=None, *, key_arrays: Optional[Sequence[Column]] = None, expected_groups: int = 0,
                  path: str = "auto", device: Optional[int] = None, stream: Optional[int] = None, row_base: int = 0,
-                 no_dense: bool = False, no_partition: bool = False, bucket_bits: int = 0, sm_reserve: int = 0, _handle=None):
+                 no_dense: bool = False, no_partition: bool = False, bucket_bits: int = 0, sm_reserve: int = 0,
+                 encode_utf8: bool = True, _handle=None):
         self._L = _lib.load()
         self._h = C.c_void_p()
         self._frame = self._as_dict(frame)
         self._dicts: List[Optional[pa.Array]] = []
+        self._encode_utf8 = encode_utf8
         if _handle is not None:
             self._h = _handle
             self.key_names = ["__resampler_idx__"]
@@ -206,9 +213,10 @@ class GroupBy:
         if isinstance(k, pa.ChunkedArray):
             k = k.combine_chunks()
         if (isinstance(k, pa.Array) and (pa.types.is_string(k.type) or pa.types.is_large_string(k.type))
-                and len(self.key_names) > 1):
+                and len(self.key_names) > 1 and self._encode_utf8):
             # a utf8 column inside a COMPOSITE key is dictionary-encoded (its codes pack into the 64-bit key); a single
-            # utf8 key goes to the device as strings (format "u": offsets + bytes, csrc/strkeys.cuh)
+            # utf8 key, or any with encode_utf8=False, goes to the device as strings (format "u": offsets + bytes,
+            # csrc/strkeys.cuh, csrc/rowkeys.cuh)
             k = k.dictionary_encode()
         self._dicts.append(k.dictionary if isinstance(k, pa.DictionaryArray) else None)
         return k
@@ -354,7 +362,8 @@ class GroupBy:
 
     # ---- a single utf8 / large_utf8 key across shards: records travel with their key bytes ----
     def key_hash_seed(self) -> int:
-        """pa_groupby_key_hash_seed: the seed this utf8 key is hashed with (raised by the handle's own byte check)."""
+        """pa_groupby_key_hash_seed: the seed this utf8 key, or hashed composite key, is hashed with (raised by the
+        handle's own check)."""
         out = C.c_uint64()
         _check(self._L.pa_groupby_key_hash_seed(self._h, C.byref(out)))
         return out.value
