@@ -23,6 +23,7 @@
 #include "emit.cuh"
 #include "gtable.cuh"
 #include "lowcard.cuh"
+#include "lowcard_known.cuh"
 #include "merge.cuh"
 #include "partition.cuh"
 #include "bucketed.cuh"
@@ -492,6 +493,12 @@ struct pa_groupby {
   uint32_t pending_mask = 0;
   uint32_t pending_prev_G = 0;
   bool pending_had_groups = false;
+  bool pending_lk_record = false;         // the pending pass records the dense facts below
+  // Dense low-cardinality facts of this handle's keys (lowcard_known.cuh): window, group count, id -> rank, count /
+  // first row / key by rank.  Recorded by a full dense narrow-set pass; trusted (lk_valid) once the host has read that
+  // pass's clean status; dropped with everything else computed from the key words and on any aborted pass.
+  DevBuf lk_buf;
+  bool lk_valid = false;
   // deferred fused merge of padded blocks (multi-GPU): status not read yet; the caller keeps the blocks alive
   bool pending_merge = false;
   const void* pm_blocks = nullptr;
@@ -589,12 +596,34 @@ int launch_lowcard_t(pa_groupby* g, const LcArgs& a, const LmArgs& m, int grid, 
   return PA_OK;
 }
 
+// one persistent CTA per SM the handle may use (the order of the floating-point sums depends on it)
+int lc_grid(const pa_groupby* g) {
+  return std::max<int>(1, g->num_sms - static_cast<int>(std::max<int64_t>(0, std::min<int64_t>(g->opt.sm_reserve, g->num_sms - 1))));
+}
+
+// The handle's fact buffers (lowcard_known.cuh): LkHead | id_rank [GP] | count [GP] | first [GP] | key [GP] | kind [GP]
+int lk_facts(pa_groupby* g, LkFacts* f) {
+  constexpr size_t gp = LcCfg<VC_F, false>::GP;
+  PA_TRY(g->lk_buf.alloc(sizeof(LkHead) + gp * (4 + 4 + 4 + 8 + 1), g->stream));
+  char* p = g->lk_buf.as<char>();
+  f->head = reinterpret_cast<LkHead*>(p);
+  f->key = reinterpret_cast<uint64_t*>(p + sizeof(LkHead));
+  f->id_rank = reinterpret_cast<uint32_t*>(f->key + gp);
+  f->count = f->id_rank + gp;
+  f->first = f->count + gp;
+  f->kind = reinterpret_cast<uint8_t*>(f->first + gp);
+  return PA_OK;
+}
+
 int run_lowcard(pa_groupby* g, const Column* val, uint32_t mask, bool wide, bool force_hash, LcOutcome* outcome,
                 bool deferred = false) {
   cudaStream_t st = g->stream;
-  const int grid = std::max<int>(1, g->num_sms - static_cast<int>(std::max<int64_t>(0, std::min<int64_t>(g->opt.sm_reserve, g->num_sms - 1))));
+  const int grid = lc_grid(g);
   const int vc = val ? val->vc : VC_I;
   const bool kwide = lc_is_wide(mask, vc);
+  // a dense pass of the narrow set over a value column without a bitmap (count = group size) records the facts of
+  // the handle's keys for the sum-only passes after it
+  const bool record = !g->lk_valid && !kwide && !force_hash && val && !val->valid;
   const bool dsum = kwide && vc != VC_F;
   const int gp = lc_gmax(vc, kwide) + 2;
   const size_t np = static_cast<size_t>(grid) * gp;
@@ -677,9 +706,17 @@ int run_lowcard(pa_groupby* g, const Column* val, uint32_t mask, bool wide, bool
     else if (vc == VC_I) PA_TRY((launch_lowcard_t<VC_I, false>(g, a, m, grid, fast, force_hash)));
     else PA_TRY((launch_lowcard_t<VC_U, false>(g, a, m, grid, fast, force_hash)));
   }
+  if (record) {
+    LkFacts f;
+    PA_TRY(lk_facts(g, &f));
+    k_lowcard_known_record<<<1, LK_REC_THREADS, 0, st>>>(m, f);
+    CUDA_TRY(cudaGetLastError());
+    g->last_launches += 1;
+  }
   CUDA_TRY(cudaEventRecord(g->ev[3], st));
   if (deferred) {   // the scratch buffers above are released in stream order; the status is read by finish_pending()
     g->G = static_cast<uint32_t>(gp);   // upper bound until then
+    g->pending_lk_record = record;
     *outcome = LC_DONE;
     return PA_OK;
   }
@@ -689,9 +726,92 @@ int run_lowcard(pa_groupby* g, const Column* val, uint32_t mask, bool wide, bool
   if (h_status[ST_OVERFLOW]) *outcome = LC_OVERFLOW;
   else if (h_status[ST_DENSE_MISS]) *outcome = LC_DENSE_MISS;
   else { *outcome = LC_DONE; g->G = h_status[ST_NGROUPS]; }
+  if (*outcome != LC_DONE) g->lk_valid = false;
+  else if (record && h_status[ST_MODE] == 1u) g->lk_valid = true;
   g->last_mode = static_cast<int>(h_status[ST_MODE]);
   g->last_rlog = static_cast<int>(h_status[ST_RLOG]);
   if (h_status[ST_DENSE_MISS] != 2u) g->last_passes += 1;   // (2 = the dense kernel declined before scanning a row)
+  return PA_OK;
+}
+
+// Sum-only pass of a handle whose dense facts are valid (lowcard_known.cuh): narrow set, value column without a bitmap.
+bool lk_applies(const pa_groupby* g, const Column* val, uint32_t mask) {
+  if (!g->lk_valid || !val || val->valid || lc_is_wide(mask, val->vc)) return false;
+  const char* e = std::getenv("PA_LC_NO_KNOWN");   // (read per call: A/B runs in one process)
+  return !(e && std::atoi(e) != 0);
+}
+
+template <int VC>
+int launch_lowcard_known_t(pa_groupby* g, const LcArgs& a, const LmArgs& m, int grid, bool fast, const LkFacts& f) {
+  cudaStream_t st = g->stream;
+  auto scan = fast ? k_lowcard_sums<VC, true> : k_lowcard_sums<VC, false>;
+  CUDA_TRY(cudaFuncSetAttribute(scan, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(LkSmem::TOTAL)));
+  scan<<<grid, LkSmem::WARPS * 32, LkSmem::TOTAL, st>>>(a, f.head);
+  CUDA_TRY(cudaGetLastError());
+  CUDA_TRY(cudaEventRecord(g->ev[2], st));
+  k_lowcard_sums_merge<VC><<<(LcCfg<VC, false>::GP + 7) / 8, 256, 0, st>>>(m, f);
+  CUDA_TRY(cudaGetLastError());
+  g->last_launches += 2;
+  return PA_OK;
+}
+
+int run_lowcard_known(pa_groupby* g, const Column* val, uint32_t mask, LcOutcome* outcome, bool deferred) {
+  cudaStream_t st = g->stream;
+  const int grid = lc_grid(g);
+  const int vc = val->vc;
+  const int gp = lc_gmax(vc, false) + 2;
+  const size_t np = static_cast<size_t>(grid) * gp;
+  DevBuf p_sum, p_seen;
+  PA_TRY(p_sum.alloc(np * 8, st));
+  PA_TRY(p_seen.alloc(np * 4, st));
+  CUDA_TRY(cudaMemsetAsync(g->status.p, 0, sizeof(uint32_t) * ST_WORDS, st));
+  PA_TRY(alloc_result(g, gp, false, vc != VC_F));
+  LkFacts f;
+  PA_TRY(lk_facts(g, &f));
+
+  LcArgs a{};
+  a.keys = g->key_data;
+  a.kvalid = g->key_valid;
+  a.koff = g->key_bit_off;
+  a.kw = g->key_width;
+  a.vals = val->data;
+  a.vw = val->width;
+  a.n = g->n;
+  a.agg_mask = mask;
+  a.p_sum = p_sum.as<uint64_t>();
+  a.p_count = p_seen.as<uint32_t>();   // 1 where the CTA met the id
+  a.status = g->status.as<uint32_t>();
+  const bool aligned = (reinterpret_cast<uintptr_t>(a.keys) % 8 == 0) && (reinterpret_cast<uintptr_t>(a.vals) % 8 == 0);
+  const bool fast = a.vals && aligned && a.kw == 8 && a.vw == 8 && !a.kvalid;
+  LmArgs m{};
+  m.part = a;
+  m.grid = grid;
+  m.gp = gp;
+  m.out = g->res;
+  m.status = a.status;
+  CUDA_TRY(cudaEventRecord(g->ev[1], st));
+  if (vc == VC_F) PA_TRY(launch_lowcard_known_t<VC_F>(g, a, m, grid, fast, f));
+  else if (vc == VC_I) PA_TRY(launch_lowcard_known_t<VC_I>(g, a, m, grid, fast, f));
+  else PA_TRY(launch_lowcard_known_t<VC_U>(g, a, m, grid, fast, f));
+  CUDA_TRY(cudaEventRecord(g->ev[3], st));
+  g->pending_lk_record = false;
+  *outcome = LC_DONE;
+  if (deferred) {
+    g->G = static_cast<uint32_t>(gp);   // upper bound until finish_pending()
+    return PA_OK;
+  }
+  uint32_t h_status[ST_WORDS];
+  CUDA_TRY(cudaMemcpyAsync(h_status, g->status.p, sizeof h_status, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(cudaStreamSynchronize(st));
+  if (h_status[ST_ABORT]) {   // a key outside the recorded window, or a group the facts do not have
+    g->lk_valid = false;
+    *outcome = LC_DENSE_MISS;
+  } else {
+    g->G = h_status[ST_NGROUPS];
+  }
+  g->last_mode = static_cast<int>(h_status[ST_MODE]);
+  g->last_rlog = static_cast<int>(h_status[ST_RLOG]);
+  g->last_passes += 1;
   return PA_OK;
 }
 
@@ -1867,6 +1987,7 @@ int set_merged_layout(pa_groupby* g, const pa_key_layout& l, const char* const* 
 // Drops everything computed from the handle's key words (after a repack or a rehash)
 void drop_results(pa_groupby* g) {
   g->have_groups = false; g->bk_have_hist = false; g->G = 0; g->outs.clear();
+  g->lk_valid = false;
   g->have_groupings = false;
   g->parts_n = 0;
   g->s2_ext = 0; g->s2_m2.reset(); g->s2_prod.reset();
@@ -1922,11 +2043,14 @@ int aggregate_impl_raw(pa_groupby* g, const Column* val, uint32_t mask, bool def
     if (g->n / (static_cast<int64_t>(g->num_sms) * 12) >= (1ll << 24) - 1) try_low = false;
     bool done = false;
     if (start_at == 2) try_low = false;                       // (resuming after a deferred pass overflowed)
+    // the groups of this handle's keys are known from an earlier dense pass: accumulate the sums only
+    const bool known = try_low && start_at == 0 && !g->opt.lowcard_no_dense && lk_applies(g, val, mask);
     if (try_low && deferred && start_at == 0 && !g->opt.lowcard_no_dense) {
       // Deferred: queue the dense-mode pass and the emit without reading the status back.  If the pass turns
       // out to have declined / aborted / overflowed, finish_pending() resumes synchronously from there.
       LcOutcome oc = LC_DONE;
-      PA_TRY(run_lowcard(g, val, mask, wide, false, &oc, true));
+      if (known) PA_TRY(run_lowcard_known(g, val, mask, &oc, true));
+      else PA_TRY(run_lowcard(g, val, mask, wide, false, &oc, true));
       g->last_path = PA_PATH_LOWCARD;
       g->have_groups = true;
       g->last_wide = wide;
@@ -1940,6 +2064,11 @@ int aggregate_impl_raw(pa_groupby* g, const Column* val, uint32_t mask, bool def
       CUDA_TRY(cudaEventRecord(g->ev[4], st));
       g->pending = true;
       return PA_OK;
+    }
+    if (known) {
+      LcOutcome oc = LC_DONE;
+      PA_TRY(run_lowcard_known(g, val, mask, &oc, false));
+      if (oc == LC_DONE) { done = true; try_low = false; g->last_path = PA_PATH_LOWCARD; }   // (else: the full pass below)
     }
     if (try_low) {
       LcOutcome oc = LC_DONE;
@@ -2203,16 +2332,22 @@ int finish_pending(pa_groupby* g) {
   CUDA_TRY(cudaStreamSynchronize(st));
   const Column* val = g->pending_has_val ? &g->pending_val : nullptr;
   int rc = PA_OK;
+  const bool recorded = g->pending_lk_record;
+  g->pending_lk_record = false;
   if (!h_status[ST_OVERFLOW] && !h_status[ST_DENSE_MISS]) {
     g->G = h_status[ST_NGROUPS];
     g->last_mode = static_cast<int>(h_status[ST_MODE]);
     g->last_rlog = static_cast<int>(h_status[ST_RLOG]);
     g->last_passes = 1;
+    if (recorded && h_status[ST_MODE] == 1u && !(g->pending_had_groups && g->pending_prev_G != g->G)) g->lk_valid = true;
   } else {
     const int passes = h_status[ST_DENSE_MISS] == 2u ? 0 : 1;
+    // a sum-only pass that met keys its facts do not describe drops them and redoes the full dense pass
+    const bool known = h_status[ST_MODE] == LK_MODE;
+    g->lk_valid = false;
     g->have_groups = g->pending_had_groups;
     g->G = g->pending_prev_G;
-    rc = aggregate_impl(g, val, g->pending_mask, false, h_status[ST_OVERFLOW] ? 2 : 1);
+    rc = aggregate_impl(g, val, g->pending_mask, false, known ? 0 : (h_status[ST_OVERFLOW] ? 2 : 1));
     g->last_passes += passes;
   }
   if (rc == PA_OK && g->pending_had_groups && g->pending_prev_G != g->G)

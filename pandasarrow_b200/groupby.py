@@ -410,7 +410,8 @@ class GroupBy:
         _check(self._L.pa_groupby_last_detail(self._h, det))
         return {"total_ms": total.value, "pack_ms": st[0], "scan_ms": st[1], "merge_ms": st[2], "emit_ms": st[3],
                 "path": {1: "lowcard", 2: "global", 3: "resample"}.get(path.value, "?"), "launches": launches.value,
-                "mode": {0: None, 1: "dense", 2: "hash", 3: "smem-front", 4: "partitioned", 5: "bucketed"}.get(det[0]), "replication": 1 << det[1], "passes": det[2]}
+                "mode": {0: None, 1: "dense", 2: "hash", 3: "smem-front", 4: "partitioned", 5: "bucketed",
+                         6: "dense-known"}.get(det[0]), "replication": 1 << det[1], "passes": det[2]}
 
     # ---- the reference's method surface (group_by.h:85-139): name -> array, [names] -> {name: array} ----
     def _agg(self, agg: str, arg):
